@@ -115,7 +115,8 @@ def pool_sims_per_s(workers=None, moves=2, sims=100, loggers_on=True):
 
 def measure(engine_budget_s=4.0, moves=2, sims=100, both_logger_modes=True):
     if not available():
-        return {"unavailable": "baseline/_ref not staged (python baseline/stage_ref.py needs /root/reference)"}
+        return {"unavailable": "baseline/_ref not staged (python baseline/stage_ref.py --src <checkout of the reference>, "
+                               "or with HZ_REFERENCE_ROOT set)"}
     out = {"cores": os.cpu_count() or 1, "engine": steps_per_core(engine_budget_s)}
     out["mcts_loggers_on"] = pool_sims_per_s(moves=moves, sims=sims, loggers_on=True)
     if both_logger_modes:

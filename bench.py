@@ -8,8 +8,12 @@ steps/s (1 step = one apply_move-equivalent action on one game) over all ranks, 
 initial states resident in HBM; `e2e` = the same metric through the C-ABI with HOST buffers
 (pinned H2D of the initial states and D2H of the final states inside the timed region).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--games G]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--games G] [--dump-outputs DIR]
     torchrun ... bench.py --gpus N ...        (one rank per GPU, games sharded by rank)
+
+--dump-outputs DIR writes what the last timed wave returned on rank 0 (final records, steps per game,
+total steps) as float64 .npy files, so that two builds can be compared output for output: the inputs
+depend only on the arguments.
 """
 
 import argparse
@@ -47,7 +51,37 @@ def parse():
     ap.add_argument("--mcts-tower", default="hand", choices=["hand", "cudnn"], help="residual tower: the hand-written sm_100a kernel or cuDNN (A/B)")
     ap.add_argument("--mcts-play-games", type=int, default=8192, help="whole self-play games per GPU for the configs[3] measurement (0 = skip)")
     ap.add_argument("--no-python-reference", action="store_true", help="skip timing the staged Python reference (baseline/_ref)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed wave's outputs to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm sizes its waves from a timing calibration)")
+    return a
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, states, steps):
+    """The last timed wave's outputs as float64 (exact for the uint32 record words): final records
+    [n, 32], actions played per game [n] and their total.  Above DUMP_LIMIT_BYTES the games are a fixed
+    seeded sample, whose indices are written as rows.npy."""
+    import numpy as np
+
+    states = states.cpu().numpy().view(np.uint32)
+    steps = steps.cpu().numpy()
+    n = len(states)
+    total = np.array([steps.astype(np.int64).sum()], dtype=np.float64)
+    # 8 bytes per value: 32 record words, the step count and (when sampled) the row index; 4 KB for the headers
+    keep = min(n, (DUMP_LIMIT_BYTES - 4096) // (8 * (32 + 1 + 1)))
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "states.npy"), states[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "steps.npy"), steps[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "total_steps.npy"), total)
+    if keep < n:
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
 
 
 def kernel_counters(name, files):
@@ -231,14 +265,10 @@ def cpu_baseline(budget_s=12.0):
 
 def python_reference(args):
     """The unmodified Python reference (baseline/_ref, staged by baseline/stage_ref.py) on this box's host
-    cores: SURVEY.md §8(d) "CPU baseline timing"."""
+    cores: SURVEY.md §8(d) "CPU baseline timing".  Stage it beforehand with baseline/stage_ref.py."""
     try:
         from baseline import ref_timing as rt
 
-        if not rt.available():
-            from baseline import stage_ref
-
-            stage_ref.stage()              # works where /root/reference exists (the dev container)
         return rt.measure(engine_budget_s=4.0, moves=2, sims=args.mcts_sims)
     except Exception as e:  # noqa: BLE001
         return {"unavailable": repr(e)}
@@ -567,6 +597,7 @@ def run_b200(args):
     barrier()
     wall = time.perf_counter() - wall0
     clocks = sampler.stop()
+    last_states = st
     ms = sum(a.elapsed_time(b) for a, b in ev)
     steps_done = int(total.item())
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -761,6 +792,8 @@ def run_b200(args):
             out["mcts"]["cpu_baseline"] = cpu_mcts_baseline()
             if pyref is not None:
                 out["mcts"]["cpu_baseline"]["python_reference"] = {k: v for k, v in pyref.items() if k != "engine"}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_states, steps_buf)
     if rank == 0:
         print(json.dumps(out))
     if world > 1:

@@ -235,6 +235,30 @@ def test_trainer_hook_fills_replay_buffer(eng):
     assert not trainer_hooks.evaluate_model(et, eval_config=cfg_eval)["promoted"] and calls == []
 
 
+def test_trainer_hook_with_the_test_run_buffer(eng):
+    """The self-play outcome tests/ref_dropin_runner.py checks on the reference's Trainer, on the hook alone: six games into
+    test_run.py's deque(maxlen=100) (config.py:160) leave its last 100 examples, and a second phase plays new games."""
+    from harmonies_alphazero_b200 import net, trainer_hooks
+
+    class Manager:
+        model = net.AlphaZeroNet.from_config(net.TEST_MODEL_CONFIG)
+
+    class Trainer:
+        self_play_config = {"num_games_per_iter": 6}
+        mcts_config = {"num_simulations": 4, "cpuct": 1.0, "dirichlet_alpha": 0.3, "dirichlet_epsilon": 0.25,
+                       "turns_until_tau0": 15, "action_size": 143, "testing": True}
+        replay_buffer = deque(maxlen=100)
+
+    t = Trainer()
+    assert trainer_hooks.execute_self_play_phase(t, Manager(), n_slots=4)["games"] == 6
+    assert len(t.replay_buffer) == 100
+    assert [tuple(x.shape) for x in t.replay_buffer[-1]] == [(38, 5, 7), (42,), (143,), (1,)]
+    first = torch.stack([e[0] for e in t.replay_buffer])
+    trainer_hooks.execute_self_play_phase(t, Manager(), n_slots=4)
+    assert len(t.replay_buffer) == 100
+    assert not torch.equal(torch.stack([e[0] for e in t.replay_buffer]), first)
+
+
 # ---- the reference's private helpers (harmonies_engine.py:120-143,301-354,369-523) -------------
 def test_end_turn_actions_equals_the_tail_of_apply_move(eng):
     """apply_move of a third placement = place the tile, then _end_turn_actions (harmonies_engine.py:
