@@ -93,16 +93,15 @@ __device__ __forceinline__ RandTab rand_table_handle(const uint64_t* rtab) {   /
     __builtin_assume(a != 0);
     return RandTab(a);
 }
+// rand64(key, ctr) with the inner mix read from the table; the caller guarantees a table and ctr < RTAB_N
+__device__ __forceinline__ uint64_t rand64_tab(RandTab rtab, uint64_t key, uint32_t ctr) {
+    uint32_t lo, hi;
+    asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(lo), "=r"(hi) : "r"(rtab.saddr + ctr * 8u));
+    return mix64(key ^ ((uint64_t)lo | ((uint64_t)hi << 32)));
+}
 __device__ __forceinline__ uint64_t rand64_t(RandTab rtab, uint64_t key, uint64_t ctr) {
-    uint64_t inner;
-    if (rtab.saddr != 0 && ctr < (uint64_t)RTAB_N) {
-        uint32_t lo, hi;
-        asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(lo), "=r"(hi) : "r"(rtab.saddr + (uint32_t)ctr * 8u));
-        inner = (uint64_t)lo | ((uint64_t)hi << 32);
-    } else {
-        inner = mix64(ctr + 0x9E3779B97F4A7C15ull);
-    }
-    return mix64(key ^ inner);
+    if (rtab.saddr != 0 && ctr < (uint64_t)RTAB_N) return rand64_tab(rtab, key, (uint32_t)ctr);
+    return mix64(key ^ mix64(ctr + 0x9E3779B97F4A7C15ull));
 }
 
 // ---- state access -------------------------------------------------------------------------
@@ -478,27 +477,37 @@ __device__ __forceinline__ uint32_t shl_clamped(uint32_t v, uint32_t n) {   // v
     asm("shl.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
     return r;
 }
+// draw j (0..2) of a pile from a bag of `total` > 0 tiles, the bag as two 32-bit halves (types 0..3 | 4,5): the
+// cumulative counts and the decrement stay 32-bit operations.  Returns the tile's increment of the pile code.
+__device__ __forceinline__ uint32_t draw_tile(uint32_t& lo, uint32_t& hi, uint32_t total, uint64_t z, int j) {
+    uint32_t x = (uint32_t)(z >> (21 * j)) & 0x1FFFFFu;
+    uint32_t r = (x * total) >> 21;                                  // 21+7 bits < 32
+    uint32_t clo = lo * 0x01010101u;                                 // byte k = sum of bytes 0..k (totals <= 255: no carries)
+    uint32_t c4 = (clo >> 24) + (hi & 0xFFu);
+    uint32_t rr = r * 0x01010101u;
+    int t = __popc(__vcmpleu4(clo, rr) & 0x01010101u) + (c4 <= r ? 1 : 0);
+    lo -= shl_clamped(1u, 8u * (uint32_t)t);                         // t >= 4: shifted out
+    hi -= shl_clamped(1u, 8u * (uint32_t)t - 32u);                   // t < 4: the count wraps to >= 32, shifted out
+    return 1u << (2 * t);
+}
 __device__ __forceinline__ uint32_t draw_pile(uint64_t& bag, uint64_t z) {
-    // the bag as two 32-bit halves (types 0..3 | 4,5): the cumulative counts and the decrement stay 32-bit operations
     uint32_t lo = (uint32_t)bag, hi = (uint32_t)(bag >> 32), code = 0;
     int total = bag_total(bag);
 #pragma unroll
     for (int j = 0; j < 3; j++) {
         if (total > 0) {
-            uint32_t x = (uint32_t)(z >> (21 * j)) & 0x1FFFFFu;
-            uint32_t r = (x * (uint32_t)total) >> 21;               // 21+7 bits < 32
-            uint32_t clo = lo * 0x01010101u;                         // byte k = sum of bytes 0..k (totals <= 255: no carries)
-            uint32_t c4 = (clo >> 24) + (hi & 0xFFu);
-            uint32_t rr = r * 0x01010101u;
-            int t = __popc(__vcmpleu4(clo, rr) & 0x01010101u) + (c4 <= r ? 1 : 0);
-            lo -= shl_clamped(1u, 8u * (uint32_t)t);                 // t >= 4: shifted out
-            hi -= shl_clamped(1u, 8u * (uint32_t)t - 32u);           // t < 4: the count wraps to >= 32, shifted out
-            code += 1u << (2 * t);
+            code += draw_tile(lo, hi, (uint32_t)total, z, j);
             total--;
         }
     }
     bag = (uint64_t)lo | ((uint64_t)hi << 32);
     return code;
+}
+// draw_pile from a bag of total >= 3 tiles: always three draws, no branch
+__device__ __forceinline__ uint32_t draw_pile3(uint32_t& lo, uint32_t& hi, uint32_t total, uint64_t z) {
+    uint32_t code = draw_tile(lo, hi, total, z, 0);                  // (three statements: each draw sees the bag the last left)
+    code += draw_tile(lo, hi, total - 1u, z, 1);
+    return code + draw_tile(lo, hi, total - 2u, z, 2);
 }
 __device__ __forceinline__ bool pile_available(uint64_t bag, uint32_t code) {
     bool ok = true;
@@ -674,6 +683,54 @@ __device__ __forceinline__ int apply_move(State& s, int a, uint32_t explicit_cod
 }
 
 // ---- one step of the uniform-random playout (fused kernel only) -------------------------------------
+// The choose (:217-223): pile a becomes the hand, the piles behind it move up.
+__device__ __forceinline__ uint32_t take_pile(Piles& pl, int a) {
+    uint32_t hand = pl.p[0];
+#pragma unroll
+    for (int j = 1; j < 5; j++) hand = (a == j) ? pl.p[j] : hand;
+#pragma unroll
+    for (int j = 0; j < 4; j++) pl.p[j] = (j >= a) ? pl.p[j + 1] : pl.p[j];
+    pl.p[4] = 0;
+    return hand;
+}
+// A placement (:145-208 for the legal set, :250-275 for the move) on the mover's planes b[0..8] with policy draw rh:
+// the tile goes on its hex and leaves the hand.  Returns the hex's bit, or 0 when no hex is legal; b and hand are then
+// unchanged.  No branch: playout_round() runs six of these in a row.
+__device__ __forceinline__ uint32_t place_random(uint32_t* b, uint32_t& hand, uint32_t rh) {
+    struct { uint32_t occ0, occ1, occ2; } t = {b[0] | b[1] | b[2], b[3] | b[4] | b[5], b[6] | b[7] | b[8]};
+    const uint32_t empty = ~t.occ0 & VALID;                            // :173
+    // Stacking only ever looks at tops below level 3: where occ2 is clear the top tile is the level-1 tile if there is one,
+    // else the level-0 tile, so the code bits of the top need two levels (tops_of() merges all three), and a height-1 top
+    // is the level-0 code itself.
+    const uint32_t T0 = b[3] | (b[0] & ~t.occ1), T1 = b[4] | (b[1] & ~t.occ1), T2 = b[5] | (b[2] & ~t.occ1);
+    const uint32_t x1 = T0 & T1 & ~T2 & ~t.occ2, x3 = ~T0 & ~T1 & T2 & ~t.occ2;                 // wood / stone top, h <= 2: :183, :186
+    const uint32_t x4 = ((b[0] & b[1] & ~b[2]) | (~b[1] & b[2])) & ~t.occ1;                     // wood, stone or building at h == 1: :190-192
+    const uint32_t m0 = (hand & 0x003) ? empty : 0, m1 = (hand & 0x00C) ? (empty | x1) : 0, m2 = (hand & 0x030) ? empty : 0;
+    const uint32_t m3 = (hand & 0x0C0) ? (empty | x3) : 0, m4 = (hand & 0x300) ? (empty | x4) : 0, m5 = (hand & 0xC00) ? empty : 0;
+    const int c0 = __popc(m0), c1 = c0 + __popc(m1), c2 = c1 + __popc(m2), c3 = c2 + __popc(m3), c4 = c3 + __popc(m4);
+    const int n = c4 + __popc(m5);
+    const int k = (int)__umulhi(rh, (uint32_t)n);
+    // the type whose cumulative count covers k: the five comparisons are monotone, each one moves (type, mask, base) on
+    int tile = 0, below = 0;
+    uint32_t m = m0;
+    if (k >= c0) { tile = 1; m = m1; below = c0; }
+    if (k >= c1) { tile = 2; m = m2; below = c1; }
+    if (k >= c2) { tile = 3; m = m3; below = c2; }
+    if (k >= c3) { tile = 4; m = m4; below = c3; }
+    if (k >= c4) { tile = 5; m = m5; below = c4; }
+    const uint32_t any = n != 0;                                      // shifts, not selects: a select here becomes a branch
+    const uint32_t bit = any << nth_set_bit(m, k - below);
+    // place the tile on level h of the hex (:257,275)
+    const uint32_t code = (uint32_t)tile + 1u;
+    const uint32_t lvl1 = t.occ0 & ~t.occ1;
+#pragma unroll
+    for (int q = 0; q < 3; q++) {
+        const uint32_t bq = (code & (1u << q)) ? bit : 0u;            // the hex in the planes of the code's set bits
+        b[q] |= bq & ~t.occ0; b[3 + q] |= bq & lvl1; b[6 + q] |= bq & t.occ1;
+    }
+    hand -= any << (2 * tile);                                        // hand.remove, :250
+    return bit;
+}
 // legal_of + random_action + apply_move for a state whose mover is player P (a template parameter: the kernel branches on the
 // player once per step, so the mover's planes are words 9P..9P+8 statically — no per-word select on the player bit and no
 // swapping of the two boards when the player changes), for a move that is legal BY CONSTRUCTION: the action is
@@ -689,14 +746,8 @@ __device__ __forceinline__ bool playout_step(State& s, const NbrLut* lut, RandTa
     if (ph == HZ_PHASE_CHOOSE) {                                      // :158, :217-223
         const int np = n_piles_of(s);
         if (np == 0) return false;
-        const int a = (int)__umulhi(rh, (uint32_t)np);
         Piles pl = piles_of(s);
-        uint32_t hand = pl.p[0];
-#pragma unroll
-        for (int j = 1; j < 5; j++) hand = (a == j) ? pl.p[j] : hand;
-#pragma unroll
-        for (int j = 0; j < 4; j++) pl.p[j] = (j >= a) ? pl.p[j + 1] : pl.p[j];
-        pl.p[4] = 0;
+        const uint32_t hand = take_pile(pl, (int)__umulhi(rh, (uint32_t)np));
         set_piles(s, pl, hand, np - 1);
         set_meta(s, (meta(s) & ~0xEu) | (HZ_PHASE_PLACE1 << 1));
         s.w[HZ_W_MOVES]++;
@@ -704,46 +755,71 @@ __device__ __forceinline__ bool playout_step(State& s, const NbrLut* lut, RandTa
     }
     if (ph > HZ_PHASE_PLACE3) return false;
     uint32_t hand = hand_of(s);
-    const uint32_t* b = &s.w[9 * P];
-    struct { uint32_t occ0, occ1, occ2; } t = {b[0] | b[1] | b[2], b[3] | b[4] | b[5], b[6] | b[7] | b[8]};
-    const uint32_t empty = ~t.occ0 & VALID;                            // :173
-    // Stacking only ever looks at tops below level 3: where occ2 is clear the top tile is the level-1 tile if there is one,
-    // else the level-0 tile, so the code bits of the top need two levels (tops_of() merges all three), and a height-1 top
-    // is the level-0 code itself.
-    const uint32_t T0 = b[3] | (b[0] & ~t.occ1), T1 = b[4] | (b[1] & ~t.occ1), T2 = b[5] | (b[2] & ~t.occ1);
-    const uint32_t x1 = T0 & T1 & ~T2 & ~t.occ2, x3 = ~T0 & ~T1 & T2 & ~t.occ2;                 // wood / stone top, h <= 2: :183, :186
-    const uint32_t x4 = ((b[0] & b[1] & ~b[2]) | (~b[1] & b[2])) & ~t.occ1;                     // wood, stone or building at h == 1: :190-192
-    const uint32_t m0 = (hand & 0x003) ? empty : 0, m1 = (hand & 0x00C) ? (empty | x1) : 0, m2 = (hand & 0x030) ? empty : 0;
-    const uint32_t m3 = (hand & 0x0C0) ? (empty | x3) : 0, m4 = (hand & 0x300) ? (empty | x4) : 0, m5 = (hand & 0xC00) ? empty : 0;
-    const int c0 = __popc(m0), c1 = c0 + __popc(m1), c2 = c1 + __popc(m2), c3 = c2 + __popc(m3), c4 = c3 + __popc(m4);
-    const int n = c4 + __popc(m5);
-    if (n == 0) return false;
-    const int k = (int)__umulhi(rh, (uint32_t)n);
-    // the type whose cumulative count covers k: the five comparisons are monotone, each one moves (type, mask, base) on
-    int tile = 0, below = 0;
-    uint32_t m = m0;
-    if (k >= c0) { tile = 1; m = m1; below = c0; }
-    if (k >= c1) { tile = 2; m = m2; below = c1; }
-    if (k >= c2) { tile = 3; m = m3; below = c2; }
-    if (k >= c3) { tile = 4; m = m4; below = c3; }
-    if (k >= c4) { tile = 5; m = m5; below = c4; }
-    const uint32_t bit = 1u << nth_set_bit(m, k - below);
-    // place the tile on level h of the hex (:257,275)
-    const uint32_t code = (uint32_t)tile + 1u;
-    const uint32_t lvl1 = t.occ0 & ~t.occ1;
-#pragma unroll
-    for (int q = 0; q < 3; q++) {
-        const uint32_t bq = (code & (1u << q)) ? bit : 0u;            // the hex in the planes of the code's set bits
-        s.w[9 * P + q] |= bq & ~t.occ0; s.w[9 * P + 3 + q] |= bq & lvl1; s.w[9 * P + 6 + q] |= bq & t.occ1;
-    }
-    hand -= 1u << (2 * tile);                                         // hand.remove, :250
+    if (!place_random(&s.w[9 * P], hand, rh)) return false;
     s.w[HZ_W_PILE4H] = (s.w[HZ_W_PILE4H] & 0xFFFFu) | (hand << 16);
     s.w[HZ_W_MOVES]++;
     if (ph != HZ_PHASE_PLACE3) {
         set_meta(s, meta(s) + 2u);                                    // phase+1, :287-290
         return true;
     }
-    end_turn<DEFER_SCORE, false>(s, P, t.occ0 | bit, hand, false, HZ_NO_DRAW, key_of(s), s.w[HZ_W_EVENT], true, lut, rtab);
+    const uint32_t occ_after = s.w[9 * P] | s.w[9 * P + 1] | s.w[9 * P + 2];
+    end_turn<DEFER_SCORE, false>(s, P, occ_after, hand, false, HZ_NO_DRAW, key_of(s), s.w[HZ_W_EVENT], true, lut, rtab);
+    return true;
+}
+
+// ---- one whole round of the uniform-random playout (fused kernel only) -------------------------------------------
+// A round is player 0's turn and then player 1's: choose a pile, place three tiles, top the piles up — 8 actions.  From
+// (player 0, CHOOSE, not ending, 5 piles) all ten random numbers of the round are known up front (8 policy draws at
+// moves+0..7, the two top-ups' pile draws at events ev, ev+1), and the round is three chains that do not wait on each
+// other: piles, hands and bag; player 0's placements on board 0; player 1's on board 1, which needs only player 1's
+// hand from the first chain.  playout_round() is one straight-line body over registers that the compiler can interleave,
+// and writes the record once; playout_step runs them one after the other with a branch on phase and player per action.
+// The straight line covers the regular round: every placement has a legal hex and each top-up draws three tiles from a
+// bag of >= 3.  Anything else returns false with s untouched, and the caller plays the round with playout_step.
+// Same draws, same result as eight playout_step<P, true> calls; the final scoring is left to the caller as there.
+__device__ __forceinline__ bool round_ready(const State& s) {
+    // the rand table covers every counter of the round (moves+7, (ev+1)*8 < RTAB_N)
+    return (meta(s) & 0x1Fu) == (0u | (HZ_PHASE_CHOOSE << 1)) && n_piles_of(s) == 5 &&
+           s.w[HZ_W_MOVES] <= (uint32_t)RTAB_N - 8u && s.w[HZ_W_EVENT] <= (uint32_t)RTAB_N / 8u - 2u;
+}
+// precondition: round_ready(s), rtab a table
+__device__ __forceinline__ bool playout_round(State& s, RandTab rtab) {
+    const uint64_t key = key_of(s), pkey = key ^ HZ_PLAYOUT_SALT;
+    const uint32_t mv = s.w[HZ_W_MOVES], ev = s.w[HZ_W_EVENT];
+    uint32_t rh[8];
+#pragma unroll
+    for (int i = 0; i < 8; i++) rh[i] = (uint32_t)(rand64_tab(rtab, pkey, mv + (uint32_t)i) >> 32);
+    const uint64_t z0 = rand64_tab(rtab, key, ev * 8u), z1 = rand64_tab(rtab, key, (ev + 1u) * 8u);
+    // piles, hands and bag: both chooses of 5 piles, both top-ups of one pile (:132-137, :217-223)
+    Piles pl = piles_of(s);
+    uint32_t lo = s.w[HZ_W_BAG0], hi = s.w[HZ_W_BAG1META] & 0xFFFFu;
+    const uint32_t total = (uint32_t)bag_total((uint64_t)lo | ((uint64_t)hi << 32));
+    uint32_t hand0 = take_pile(pl, (int)__umulhi(rh[0], 5u));
+    pl.p[4] = draw_pile3(lo, hi, total, z0);
+    uint32_t hand1 = take_pile(pl, (int)__umulhi(rh[4], 5u));
+    pl.p[4] = draw_pile3(lo, hi, total - 3u, z1);
+    // the two boards' placements, interleaved
+    uint32_t b0[9], b1[9];
+#pragma unroll
+    for (int q = 0; q < 9; q++) { b0[q] = s.w[q]; b1[q] = s.w[9 + q]; }
+    bool ok = total >= 6u;
+#pragma unroll
+    for (int i = 1; i <= 3; i++) {
+        ok &= place_random(b0, hand0, rh[i]) != 0u;
+        ok &= place_random(b1, hand1, rh[4 + i]) != 0u;
+    }
+    if (!ok) return false;
+#pragma unroll
+    for (int q = 0; q < 9; q++) { s.w[q] = b0[q]; s.w[9 + q] = b1[q]; }
+    s.w[HZ_W_BAG0] = lo;
+    s.w[HZ_W_BAG1META] = (s.w[HZ_W_BAG1META] & 0xFFFF0000u) | hi;
+    set_piles(s, pl, hand1, 5);       // player 0's leftover hand was replaced by player 1's choose
+    // end of both turns (:301-329): 2 or fewer empty hexes after either turn ends the game after player 1's; else player 0
+    // chooses next.  The bag is not empty before either top-up and both leave 5 piles, so only the boards can trigger.
+    const bool trig0 = 23 - __popc(b0[0] | b0[1] | b0[2]) <= 2, trig1 = 23 - __popc(b1[0] | b1[1] | b1[2]) <= 2;
+    set_meta(s, (trig0 || trig1) ? 1u | (HZ_PHASE_OVER << 1) | (1u << 4) : 0u | (HZ_PHASE_CHOOSE << 1));
+    s.w[HZ_W_MOVES] = mv + 8u;
+    s.w[HZ_W_EVENT] = ev + 2u;
     return true;
 }
 

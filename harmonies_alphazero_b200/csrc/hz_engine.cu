@@ -256,8 +256,10 @@ __global__ void __launch_bounds__(GWPB * 32) k_greedy(const void* states, int64_
 constexpr int PTPB = 64;   // 65,536 games -> 1024 blocks: 6.9 per SM, <2 % tail imbalance over 148 SMs
 // FROM_KEYS: the game is created in registers from its 64-bit key (k_init fused in) and only
 // (meta word, score word, actions played) leave the chip: 8 B in, 12 B out per game.
+// 7 blocks per SM hold a 65,536-game wave: the register cap of 7 x 64 threads (<= 144 per thread) leaves the round path
+// room without spills, where the compiler's own choice for __launch_bounds__(PTPB) alone was 80 registers and a spill.
 template <bool FROM_KEYS>
-__global__ void __launch_bounds__(PTPB) k_playout(void* states, int64_t n, int max_steps, uint32_t* steps,
+__global__ void __launch_bounds__(PTPB, 7) k_playout(void* states, int64_t n, int max_steps, uint32_t* steps,
                                                   unsigned long long* total_steps, const uint64_t* keys,
                                                   uint64_t seed, uint64_t first_id, uint32_t* results) {
     __shared__ NbrLut lut;
@@ -286,9 +288,17 @@ __global__ void __launch_bounds__(PTPB) k_playout(void* states, int64_t n, int m
         }
         if (player_of(s)) swap_boards(s);
 #else
-        // one branch on the player per step: fresh games move in lockstep (same player, same phase in every lane until games
-        // end), and inside a branch the mover's planes are fixed registers
+        // Whole rounds (playout_round: eight actions, both players' placements interleaved) wherever a round starts and fits
+        // in max_steps, single steps elsewhere: mid-turn starts, the tail of a max_steps slice and irregular rounds.
+        // HZ_PLAYOUT_STEPWISE: steps only (A/B).  A step branches on the player once: fresh games move in lockstep (same
+        // player, same phase in every lane until games end), and inside a branch the mover's planes are fixed registers.
         while ((int)k < max_steps && phase_of(s) != HZ_PHASE_OVER) {
+#ifndef HZ_PLAYOUT_STEPWISE
+            if ((int)k <= max_steps - 8 && round_ready(s) && playout_round(s, rtab)) {
+                k += 8;
+                continue;
+            }
+#endif
             const bool ok = player_of(s) ? playout_step<1, true>(s, &lut, rtab) : playout_step<0, true>(s, &lut, rtab);
             if (!ok) break;  // stuck position (no legal move, not over): harmonies_engine.py:205-208
             k++;
