@@ -39,6 +39,7 @@ SIGNATURES = {
     "hz_tree_select": (_i, [_vp, _f, _vp, _vp, _vp, _i, _i, _vp]),
     "hz_tree_expand_backup": (_i, [_vp, _vp, _vp, _i, _vp, _d, _vp]),
     "hz_tree_fake_eval": (_i, [_vp, _vp, _vp, _vp]),
+    "hz_tree_rollout_eval": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "hz_tree_root_policy": (_i, [_vp, _vp, _vp, _vp]),
     "hz_tree_choose": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "hz_tree_stats": (_i, [_vp, _vp, _vp, _vp, _vp]),

@@ -12,12 +12,19 @@ excludes draws (trainer.py:338-342).
 import torch
 
 from . import batched as hb
+from .selfplay import RolloutEvaluator
 from .tree import BatchedMCTS
 
 
 def _search(tree, net, states, sims, cpuct, bufs):
     board, glob, logits, value = bufs
     tree.reset(states)
+    if isinstance(net, RolloutEvaluator):
+        for _ in range(sims // tree.leaves):
+            tree.select(cpuct)
+            tree.rollout_eval(logits, value, net.rollouts)
+            tree.expand_backup(logits, value, is_logits=False)
+        return
     tiles = board.dtype == torch.uint8
     pad40 = not tiles and board.shape[1] == 40
     for _ in range(sims // tree.leaves):
@@ -34,8 +41,9 @@ GREEDY = "greedy"   # pass as either side to play the 1-ply greedy agent of eval
 
 def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cuda", seed=0, key_mode=hb.KEY_REFERENCE, leaves=1):
     """Returns dict(candidate_wins, best_wins, draws, win_rate, games).  Each side is an
-    InferenceNet on ``device`` or ``arena.GREEDY`` (run_tournament of evaluation.py:7-65:
-    AlphaZero vs the greedy agent, sides alternating by game index).  leaves > 1 switches the
+    InferenceNet on ``device``, ``arena.GREEDY`` (run_tournament of evaluation.py:7-65:
+    AlphaZero vs the greedy agent, sides alternating by game index) or a
+    ``selfplay.RolloutEvaluator`` (a network-free search of the same simulation count).  leaves > 1 switches the
     searches to the virtual-loss mode (K simulations in flight per tree): not the reference's
     visit counts any more, but a 30-game match then fills the network batch K times better."""
     dev = torch.device(device)
@@ -49,15 +57,18 @@ def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cud
         states = hb.init_states(n, device=dev, seed=seed, first_id=0 if g == 0 else num_games)   # distinct games per group
         if sims % leaves:
             raise ValueError("num_simulations must be a multiple of leaves")
-        anynet = candidate_net if candidate_net is not GREEDY else best_net
-        if anynet is GREEDY:
-            anynet = None
+        searchers = [x for x in (candidate_net, best_net) if x is not GREEDY]
+        nets = [x for x in searchers if not isinstance(x, RolloutEvaluator)]
+        anynet = nets[0] if nets else None
         tree = bufs = None
-        if anynet is not None:                                       # greedy vs greedy needs no search arena
+        if searchers:                                                # greedy vs greedy needs no search arena
             tree = BatchedMCTS(n, sims, device=dev, key_mode=key_mode, leaves=leaves)
             rows = n * leaves
-            both_tiles = all(x is GREEDY or getattr(x, "wants_tiles", False) for x in (candidate_net, best_net))
-            if both_tiles:                       # both sides evaluate from the hand-written tower's input image
+            both_tiles = all(x not in nets or getattr(x, "wants_tiles", False) for x in (candidate_net, best_net))
+            if anynet is None:                   # rollouts only: priors and values, no leaf encoding
+                bufs = (None, None, torch.zeros((rows, 143), dtype=torch.float32, device=dev),
+                        torch.zeros(rows, dtype=torch.float32, device=dev))
+            elif both_tiles:                     # every network evaluates from the hand-written tower's input image
                 bufs = anynet.leaf_buffers(rows)
             else:
                 C = 40 if hasattr(anynet, "stem40") else 38

@@ -823,6 +823,42 @@ __device__ __forceinline__ bool playout_round(State& s, RandTab rtab) {
     return true;
 }
 
+// ---- the game loop of the fused playout kernels (k_playout, k_tree_rollout_eval) ------------------------------------
+// Plays s with hz_playout's semantics until the game is over, no move is legal, or max_steps actions were applied, and
+// returns the number of actions applied.  The final scoring is deferred: a game that ended here is left at phase game_over
+// with winner None, and the caller scores it with the lanes of the block converged (partial_scores + resolve_water).
+// lut and rtab: the block's shared neighbour LUT and rand table.
+__device__ __forceinline__ uint32_t play_random(State& s, int max_steps, const NbrLut* lut, RandTab rtab) {
+    uint32_t k = 0;
+#ifdef HZ_PLAYOUT_CHECKED   // A/B: the three general calls on a mover-relative state (validation + board copy in apply_move)
+    if (player_of(s)) swap_boards(s);
+    while ((int)k < max_steps && phase_of(s) != HZ_PHASE_OVER) {
+        int a = random_action(s, legal_of<true>(s), rtab);
+        if (a < 0) break;  // stuck position (no legal move, not over): harmonies_engine.py:205-208
+        if (apply_move<true, true>(s, a, HZ_NO_DRAW, key_of(s), s.w[HZ_W_EVENT], true, lut, rtab) != HZ_MOVE_OK) break;
+        k++;
+    }
+    if (player_of(s)) swap_boards(s);
+#else
+    // Whole rounds (playout_round: eight actions, both players' placements interleaved) wherever a round starts and fits
+    // in max_steps, single steps elsewhere: mid-turn starts, the tail of a max_steps slice and irregular rounds.
+    // HZ_PLAYOUT_STEPWISE: steps only (A/B).  A step branches on the player once: fresh games move in lockstep (same
+    // player, same phase in every lane until games end), and inside a branch the mover's planes are fixed registers.
+    while ((int)k < max_steps && phase_of(s) != HZ_PHASE_OVER) {
+#ifndef HZ_PLAYOUT_STEPWISE
+        if ((int)k <= max_steps - 8 && round_ready(s) && playout_round(s, rtab)) {
+            k += 8;
+            continue;
+        }
+#endif
+        const bool ok = player_of(s) ? playout_step<1, true>(s, lut, rtab) : playout_step<0, true>(s, lut, rtab);
+        if (!ok) break;  // stuck position (no legal move, not over): harmonies_engine.py:205-208
+        k++;
+    }
+#endif
+    return k;
+}
+
 // ---- canonical keys ----------------------------------------------------------------------------
 // Leftmost-embedding normal form of one board under the reference's hash aliasing
 // (HZ_KEY_REFERENCE in harmonies_b200.h).  Alias pairs {1,6},{2,7},{3,8} (shift 5) and

@@ -278,32 +278,7 @@ __global__ void __launch_bounds__(PTPB, 7) k_playout(void* states, int64_t n, in
     if (g < n) {
         if (FROM_KEYS) init_state(s, keys ? keys[g] : rand64(seed, first_id + (uint64_t)g), rtab);
         else load_state(s, states, g);
-#ifdef HZ_PLAYOUT_CHECKED   // A/B: the three general calls on a mover-relative state (validation + board copy in apply_move)
-        if (player_of(s)) swap_boards(s);
-        while ((int)k < max_steps && phase_of(s) != HZ_PHASE_OVER) {
-            int a = random_action(s, legal_of<true>(s), rtab);
-            if (a < 0) break;  // stuck position (no legal move, not over): harmonies_engine.py:205-208
-            if (apply_move<true, true>(s, a, HZ_NO_DRAW, key_of(s), s.w[HZ_W_EVENT], true, &lut, rtab) != HZ_MOVE_OK) break;
-            k++;
-        }
-        if (player_of(s)) swap_boards(s);
-#else
-        // Whole rounds (playout_round: eight actions, both players' placements interleaved) wherever a round starts and fits
-        // in max_steps, single steps elsewhere: mid-turn starts, the tail of a max_steps slice and irregular rounds.
-        // HZ_PLAYOUT_STEPWISE: steps only (A/B).  A step branches on the player once: fresh games move in lockstep (same
-        // player, same phase in every lane until games end), and inside a branch the mover's planes are fixed registers.
-        while ((int)k < max_steps && phase_of(s) != HZ_PHASE_OVER) {
-#ifndef HZ_PLAYOUT_STEPWISE
-            if ((int)k <= max_steps - 8 && round_ready(s) && playout_round(s, rtab)) {
-                k += 8;
-                continue;
-            }
-#endif
-            const bool ok = player_of(s) ? playout_step<1, true>(s, &lut, rtab) : playout_step<0, true>(s, &lut, rtab);
-            if (!ok) break;  // stuck position (no legal move, not over): harmonies_engine.py:205-208
-            k++;
-        }
-#endif
+        k = play_random(s, max_steps, &lut, rtab);
         // final scoring deferred to here: the lanes of the warp are converged again; rivers of >= 5
         // hexes go to the block's queue and get a whole warp each (resolve_water)
         fin = phase_of(s) == HZ_PHASE_OVER && winner_code(s) == 0;

@@ -552,6 +552,85 @@ __global__ void __launch_bounds__(TTPB) k_tree_fake_eval(hz_tree T, float* polic
     }
 }
 
+// ---- rollout evaluator: leaf values from random playouts (hz_tree_rollout_eval) ------------------------------------
+// One thread per rollout: thread i*R + r plays rollout r of leaf row i with k_playout's game loop (play_random), shared
+// neighbour LUT, rand table and water queue.  With R >= 32 the lanes of a warp start from the same leaf and move in
+// lockstep; with R < 32 a warp holds 32/R leaves.  The row's outcomes are summed as integers (shuffles inside the R lanes,
+// shared memory across the block's two warps for R = 64), so the value does not depend on the order of the sum.
+// 64-thread blocks under (64, 7) for the reason given at k_playout: the register cap leaves the round path room.
+constexpr int RTPB = 64;
+constexpr int ROLLOUT_MAX_STEPS = 1000;
+__global__ void __launch_bounds__(RTPB, 7) k_tree_rollout_eval(hz_tree T, int log2r, float* policy, float* value,
+                                                               unsigned long long* total_steps) {
+    const int R = 1 << log2r;
+    const int64_t rows = (int64_t)active_trees(T) * T.leaves;
+    if ((int64_t)blockIdx.x * RTPB >= (rows << log2r)) return;      // the whole block lies past the active rows
+    __shared__ NbrLut lut;
+    __shared__ uint64_t rtab_s[RTAB_N];
+    __shared__ WaterQueue<2 * RTPB, 2 * RTPB> wq;
+    __shared__ int warp_sum[RTPB / 32];
+    build_nbr_lut(&lut);
+    build_rand_table(rtab_s);
+    const RandTab rtab = rand_table_handle(rtab_s);
+    water_queue_init(&wq);
+    __syncthreads();
+    const int64_t gid = (int64_t)blockIdx.x * RTPB + threadIdx.x, row = gid >> log2r;
+    const int r = (int)(gid & (R - 1));
+    const bool on = row < rows;
+    uint32_t k = 0;
+    int s0 = 0, s1 = 0, sigma = 0;
+    bool fin = false, leaf_over = true;
+    State s;
+    if (on) {
+        const int t = (int)(row / T.leaves), leaf = T.leaf[row];
+        HZ_BOUND(leaf, T.max_nodes, 501);
+        load_state(s, T.node_state + (size_t)t * T.max_nodes * 8, leaf);   // the row's R threads read one 128 B line
+        leaf_over = is_over(s);
+        sigma = player_of(s) ? -1 : 1;
+        {   // priors: uniform over the legal moves, the R threads of the row split the 143 entries
+            const Legal L = legal_of(s);
+            const int n = leaf_over ? 0 : legal_count(L);
+            uint32_t lw[5];
+            legal_words(L, lw);
+            const float p = n ? 1.0f / (float)n : 0.0f;
+            for (int a = r; a < HZ_ACTION_SIZE; a += R) {
+                const int i = a >> 5;   // selects, not lw[i]: a dynamic index would put lw in local memory
+                const uint32_t w = i == 0 ? lw[0] : i == 1 ? lw[1] : i == 2 ? lw[2] : i == 3 ? lw[3] : lw[4];
+                policy[row * HZ_ACTION_SIZE + a] = ((w >> (a & 31)) & 1u) ? p : 0.0f;
+            }
+        }
+        if (!leaf_over) {
+            const uint64_t base = rand64(T.search_key[t] ^ HZ_ROLLOUT_SALT, canon_hash(s, HZ_KEY_EXACT));
+            const uint64_t key = rand64(base, (uint64_t)r);
+            s.w[HZ_W_KEYLO] = (uint32_t)key;
+            s.w[HZ_W_KEYHI] = (uint32_t)(key >> 32);
+            k = play_random(s, ROLLOUT_MAX_STEPS, &lut, rtab);
+            fin = phase_of(s) == HZ_PHASE_OVER && winner_code(s) == 0;
+            if (fin) partial_scores(s, &lut, &wq, s0, s1);
+        }
+    }
+    __syncthreads();
+    resolve_water(&lut, &wq);
+    __syncthreads();
+    if (fin) store_final_scores(s, s0 + wq.extra[threadIdx.x * 2], s1 + wq.extra[threadIdx.x * 2 + 1]);
+    int sum = on && !leaf_over ? sigma * outcome_of(s) : 0;      // a stuck or capped rollout is not over: 0
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1)
+        if (o < R) sum += __shfl_xor_sync(FULL, sum, o);
+    if (R == 64) {                                                // block-uniform
+        if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = sum;
+        __syncthreads();
+        sum = warp_sum[0] + warp_sum[1];
+    }
+    if (on && r == 0) value[row] = (float)sum / (float)R;
+    if (total_steps) {
+        uint32_t steps = k;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) steps += __shfl_xor_sync(FULL, steps, o);
+        if ((threadIdx.x & 31) == 0 && steps) atomicAdd(total_steps, (unsigned long long)steps);
+    }
+}
+
 // ---- root statistics (MCTS.py:355-381) and move choice (MCTS.py:394-441) -------------------------
 __global__ void __launch_bounds__(TTPB) k_tree_root_policy(hz_tree T, int32_t* visits, float* pi) {
     int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -751,6 +830,17 @@ int hz_tree_expand_backup(hz_tree* t, const float* policy, const float* value, i
 int hz_tree_fake_eval(hz_tree* t, float* policy, float* value, void* stream) {
     if (!t || !policy || !value) return HZ_ERR_ARG;
     k_tree_fake_eval<<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value);
+    return hz_launched(1);
+}
+
+int hz_tree_rollout_eval(hz_tree* t, int rollouts, float* policy, float* value, unsigned long long* total_steps,
+                         void* stream) {
+    if (!t || !policy || !value || rollouts < 1 || rollouts > 64 || (rollouts & (rollouts - 1))) return HZ_ERR_ARG;
+    int log2r = 0;
+    while ((1 << log2r) < rollouts) log2r++;
+    int64_t threads = (int64_t)t->n_trees * t->leaves * rollouts;
+    k_tree_rollout_eval<<<(unsigned)((threads + RTPB - 1) / RTPB), RTPB, 0, (cudaStream_t)stream>>>(*t, log2r, policy, value,
+                                                                                                   total_steps);
     return hz_launched(1);
 }
 

@@ -28,6 +28,7 @@ NO_DRAW = 0xFFFF
 M64 = (1 << 64) - 1
 PLAYOUT_SALT = 0xA5A5F00DC0FFEE11
 SEARCH_SALT = 0x5EA2C47EE5A17B00   # default in-tree draw stream key: rand(state key ^ SEARCH_SALT, moves)
+ROLLOUT_SALT = 0x2011C0A75EED5A17  # rollout keys of hz_tree_rollout_eval: rand(search key ^ ROLLOUT_SALT, exact canonical hash)
 
 W_BOARD0, W_BOARD1 = 0, 9
 W_PILES01, W_PILES23, W_PILE4H = 18, 19, 20

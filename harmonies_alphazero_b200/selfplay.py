@@ -118,6 +118,25 @@ class SyntheticEvaluator:
         raise RuntimeError("SyntheticEvaluator is evaluated on the tree (hz_tree_fake_eval), not on tensors")
 
 
+class RolloutEvaluator:
+    """Network-free evaluator: every leaf is valued by ``rollouts`` random playouts on the GPU (hz_tree_rollout_eval)
+    and its priors are uniform over the legal moves.  Its strength is set by (simulations, rollouts) alone, so it is a
+    fixed opponent for arena matches and gives iteration 0 real policy and value targets.  Pass it as ``net`` (self-play)
+    or as either side of ``arena.play_match``.  rollouts: a power of two <= 64."""
+
+    dtype = torch.float32
+
+    def __init__(self, rollouts=32, device="cuda"):
+        rollouts = int(rollouts)
+        if rollouts < 1 or rollouts > 64 or rollouts & (rollouts - 1):
+            raise ValueError("rollouts must be a power of two in 1..64")
+        self.rollouts = rollouts
+        self.device = torch.device(device)
+
+    def __call__(self, board, glob, out=None):
+        raise RuntimeError("RolloutEvaluator is evaluated on the tree (hz_tree_rollout_eval), not on tensors")
+
+
 class _Group:
     """A contiguous range of slots with its own trees, static network buffers, CUDA graph and
     stream.  Two groups on two streams let one group's tree kernels (HBM/latency-bound) run
@@ -134,7 +153,11 @@ class _Group:
         rows = n * K                  # the network sees K leaves per tree and step
         dt, cl = net.dtype, owner.channels_last
         self.tiles = bool(getattr(net, "wants_tiles", False))   # leaves go straight into the hand-written tower's input image
-        if self.tiles:
+        if isinstance(net, RolloutEvaluator):                    # the leaves are never encoded
+            self.board = self.glob = None
+            self.logits = torch.zeros((rows, 143), dtype=torch.float32, device=dev)
+            self.value = torch.zeros(rows, dtype=torch.float32, device=dev)
+        elif self.tiles:
             self.board, self.glob, self.logits, self.value = net.leaf_buffers(rows)
         else:
             self.board = torch.empty((rows, 40 if owner.pad40 else 38, 5, 7), dtype=dt, device=dev,
@@ -158,8 +181,13 @@ class _Group:
         self.n_active[1:2].fill_(int(n_trees) * K)
 
     def sim_step(self):
-        """one simulation for every tree of the group: select -> network -> expand+backup"""
+        """one simulation for every tree of the group: select -> network (or rollouts) -> expand+backup"""
         o, t = self.o, self.tree
+        if isinstance(o.net, RolloutEvaluator):
+            t.select(o.cfg.cpuct)
+            t.rollout_eval(self.logits, self.value, o.net.rollouts)
+            t.expand_backup(self.logits, self.value, is_logits=False, noise=self.noise, eps=o.cfg.dirichlet_epsilon)
+            return
         t.select(o.cfg.cpuct, self.board, self.glob, dtype=o.net.dtype, channels_last=o.channels_last, pad40=o.pad40, tiles=self.tiles)
         if getattr(o.net, "tree_eval", False):
             t.fake_eval(self.logits, self.value)       # priors, not logits

@@ -97,6 +97,21 @@ class BatchedMCTS:
         with torch.cuda.device(self.device):
             _lib.check(self.lib.hz_tree_fake_eval(self.handle, _ptr(policy), _ptr(value), self._stream()), "hz_tree_fake_eval")
 
+    def rollout_eval(self, policy, value, rollouts, total_steps=None):
+        """Network-free leaf evaluation (hz_tree_rollout_eval): ``rollouts`` (a power of two <= 64) random
+        playouts per leaf row of the last ``select``; value = mean outcome for the leaf's mover, priors uniform
+        over the legal moves (probabilities: pass ``is_logits=False`` to ``expand_backup``).  total_steps: an
+        int64 device tensor with one element to which the rollout actions played are added, or None."""
+        assert policy.dtype == torch.float32 and policy.shape == (self.rows, 143) and policy.is_contiguous()
+        assert value.dtype == torch.float32 and value.numel() == self.rows and value.is_contiguous()
+        if total_steps is not None:
+            assert total_steps.dtype == torch.int64 and total_steps.numel() >= 1 and total_steps.device == self.workspace.device
+        with torch.cuda.device(self.device):
+            _lib.check(
+                self.lib.hz_tree_rollout_eval(self.handle, int(rollouts), _ptr(policy), _ptr(value), _ptr(total_steps), self._stream()),
+                "hz_tree_rollout_eval",
+            )
+
     def root_policy(self):
         visits = torch.empty((self.n, 143), dtype=torch.int32, device=self.device)
         pi = torch.empty((self.n, 143), dtype=torch.float32, device=self.device)

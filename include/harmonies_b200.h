@@ -284,6 +284,28 @@ int hz_tree_expand_backup(hz_tree *t, const float *policy, const float *value,
  * 2^-23 - 1.  Stands in for ModelManager.predict (model.py:81-110). */
 int hz_tree_fake_eval(hz_tree *t, float *policy, float *value, void *stream);
 
+/* Rollout evaluator: for every leaf row of the last hz_tree_select (rows of active trees only),
+ * R = rollouts random playouts from the leaf, R in {1,2,4,8,16,32,64} (else HZ_ERR_ARG).  A
+ * network-free evaluator with the same output contract as hz_tree_fake_eval.
+ *  keys:     leaf = the node's stored 32 words, sk = the tree's search key (hz_tree_reset);
+ *            base = rand(sk ^ HZ_ROLLOUT_SALT, canon_hash(leaf, HZ_KEY_EXACT)),
+ *            key_r = rand(base, r) for r = 0..R-1.  Rollout r is a copy of leaf with words
+ *            HZ_W_KEYLO/HI replaced by key_r (nothing else changes), played with hz_playout's
+ *            semantics (random policy, draws, round path) for at most 1,000 actions.  The keys
+ *            depend on the leaf and the search key only: a leaf that two virtual-loss rows reach
+ *            in one step gets the same value.
+ *  value:    value[row] = (float)(sigma * sum_r o_r) / (float)R, o_r in {+1,-1,0} = hz_outcome
+ *            (player 0's view) of rollout r's final state (0 if it is not over: stuck or capped),
+ *            sigma = +1 if the leaf's player to move is 0, else -1.  Exact (R is a power of two).
+ *  policy:   policy[row][a] = 1.0f / (float)n_legal for legal a, 0 otherwise: probabilities
+ *            (pass is_logits = 0 to hz_tree_expand_backup).
+ *  A leaf that is over gets no rollouts, value 0 and a zero policy row (hz_tree_expand_backup
+ *  uses its outcome).  A leaf with no legal move gets a zero policy row and value 0.
+ *  total_steps (nullable): device uint64 to which the launch adds the rollout actions played.
+ *  Rows of trees beyond the active prefix (hz_tree_set_active) are not written. */
+int hz_tree_rollout_eval(hz_tree *t, int rollouts, float *policy, float *value,
+                         unsigned long long *total_steps, void *stream);
+
 /* Root visit counts and pi = N / sum N (MCTS.py:355-381): visits [n,143] int32,
  * pi [n,143] fp32 (either nullable). */
 int hz_tree_root_policy(hz_tree *t, int32_t *visits, float *pi, void *stream);
@@ -423,6 +445,7 @@ int hz_tower_forward_heads(const void *x0_tiles, const void *const *w_tiles,
 
 #define HZ_PLAYOUT_SALT 0xA5A5F00DC0FFEE11ull
 #define HZ_SEARCH_SALT  0x5EA2C47EE5A17B00ull
+#define HZ_ROLLOUT_SALT 0x2011C0A75EED5A17ull
 
 #ifdef __cplusplus
 }
