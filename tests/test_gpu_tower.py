@@ -152,8 +152,8 @@ def test_conv_random_values_bf16_tolerance(tw):
 
 def test_fused_launch_equals_layer_by_layer(tw):
     """The persistent all-layers launch (each CTA carries its tiles through the 17 layers) must
-    reproduce the one-launch-per-layer result bit for bit — also with several tiles per CTA and
-    with more tiles per CTA than the fused launch tracks (it then falls back to per-layer launches)."""
+    reproduce the one-launch-per-layer result bit for bit — with one tile per CTA, several tiles per
+    CTA, and all ten tiles through a single CTA (the ready queue hands it every item of every layer)."""
     from harmonies_alphazero_b200 import net as hnet
 
     torch.manual_seed(2)
@@ -168,7 +168,7 @@ def test_fused_launch_equals_layer_by_layer(tw):
     want = ht.forward(b40).clone()
     ht.fused_layers = True
     try:
-        for ctas in (0, 4, 1):       # 10 tiles: one per CTA / 3 per CTA / 10 per CTA (> 8: fallback path)
+        for ctas in (0, 4, 1):       # 10 tiles: one per CTA / up to 3 per CTA / all 10 in one CTA
             ht.lib.hz_tower_set_max_ctas(ctas)
             got = ht.forward(b40).clone()
             torch.cuda.synchronize()
