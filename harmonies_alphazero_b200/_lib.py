@@ -45,10 +45,7 @@ SIGNATURES = {
     "hz_tree_stats": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "hz_tree_root_edges": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "hz_net_heads": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp]),
-    "hz_net_head_conv_t16": (_i, [_vp, _i64, _vp, _vp, _vp, _vp]),
-    "hz_net_heads_fc": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp]),
-    "hz_net_head_conv_t16_active": (_i, [_vp, _i64, _vp, _vp, _vp, _vp, _vp]),
-    "hz_net_heads_fc_active": (_i, [_vp, _vp, _i64, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp]),
+    "hz_net_heads_fc_active": (_i, [_vp, _vp, _i64, _vp, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp]),
     "hz_tower_tile_bytes": (C.c_size_t, [_i64, _i]),
     "hz_tower_set_max_ctas": (_i, [_i]),
     "hz_tower_set_debug": (_i, [_i]),
@@ -56,8 +53,6 @@ SIGNATURES = {
     "hz_tower_to_tiles": (_i, [_vp, _vp, _i64, _i, _i, _vp]),
     "hz_tower_from_tiles": (_i, [_vp, _vp, _i64, _vp]),
     "hz_tower_sched_bytes": (C.c_size_t, [_i64, _i]),
-    "hz_tower_forward": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp]),
-    "hz_tower_forward_active": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "hz_tower_forward_heads": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hz_tower_conv3x3": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _i64, _i, _vp, _vp]),
 }
@@ -85,7 +80,7 @@ def load(path=None):
     for name, (res, args) in SIGNATURES.items():
         fn = getattr(lib, name)  # AttributeError if the symbol is missing
         fn.restype, fn.argtypes = res, args
-    if lib.hz_abi_version() != 5:
+    if lib.hz_abi_version() != 6:
         raise HarmoniesLibraryError("ABI version mismatch")
     if path is None:
         _lib = lib

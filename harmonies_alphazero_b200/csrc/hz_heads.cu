@@ -14,7 +14,6 @@
 // the 1x1 convs, then thread = output unit for the FC layers with the 7 positions held as 7
 // accumulators, so each weight is read once per 7 positions (weights stay in L1/L2).
 #include <math.h>
-#include <stdlib.h>
 
 #include "hz_common.cuh"
 
@@ -215,12 +214,9 @@ __device__ __forceinline__ uint32_t pack_bf16(__nv_bfloat16 lo, __nv_bfloat16 hi
     return (uint32_t)__bfloat16_as_ushort(lo) | ((uint32_t)__bfloat16_as_ushort(hi) << 16);
 }
 
-// hc (nullable): the 1x1 head convolutions already evaluated (hz_net_head_conv_t16): [n][105] fp32 =
-// relu(conv + bias) as policy ch0 [35 cells], policy ch1 [35], value ch0 [35]; phase 1 is then a copy.
 __global__ void __launch_bounds__(FTPB, 1) k_heads_p(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ glob,
                                                      int64_t n, HeadParams P, float* __restrict__ logits,
-                                                     float* __restrict__ value, const float* __restrict__ hc,
-                                                     const int* __restrict__ n_active, int hc_tiled) {
+                                                     float* __restrict__ value) {
     extern __shared__ __align__(16) float smem[];
     float* s_wp = smem;                      // [112][143] (+ slack)
     float* s_wv = s_wp + WPN;                // [77][256]
@@ -241,15 +237,14 @@ __global__ void __launch_bounds__(FTPB, 1) k_heads_p(const __nv_bfloat16* __rest
 #pragma unroll
         for (int w = 0; w < 2; w++) {
             int ch = 32 * (ks >> 1) + 8 * q4 + 4 * (ks & 1) + 2 * w;
-            const bool live = g8 < 3 && !hc;
+            const bool live = g8 < 3;
             float w0 = live ? P.w_conv[g8 * FC + ch] : 0.0f, w1 = live ? P.w_conv[g8 * FC + ch + 1] : 0.0f;
             __nv_bfloat16 h0 = __float2bfloat16_rn(w0), h1 = __float2bfloat16_rn(w1);
             bh[ks * 2 + w] = pack_bf16(h0, h1);
             bl[ks * 2 + w] = pack_bf16(__float2bfloat16_rn(w0 - __bfloat162float(h0)), __float2bfloat16_rn(w1 - __bfloat162float(h1)));
         }
     }
-    const float bc0 = hc ? 0.0f : P.b_conv[0], bc1 = hc ? 0.0f : P.b_conv[1], bc2 = hc ? 0.0f : P.b_conv[2];
-    if (n_active) n = min(n, (int64_t)max(*n_active, 0));   // only the active prefix of the rows (hz_tree_set_active)
+    const float bc0 = P.b_conv[0], bc1 = P.b_conv[1], bc2 = P.b_conv[2];
     int64_t n_groups = (n + FG - 1) / FG;
     bool weights_pending = true;
     for (int64_t grp = blockIdx.x; grp < n_groups; grp += gridDim.x) {
@@ -257,18 +252,8 @@ __global__ void __launch_bounds__(FTPB, 1) k_heads_p(const __nv_bfloat16* __rest
         int cnt = (int)min((int64_t)FG, n - base), ncell = cnt * CELLS;
         __syncthreads();
         // ---- phase 1: 1x1 convs + ReLU (model.py:340-343,349-351)
-        if (hc) {
-            for (int i = t; i < cnt * 3 * CELLS; i += FTPB) {
-                int p = i / (3 * CELLS), j = i - 3 * CELLS * p;
-                // hc_tiled: the layout the tower's head item writes: [tile of 16 boards][filter * 35 + cell][board in tile]
-                const int64_t bd = base + p;
-                float v = hc_tiled ? hc[(bd >> 4) * (3 * CELLS * 16) + j * 16 + (bd & 15)] : hc[bd * (3 * CELLS) + j];
-                if (j < 2 * CELLS) s_pin[p * PIN + j] = v;
-                else s_vin[p * 80 + j - 2 * CELLS] = v;
-            }
-        }
         const uint4* rows = reinterpret_cast<const uint4*>(x + base * CELLS * (int64_t)FC);
-        for (int tile = warp; !hc && tile * 16 < ncell; tile += FTPB / 32) {
+        for (int tile = warp; tile * 16 < ncell; tile += FTPB / 32) {
             int r0 = tile * 16 + g8, r1 = r0 + 8;
             uint4 qa[4], qb[4];
 #pragma unroll
@@ -388,13 +373,13 @@ __global__ void __launch_bounds__(FTPB, 1) k_heads_p(const __nv_bfloat16* __rest
     }
 }
 
-// ---- FC heads on the tensor cores (the tile path's default) --------------------------------------------------
+// ---- FC heads on the tensor cores (the tile path) --------------------------------------------------
 // policy_fc (112 -> 143) and value_fc1 (77 -> 256) + value_fc2 + tanh for 32 positions per block, as mma.sync
 // m16n8k16: M = 16 output units, N = 8 positions, K = 16 inputs.  Weights AND inputs are split into bf16 high + low
 // parts and three products are accumulated in fp32 (hi*hi + hi*lo + lo*hi: 2^-16 relative, fp32-weight accuracy).
 // A warp owns output-unit tiles; it reads its weight fragments straight from global memory (L2) into registers ONCE
 // and reuses them for the block's four position tiles, so the 143 KB of weights are never staged in shared memory and
-// there is a single block barrier before the arithmetic (the FMA kernel above spent most of its 21 us at barriers).
+// there is a single block barrier before the arithmetic (the FMA kernel above, measured on this path, spent most of its 21 us at barriers).
 constexpr int MB = 32;                        // positions per block
 constexpr int MT_POL = 9, MT_VAL = 16;        // 16-unit tiles: 144 >= 143 policy logits, 256 hidden units
 constexpr int KS_POL = 7, KS_VAL = 5;         // 16-input steps: 112, 80 >= 77
@@ -406,14 +391,15 @@ __device__ __forceinline__ void split_bf16(float v, __nv_bfloat16& hi, __nv_bflo
 }
 __global__ void __launch_bounds__(MTPB, 1) k_heads_fc_mma(const float* __restrict__ hc, const __nv_bfloat16* __restrict__ glob, int64_t n,
                                                           HeadParams P, float* __restrict__ logits, float* __restrict__ value,
-                                                          const int* __restrict__ n_active, int hc_tiled) {
+                                                          const int* __restrict__ n_active) {
     __shared__ __align__(16) __nv_bfloat16 s_ph[MB][SP], s_pl[MB][SP], s_vh[MB][SV], s_vl[MB][SV];
     __shared__ float s_part[MT_VAL][MB];       // value_fc2 partial sums per unit tile: summed in a fixed order (bit-reproducible)
     if (n_active) n = min(n, (int64_t)max(*n_active, 0));
     const int64_t base = (int64_t)blockIdx.x * MB;
     if (base >= n) return;
     const int cnt = (int)min((int64_t)MB, n - base), t = threadIdx.x;
-    auto hc_at = [&](int64_t bd, int j) { return hc_tiled ? hc[(bd >> 4) * (3 * CELLS * 16) + j * 16 + (bd & 15)] : hc[bd * (3 * CELLS) + j]; };
+    // hc: what the tower's head item writes, [tile of 16 boards][filter * 35 + cell][board in tile]
+    auto hc_at = [&](int64_t bd, int j) { return hc[(bd >> 4) * (3 * CELLS * 16) + j * 16 + (bd & 15)]; };
     // inputs (model.py:343-346,351-352): policy = [conv ch0 | conv ch1 | global], value = [conv ch2 | global], as bf16 hi + lo
     for (int i = t; i < MB * PIN; i += MTPB) {
         const int p = i / PIN, j = i - PIN * p;
@@ -504,98 +490,9 @@ __global__ void __launch_bounds__(MTPB, 1) k_heads_fc_mma(const float* __restric
     }
 }
 
-// ---- 1x1 head convolutions on the tower's T16 tiles (include/harmonies_b200.h) --------------------
-// One block per 16-board tile, all 256 tiles of a 4,096-leaf step resident at once (two blocks per SM).
-// Thread = (8 consecutive positions, one quarter of the channels): a 16-byte load is 8 positions of one
-// channel, so the loads need no transpose; a thread keeps 16 of them in flight (the kernel is a 37 MB
-// read: latency, not arithmetic); the four channel quarters of a position group are adjacent lanes and
-// meet by two shuffles.  fp32 weights and sums.
-constexpr int HCT = 288;                  // 70 position groups x 4 channel quarters = 280 working threads
-__global__ void __launch_bounds__(HCT, 2) k_head_conv_t16(const uint8_t* __restrict__ tiles, int64_t n, const float* __restrict__ w_conv,
-                                                          const float* __restrict__ b_conv, float* __restrict__ hc,
-                                                          const int* __restrict__ n_active) {
-    __shared__ float s_w[3 * 128];
-    const int t = threadIdx.x;
-    for (int i = t; i < 3 * 128; i += HCT) s_w[i] = w_conv[i];
-    __syncthreads();
-    if (n_active) n = min(n, (int64_t)max(*n_active, 0));
-    if ((int64_t)blockIdx.x * 16 >= n) return;
-    const int64_t tile = blockIdx.x;
-    const uint8_t* base = tiles + tile * (size_t)(2 * 71680);
-    const int cq = t & 3, pg = min(t >> 2, 69);       // threads 280..287 shadow the last group (they never store)
-    const bool live = t < 280;
-    float acc[3][8];
-#pragma unroll
-    for (int j = 0; j < 3; j++)
-#pragma unroll
-        for (int e = 0; e < 8; e++) acc[j][e] = 0.0f;
-#pragma unroll
-    for (int half = 0; half < 2; half++) {
-        uint4 q[16];
-#pragma unroll
-        for (int ci = 0; ci < 16; ci++) {
-            const int c = cq * 32 + half * 16 + ci;
-            q[ci] = *reinterpret_cast<const uint4*>(base + (size_t)(c >> 3) * 8960 + pg * 128 + (c & 7) * 16);
-        }
-#pragma unroll
-        for (int ci = 0; ci < 16; ci++) {
-            const int c = cq * 32 + half * 16 + ci;
-            const uint32_t qw[4] = {q[ci].x, q[ci].y, q[ci].z, q[ci].w};
-            const float w0 = s_w[c], w1 = s_w[128 + c], w2 = s_w[256 + c];
-#pragma unroll
-            for (int h = 0; h < 4; h++) {
-                const float lo = __uint_as_float(qw[h] << 16), hi = __uint_as_float(qw[h] & 0xFFFF0000u);
-                acc[0][2 * h] = fmaf(w0, lo, acc[0][2 * h]); acc[0][2 * h + 1] = fmaf(w0, hi, acc[0][2 * h + 1]);
-                acc[1][2 * h] = fmaf(w1, lo, acc[1][2 * h]); acc[1][2 * h + 1] = fmaf(w1, hi, acc[1][2 * h + 1]);
-                acc[2][2 * h] = fmaf(w2, lo, acc[2][2 * h]); acc[2][2 * h + 1] = fmaf(w2, hi, acc[2][2 * h + 1]);
-            }
-        }
-    }
-    // the 4 channel quarters of a position group are lanes 4k..4k+3
-#pragma unroll
-    for (int j = 0; j < 3; j++)
-#pragma unroll
-        for (int e = 0; e < 8; e++) {
-            float v = acc[j][e];
-            v += __shfl_xor_sync(0xFFFFFFFFu, v, 1);
-            v += __shfl_xor_sync(0xFFFFFFFFu, v, 2);
-            acc[j][e] = v;
-        }
-    if (live && cq < 3) {                 // lane cq writes output channel cq of its 8 positions
-        const int cell = pg >> 1;
-        const float bias = b_conv[cq];
-#pragma unroll
-        for (int e = 0; e < 8; e++) {
-            const int64_t board = tile * 16 + (pg & 1) * 8 + e;
-            const float v = (cq == 0 ? acc[0][e] : cq == 1 ? acc[1][e] : acc[2][e]) + bias;
-            if (board < n) hc[board * (3 * CELLS) + cq * CELLS + cell] = fmaxf(v, 0.0f);
-        }
-    }
-}
-
 }  // namespace hz
 
-extern "C" int hz_net_head_conv_t16(const void* x_tiles, int64_t n, const float* w_conv, const float* b_conv, float* head_conv,
-                                    void* stream) {
-    return hz_net_head_conv_t16_active(x_tiles, n, nullptr, w_conv, b_conv, head_conv, stream);
-}
-
-extern "C" int hz_net_head_conv_t16_active(const void* x_tiles, int64_t n, const int32_t* n_active, const float* w_conv,
-                                           const float* b_conv, float* head_conv, void* stream) {
-    if (n == 0) return HZ_OK;
-    if (!x_tiles || !w_conv || !b_conv || !head_conv || n < 0 || ((uintptr_t)x_tiles & 15) || ((uintptr_t)n_active & 3)) return HZ_ERR_ARG;
-    int64_t tiles = (n + 15) / 16;
-    hz::k_head_conv_t16<<<(unsigned)tiles, hz::HCT, 0, (cudaStream_t)stream>>>((const uint8_t*)x_tiles, n, w_conv, b_conv, head_conv, n_active);
-    return hz_launched(1);
-}
-
-extern "C" int hz_net_heads_fc(const float* head_conv, const void* glob, int64_t n, int H, const float* w_pol_t, const float* b_pol,
-                               const float* w_v1_t, const float* b_v1, const float* w_v2, float b_v2, float* logits, float* value,
-                               void* stream) {
-    return hz_net_heads_fc_active(head_conv, glob, n, nullptr, 0, H, w_pol_t, b_pol, w_v1_t, b_v1, w_v2, b_v2, logits, value, stream);
-}
-
-extern "C" int hz_net_heads_fc_active(const float* head_conv, const void* glob, int64_t n, const int32_t* n_active, int hc_tiled, int H,
+extern "C" int hz_net_heads_fc_active(const float* head_conv, const void* glob, int64_t n, const int32_t* n_active, int H,
                                       const float* w_pol_t, const float* b_pol, const float* w_v1_t, const float* b_v1,
                                       const float* w_v2, float b_v2, float* logits, float* value, void* stream) {
     if (n == 0) return HZ_OK;
@@ -603,23 +500,8 @@ extern "C" int hz_net_heads_fc_active(const float* head_conv, const void* glob, 
     if (!head_conv || !glob || !w_pol_t || !b_pol || !w_v1_t || !b_v1 || !w_v2 || !logits || !value || n < 0) return HZ_ERR_ARG;
     if (H != hz::FH || (((uintptr_t)w_v1_t | (uintptr_t)w_pol_t) & 15)) return HZ_ERR_ARG;
     hz::HeadParams P{nullptr, nullptr, w_pol_t, b_pol, w_v1_t, b_v1, w_v2, b_v2, hz::FC, H};
-    static const bool use_fma = getenv("HZ_FC_FMA") != nullptr;           // A/B switch: the fp32-FMA kernel
-    if (!use_fma) {
-        hz::k_heads_fc_mma<<<(unsigned)((n + hz::MB - 1) / hz::MB), hz::MTPB, 0, (cudaStream_t)stream>>>(
-            head_conv, (const __nv_bfloat16*)glob, n, P, logits, value, n_active, hc_tiled);
-        return hz_launched(1);
-    }
-    static bool attr_set[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(hz::k_heads_p, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hz::FSMEM);
-        if (e != cudaSuccess) return hz_record_launch(0, e);
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
-    int64_t fgroups = (n + hz::FG - 1) / hz::FG;
-    int fgrid = (int)(fgroups < 148 ? fgroups : 148);
-    hz::k_heads_p<<<fgrid, hz::FTPB, hz::FSMEM, (cudaStream_t)stream>>>(nullptr, (const __nv_bfloat16*)glob, n, P, logits, value, head_conv, n_active, hc_tiled);
+    hz::k_heads_fc_mma<<<(unsigned)((n + hz::MB - 1) / hz::MB), hz::MTPB, 0, (cudaStream_t)stream>>>(
+        head_conv, (const __nv_bfloat16*)glob, n, P, logits, value, n_active);
     return hz_launched(1);
 }
 
@@ -632,8 +514,7 @@ extern "C" int hz_net_heads(const void* x, const void* glob, int64_t n, int C, i
         return HZ_ERR_ARG;
     if (n < 0 || C <= 0 || (C % 8) != 0 || H <= 0 || (H % 2) != 0 || ((uintptr_t)x & 15)) return HZ_ERR_ARG;
     hz::HeadParams P{w_conv, b_conv, w_pol_t, b_pol, w_v1_t, b_v1, w_v2, b_v2, C, H};
-    static const bool force_generic = getenv("HZ_HEADS_GENERIC") != nullptr;   // A/B switch for profiling
-    if (!force_generic && C == hz::FC && H == hz::FH && (((uintptr_t)w_v1_t | (uintptr_t)w_pol_t) & 15) == 0) {
+    if (C == hz::FC && H == hz::FH && (((uintptr_t)w_v1_t | (uintptr_t)w_pol_t) & 15) == 0) {
         static bool attr_set[64] = {};   // the opt-in shared-memory size is per function and per device
         int dev = 0;
         cudaGetDevice(&dev);
@@ -645,7 +526,7 @@ extern "C" int hz_net_heads(const void* x, const void* glob, int64_t n, int C, i
         int64_t fgroups = (n + hz::FG - 1) / hz::FG;
         int fgrid = (int)(fgroups < 148 ? fgroups : 148);
         hz::k_heads_p<<<fgrid, hz::FTPB, hz::FSMEM, (cudaStream_t)stream>>>((const __nv_bfloat16*)x, (const __nv_bfloat16*)glob,
-                                                                            n, P, logits, value, nullptr, nullptr, 0);
+                                                                            n, P, logits, value);
         return hz_launched(1);
     }
     size_t smem = sizeof(float) * (size_t)(3 * C + hz::HP * hz::PIN + hz::HP * 80 + hz::HP * 8);

@@ -31,13 +31,11 @@
 //     complete and drained before pass 1 starts; pass 1 runs dy = -1, 0, +1, so row 4 (no dy = +1)
 //     is drained before the next tile's row 0 needs the unit.  The epilogue of one row therefore
 //     always overlaps the MMAs of the others.
-//   * hz_tower_forward*: clusters of two CTAs take pairs of neighbouring tiles of one layer and share the weight
+//   * hz_tower_forward_heads: clusters of two CTAs take pairs of neighbouring tiles of one layer and share the weight
 //     stream: each CTA loads half of every stage and multicasts it to both (cluster mode, see Params::pair).
 //   * warp roles: 0 = weight producer, 1 and 12 = MMA issuers (alternating weight stages), 2 =
 //     activation producer, 3 = TMEM allocator + work scheduler, 4..11 = epilogue (bias + residual +
 //     ReLU + bf16, thread = output channel).
-#include <stdlib.h>
-
 #include "hz_common.cuh"
 #include "hz_sm100.cuh"
 
@@ -70,31 +68,12 @@ constexpr int B_WFULL = 0, B_WEMPTY = NSTAGE, B_AFULL = 2 * NSTAGE, B_AEMPTY = 2
 //
 // A tile's five board rows do not fit the four accumulator units at once, so a work item is a sequence of
 // SEGMENTS, each a list of taps applied to a range of rows, run per channel half (segment-outer, half-inner):
-//   HZ_TOWER_SPLIT41 = 0 (default), rows {0,1,2} + {3,4}, 9 taps each:
-//     seg 0: rows 0..2, dy = +1, 0, -1  -> row 0 (no dy = -1 tap) completes after two thirds of the segment
-//     seg 1: rows 3..4, dy = -1, 0, +1  -> row 4 (no dy = +1 tap) completes after two thirds of the segment
-//     so the unit rows 0 and 4 share is always drained before its next tenant arrives.
-//   HZ_TOWER_SPLIT41 = 1, rows {0,1,2,3} + {4}: seg 0: rows 0..3, dy = 0, +1 (6 taps); seg 1: rows 0..3, dy = -1 (3 taps);
-//     seg 2: row 4, dy = -1, 0 (6 taps).  30 weight stages per item instead of 36 and 3-4 rows per weight tile in segments
-//     0/1 (tensor-pipe bound: 830 / 640 cycles per stage in the role timeline), but the single-row segment's stages are
-//     4 MMAs (~210 tensor cycles) against a weight ring that delivers one 16 KB stage per >= 400 cycles (5 stages in flight,
-//     ~2,000 cycles from issue to arrival under load): measured 415-420 us against 394 us for the default.
-#ifndef HZ_TOWER_SPLIT41
-#define HZ_TOWER_SPLIT41 0
-#endif
-#if HZ_TOWER_SPLIT41
-constexpr int NSEG = 3;
-__host__ __device__ constexpr int seg_nt(int seg) { return seg == 1 ? 3 : 6; }
-__host__ __device__ constexpr int seg_r0(int seg) { return seg == 2 ? 4 : 0; }
-__host__ __device__ constexpr int seg_r1(int seg) { return seg == 2 ? 5 : 4; }
-__host__ __device__ constexpr int tap_at(int seg, int ti) {
-    constexpr int O[3][6] = {{4, 3, 5, 7, 6, 8}, {1, 0, 2, 0, 0, 0}, {1, 0, 2, 4, 3, 5}};
-    return O[seg][ti];
-}
-__constant__ int8_t SEG_NT[3] = {6, 3, 6};
-__constant__ int8_t SEG_TAPS[3][9] = {{4, 3, 5, 7, 6, 8, 0, 0, 0}, {1, 0, 2, 0, 0, 0, 0, 0, 0}, {1, 0, 2, 4, 3, 5, 0, 0, 0}};
-__constant__ int8_t EPI_ORDER[5] = {0, 1, 2, 3, 4};  // order in which the row accumulators complete
-#else
+// rows {0,1,2} + {3,4}, 9 taps each:
+//   seg 0: rows 0..2, dy = +1, 0, -1  -> row 0 (no dy = -1 tap) completes after two thirds of the segment
+//   seg 1: rows 3..4, dy = -1, 0, +1  -> row 4 (no dy = +1 tap) completes after two thirds of the segment
+//   so the unit rows 0 and 4 share is always drained before its next tenant arrives.
+// (A 4 + 1 split needs 30 weight stages per item instead of 36, but the single-row segment's stages are 4 MMAs (~210
+// tensor cycles) against a weight ring that delivers one 16 KB stage per >= 400 cycles: measured 415-420 us against 394.)
 constexpr int NSEG = 2;
 __host__ __device__ constexpr int seg_nt(int) { return 9; }
 __host__ __device__ constexpr int seg_r0(int seg) { return seg ? 3 : 0; }
@@ -103,10 +82,8 @@ __host__ __device__ constexpr int tap_at(int seg, int ti) {
     constexpr int O[2][9] = {{7, 6, 8, 4, 3, 5, 1, 0, 2}, {1, 0, 2, 4, 3, 5, 7, 6, 8}};
     return O[seg][ti];
 }
-__constant__ int8_t SEG_NT[3] = {9, 9, 0};
-__constant__ int8_t SEG_TAPS[3][9] = {{7, 6, 8, 4, 3, 5, 1, 0, 2}, {1, 0, 2, 4, 3, 5, 7, 6, 8}, {0, 0, 0, 0, 0, 0, 0, 0, 0}};
+__constant__ int8_t SEG_TAPS[2][9] = {{7, 6, 8, 4, 3, 5, 1, 0, 2}, {1, 0, 2, 4, 3, 5, 7, 6, 8}};
 __constant__ int8_t EPI_ORDER[5] = {0, 1, 2, 4, 3};  // order in which the row accumulators complete
-#endif
 // does stage (seg, ti) multiply into board row r?  (rows of the segment whose source row r + dy is on the board)
 __host__ __device__ constexpr bool touches(int seg, int ti, int r) {
     const int dy = tap_at(seg, ti) / 3 - 1;
@@ -160,12 +137,12 @@ struct Params {
     uint8_t* buf[4];       // activation tile buffers (T16; a kmajor layer's input buffer is T16K with one half)
     Layer layers[MAX_LAYERS];
     int n_layers, n_tiles;
-    unsigned int* sched;   // ready queue (see hz_tower_forward): [0] head, [1] tail, [2 + item] completion count, [2 + n_items + slot] queue
-    int dbg;               // profiling only (hz_tower_set_debug): 1 skip MMAs, 2 skip epilogue memory traffic, 4 skip weight copies, 8 skip activation copies, 32 single MMA issuer
+    unsigned int* sched;   // ready queue (see hz_tower_forward_heads): [0] head, [1] tail, [2 + item] completion count, [2 + n_items + slot] queue
+    int dbg;               // profiling only (hz_tower_set_debug): 1 skip MMAs, 2 skip epilogue memory traffic, 4 skip weight copies, 8 skip activation copies
     unsigned int* fault;
     unsigned long long* trace;   // profiling only (hz_tower_set_trace): SM-clock timestamps of CTA 0's roles
     const int* n_active;         // device word (nullable): only the tiles that hold boards 0..*n_active-1 are computed
-    // cluster mode (hz_tower_forward*, clusters of `pair` = 2 or 4 CTAs; 0 = off): a work item is a group of neighbouring tiles
+    // cluster mode (hz_tower_forward_heads, clusters of `pair` = 2 CTAs; 0 = off): a work item is a group of neighbouring tiles
     // of one layer, one tile per CTA, so all CTAs of the cluster stream the same weights: each loads its share of every weight
     // stage and multicasts it to all of them (the weights are 57 % of what a launch pulls through L2).  mailbox: [cluster][64]
     // words through which CTA 0 of a cluster tells the others which item it drew.
@@ -229,29 +206,6 @@ __device__ __forceinline__ uint32_t pack_bf16x2_relu(float lo, float hi) {
     return d;
 }
 
-// A-operand collector hints (csrc/hz_sm100.cuh): compile-time A/B switch, -DHZ_TOWER_COLLECTOR=0 to disable
-#ifndef HZ_TOWER_KUNROLL
-#define HZ_TOWER_KUNROLL 0      // 1: unroll the k-steps of a stage as well (A/B switch)
-#endif
-#if HZ_TOWER_KUNROLL
-#define HZ_TOWER_K_PRAGMA _Pragma("unroll")
-#else
-#define HZ_TOWER_K_PRAGMA _Pragma("unroll 1")
-#endif
-// stages per issuer turn in pass 0 / pass 1 (see StageLoop).  Measured (tower of 4,096 boards): 1/1 394 us, 1/2 406,
-// 1/3 412, 2/2 416, 3/3 420: what the second issuer buys is a warp that already waits for the NEXT stage's weights,
-// and longer turns give that up
-#ifndef HZ_TOWER_TURN_P0
-#define HZ_TOWER_TURN_P0 1
-#endif
-#ifndef HZ_TOWER_TURN_P1
-#define HZ_TOWER_TURN_P1 1
-#endif
-#ifndef HZ_TOWER_COLLECTOR
-#define HZ_TOWER_COLLECTOR 1
-#endif
-
-
 // ---- MMA issue, fully unrolled -------------------------------------------------------------------
 // One thread issues ~312 MMAs of ~50 tensor-core cycles each per tile, so the issue path has to be
 // a handful of instructions per MMA: the whole warp runs the (warp-uniform) control flow, taps /
@@ -283,7 +237,7 @@ __device__ __forceinline__ void issue_stage(uint32_t a_lo, uint32_t b_lo, uint32
     // profiles/tower_trace.py: 2-14 thousand cycles at the first stage of pass 1 of every work item; tower 435 -> 400 us).
     // Taps and rows stay compile-time: run-time loops over them were measured slower (450-470 us; the set-up between the
     // hand-over and the first MMA is what the tensor pipe waits for)
-    HZ_TOWER_K_PRAGMA
+#pragma unroll 1
     for (int k = K0; k < K1; k++) {
         const uint64_t da = desc64(a_lo + (uint32_t)(k * 2), DESC_HI_SW128);
 #pragma unroll
@@ -295,7 +249,7 @@ __device__ __forceinline__ void issue_stage(uint32_t a_lo, uint32_t b_lo, uint32
             const uint64_t db = desc64(b_lo + boff, KMAJOR ? DESC_HI_SW128 : DESC_HI_T16);
             const uint32_t acc = (k == 0 && first_touch(PASS, TI, r)) ? acc_first : 1u;
             // the rows share the weight tile: it is read from shared memory for the first one only
-            if (rb - ra == 1 || !HZ_TOWER_COLLECTOR) umma_bf16_coll<COLL_DISCARD>(d, da, db, idesc, acc);
+            if (rb - ra == 1) umma_bf16_coll<COLL_DISCARD>(d, da, db, idesc, acc);
             else if (r == ra) umma_bf16_coll<COLL_FILL>(d, da, db, idesc, acc);
             else if (r == rb - 1) umma_bf16_coll<COLL_LASTUSE>(d, da, db, idesc, acc);
             else umma_bf16_coll<COLL_USE>(d, da, db, idesc, acc);
@@ -309,7 +263,8 @@ __device__ __forceinline__ void issue_stage(uint32_t a_lo, uint32_t b_lo, uint32
 // stage s+1 while warp A's MMAs of stage s execute, and starts issuing the moment A hands over (named barrier;
 // the hand-over comes after A's last MMA of the stage, so the A-operand collector groups never interleave).
 // tcgen05 operations of one CTA execute in issue order, so accumulation order and the commits' coverage are
-// those of the single-issuer sequence.
+// those of the single-issuer sequence.  Each turn is one stage: what the second issuer buys is a warp that already
+// waits for the NEXT stage's weights, and longer turns give that up (2 stages per turn: 416 us against 394).
 __device__ __forceinline__ void named_bar_sync(int id) { asm volatile("bar.sync %0, 64;" ::"r"(id) : "memory"); }
 __device__ __forceinline__ void named_bar_arrive(int id) { asm volatile("bar.arrive %0, 64;" ::"r"(id) : "memory"); }
 
@@ -320,13 +275,7 @@ struct StageLoop {
     static __device__ __forceinline__ void run(Ctx& c, int kh, int it, bool last_kh) {
         constexpr int NT = seg_nt(PASS);
         constexpr int r0 = seg_r0(PASS), r1 = seg_r1(PASS);
-        // a TURN = the consecutive stages one issuer runs between two hand-overs (HZ_TOWER_TURN_P0 / _P1 stages of the pass,
-        // counted across its channel halves; the pass's last stage always ends a turn)
-        constexpr int T = PASS ? HZ_TOWER_TURN_P1 : HZ_TOWER_TURN_P0;   // (segment 0 / later segments)
-        const int idx = kh * NT + TI;
-        const bool first_in_turn = T == 1 || idx % T == 0, last_in_turn = T == 1 || idx % T == T - 1 || (last_kh && TI == NT - 1);
-        const bool mine = !c.dual || ((c.nturn & 1) == c.parity);
-        if (mine) {
+        if ((c.nstage & 1) == c.parity) {
             HZ_CTRACE(16 + 3 * c.nstage);
             mbar_wait(c.bar0 + 8u * (B_WFULL + c.stage), c.ph, c.fault, 0x400 + c.stage);
             if (kh == 0) {   // first touch of a row's accumulator for this tile: the unit's previous tenant must be drained
@@ -339,7 +288,7 @@ struct StageLoop {
             const uint32_t a_lo = DESC_LO_SW128 | ((c.sW + c.stage * W_BYTES) >> 4);
             const uint32_t b_lo = (KMAJOR ? DESC_LO_SW128 : DESC_LO_T16) | ((c.sX + (uint32_t)kh * KH_BYTES) >> 4);
             const uint32_t acc0 = kh == 0 ? 0u : 1u;
-            if (c.dual && first_in_turn && c.nturn > 0) named_bar_sync(c.parity ? 1 : 2);   // the other issuer has handed over
+            if (c.nstage > 0) named_bar_sync(c.parity ? 1 : 2);   // the other issuer has handed over
             tc_fence_after();
             HZ_CTRACE(16 + 3 * c.nstage + 1);
             // (handing over BEFORE the last k-step, with that step issued without collector hints, was measured: the
@@ -347,7 +296,7 @@ struct StageLoop {
             // the last MMA; the commits, which only track this thread's own MMAs, come after it)
             if (lead && !(c.dbg & 1)) issue_stage<KMAJOR, PASS, TI, 0, 4>(a_lo, b_lo, c.tbase, acc0);
             __syncwarp();
-            if (c.dual && last_in_turn) named_bar_arrive(c.parity ? 2 : 1);
+            named_bar_arrive(c.parity ? 2 : 1);
             if (lead) {
                 // frees the weight stage when these MMAs have read it (cluster mode: in every CTA of the cluster; the multicast
                 // form with a mask of 1 in a launch without clusters was tried to save the branch: it faults)
@@ -364,7 +313,6 @@ struct StageLoop {
             HZ_CTRACE(16 + 3 * c.nstage + 2);
         }
         c.nstage++;
-        if (last_in_turn) c.nturn++;
         if (++c.stage == NSTAGE) { c.stage = 0; c.ph ^= 1; }
         if constexpr (TI < NT - 1) StageLoop<KMAJOR, PASS, TI + 1>::run(c, kh, it, last_kh);
     }
@@ -376,8 +324,7 @@ struct HeadStage {
     template <class Ctx>
     static __device__ __forceinline__ void run(Ctx& c, int kh, int it, bool last_kh) {
         constexpr int r0 = HSEG ? 3 : 0, r1 = HSEG ? 5 : 3;
-        const bool mine = !c.dual || ((c.nturn & 1) == c.parity);
-        if (mine) {
+        if ((c.nstage & 1) == c.parity) {
             mbar_wait(c.bar0 + 8u * (B_WFULL + c.stage), c.ph, c.fault, 0x400 + c.stage);
             if (kh == 0) {
 #pragma unroll
@@ -387,7 +334,7 @@ struct HeadStage {
             const uint32_t a_lo = DESC_LO_SW128 | ((c.sW + c.stage * W_BYTES) >> 4);
             const uint32_t b_lo = DESC_LO_T16 | ((c.sX + (uint32_t)kh * KH_BYTES) >> 4);
             const uint32_t acc0 = kh == 0 ? 0u : 1u;
-            if (c.dual && c.nturn > 0) named_bar_sync(c.parity ? 1 : 2);
+            if (c.nstage > 0) named_bar_sync(c.parity ? 1 : 2);
             tc_fence_after();
             if (lead && !(c.dbg & 1)) {
                 constexpr uint32_t idesc = idesc_bf16_f32(128, 112) | (1u << 16);
@@ -400,15 +347,14 @@ struct HeadStage {
                         const uint32_t d = c.tbase + (uint32_t)(unit_of(r) * UNIT_COLS);
                         const uint64_t db = desc64(b_lo + boff, DESC_HI_T16);
                         const uint32_t acc = k == 0 ? acc0 : 1u;
-                        if (!HZ_TOWER_COLLECTOR) umma_bf16_coll<COLL_DISCARD>(d, da, db, idesc, acc);
-                        else if (r == r0) umma_bf16_coll<COLL_FILL>(d, da, db, idesc, acc);
+                        if (r == r0) umma_bf16_coll<COLL_FILL>(d, da, db, idesc, acc);
                         else if (r == r1 - 1) umma_bf16_coll<COLL_LASTUSE>(d, da, db, idesc, acc);
                         else umma_bf16_coll<COLL_USE>(d, da, db, idesc, acc);
                     }
                 }
             }
             __syncwarp();
-            if (c.dual) named_bar_arrive(c.parity ? 2 : 1);
+            named_bar_arrive(c.parity ? 2 : 1);
             if (lead) {
                 if (c.pair) umma_commit_mc(c.bar0 + 8u * (B_WEMPTY + c.stage), c.cmask);
                 else umma_commit(c.bar0 + 8u * (B_WEMPTY + c.stage));
@@ -421,7 +367,6 @@ struct HeadStage {
             __syncwarp();
         }
         c.nstage++;
-        c.nturn++;
         if (++c.stage == NSTAGE) { c.stage = 0; c.ph ^= 1; }
     }
 };
@@ -431,10 +376,8 @@ struct IssueCtx {
     unsigned int* fault;
     int dbg;
     unsigned long long* trace;   // null unless CTA 0 is being traced
-    int nstage;                  // running stage count of the CTA (trace index)
-    int nturn;                   // running turn count of the CTA
-    int parity;                  // this warp issues the turns with nturn % 2 == parity
-    bool dual;                   // two issuer warps (false: this warp issues everything)
+    int nstage;                  // running stage count of the CTA (turn and trace index)
+    int parity;                  // this warp issues the stages with nstage % 2 == parity
     bool pair;                   // cluster mode: weight stages are shared with the other CTAs of the cluster
     uint16_t cmask;              // ... their mask
 };
@@ -482,8 +425,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tower(const __grid_constant__ P
         for (int i = 0; i < NSTAGE; i++) { mbar_init(bar(B_WFULL + i), 1); mbar_init(bar(B_WEMPTY + i), P.pair ? P.pair : 1); }
         for (int i = 0; i < 2; i++) { mbar_init(bar(B_AFULL + i), 1); mbar_init(bar(B_AEMPTY + i), 1); }
         for (int i = 0; i < NUNIT; i++) { mbar_init(bar(B_TFULL + i), 1); mbar_init(bar(B_TEMPTY + i), 8); }
-        mbar_init(bar(B_DONE), (P.dbg & 32) ? 1 : 2);
-        for (int i = 0; i < 2; i++) { mbar_init(bar(B_QFULL + i), 1); mbar_init(bar(B_QEMPTY + i), (P.dbg & 32) ? N_CONSUMERS - 1 : N_CONSUMERS); }
+        mbar_init(bar(B_DONE), 2);
+        for (int i = 0; i < 2; i++) { mbar_init(bar(B_QFULL + i), 1); mbar_init(bar(B_QEMPTY + i), N_CONSUMERS); }
         mbar_init_fence();
     }
     if (warp == 3) tmem_alloc(smem_u32(tmem_slot), 512);
@@ -557,7 +500,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tower(const __grid_constant__ P
                 const int nseg = L.head ? 2 : NSEG;
                 for (int seg = 0; seg < nseg; seg++)
                     for (int kh = 0; kh < nkh; kh++)
-                        for (int ti = 0; ti < (L.head ? 1 : SEG_NT[seg]); ti++, ns++) {
+                        for (int ti = 0; ti < (L.head ? 1 : seg_nt(seg)); ti++, ns++) {
                             int tap = L.head ? 0 : SEG_TAPS[seg][ti];
                             mbar_wait(bar(B_WEMPTY + stage), ph ^ 1, P.fault, 0x100 + stage);
                             if (ns < 600) { HZ_TRACE(2000 + ns); }
@@ -605,52 +548,41 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_tower(const __grid_constant__ P
         }
     } else if (warp == 1 || warp == 12) {
         // ---- MMA issuers: the whole warp runs the loop, one elected lane issues its stages ----
-        const bool dual = !(P.dbg & 32);
-        if (warp == 12 && !dual) {
-            // single-issuer mode (profiling A/B): nothing to do
-        } else {
-            IssueCtx c{sBar, sW, sX, tbase, 0u, 0u, P.fault, P.dbg, (blockIdx.x == 0 && lane == 0) ? P.trace : nullptr, 0, 0, warp == 12 ? 1 : 0, dual, P.pair != 0, (uint16_t)((1u << (P.pair ? P.pair : 1)) - 1u)};
-            uint32_t cnt0 = 0, cnt1 = 0;
-            int wi = 0, k = 0;                 // wi: work items done (phase of the accumulator units)
-            for (;; wi++) {
-                int item;
-                HZ_NEXT_ITEM(k, item, true);
-                if (item < 0) break;
-                const Layer& L = P.layers[item / n_units];
-                const int nkh = L.nkh;
-                const bool kmajor = L.kmajor != 0;
-                if (L.head) {
-                    for (int kh = 0; kh < nkh; kh++) {
-                        mbar_wait(bar(B_AFULL + kh), (kh ? cnt1 : cnt0) & 1u, P.fault, 0x300 + kh);
-                        if (kh) cnt1++; else cnt0++;
-                        HeadStage<0>::run(c, kh, wi, kh == nkh - 1);
-                    }
-                    for (int kh = 0; kh < nkh; kh++) HeadStage<1>::run(c, kh, wi, kh == nkh - 1);
-                    continue;
-                }
+        IssueCtx c{sBar, sW, sX, tbase, 0u, 0u, P.fault, P.dbg, (blockIdx.x == 0 && lane == 0) ? P.trace : nullptr, 0, warp == 12 ? 1 : 0, P.pair != 0, (uint16_t)((1u << (P.pair ? P.pair : 1)) - 1u)};
+        uint32_t cnt0 = 0, cnt1 = 0;
+        int wi = 0, k = 0;                 // wi: work items done (phase of the accumulator units)
+        for (;; wi++) {
+            int item;
+            HZ_NEXT_ITEM(k, item, true);
+            if (item < 0) break;
+            const Layer& L = P.layers[item / n_units];
+            const int nkh = L.nkh;
+            const bool kmajor = L.kmajor != 0;
+            if (L.head) {
                 for (int kh = 0; kh < nkh; kh++) {
-                    mbar_wait(bar(B_AFULL + kh), (kh ? cnt1 : cnt0) & 1u, P.fault, 0x300 + kh);   // both issuers observe the tile half
+                    mbar_wait(bar(B_AFULL + kh), (kh ? cnt1 : cnt0) & 1u, P.fault, 0x300 + kh);
                     if (kh) cnt1++; else cnt0++;
-                    if (kmajor) StageLoop<true, 0, 0>::run(c, kh, wi, kh == nkh - 1);
-                    else StageLoop<false, 0, 0>::run(c, kh, wi, kh == nkh - 1);
+                    HeadStage<0>::run(c, kh, wi, kh == nkh - 1);
                 }
-                for (int kh = 0; kh < nkh; kh++) {
-                    if (kmajor) StageLoop<true, 1, 0>::run(c, kh, wi, kh == nkh - 1);
-                    else StageLoop<false, 1, 0>::run(c, kh, wi, kh == nkh - 1);
-                }
-                if constexpr (NSEG > 2) {
-                    for (int kh = 0; kh < nkh; kh++) {
-                        if (kmajor) StageLoop<true, NSEG - 1, 0>::run(c, kh, wi, kh == nkh - 1);
-                        else StageLoop<false, NSEG - 1, 0>::run(c, kh, wi, kh == nkh - 1);
-                    }
-                }
+                for (int kh = 0; kh < nkh; kh++) HeadStage<1>::run(c, kh, wi, kh == nkh - 1);
+                continue;
             }
-            // the last hand-over has no taker yet: the warp whose turn would be next consumes it
-            if (dual && c.nturn > 0 && (c.nturn & 1) == c.parity) named_bar_sync(c.parity ? 1 : 2);
-            if (elect_one()) umma_commit(bar(B_DONE));
-            __syncwarp();
-            mbar_wait(bar(B_DONE), 0, P.fault, 0x600);
+            for (int kh = 0; kh < nkh; kh++) {
+                mbar_wait(bar(B_AFULL + kh), (kh ? cnt1 : cnt0) & 1u, P.fault, 0x300 + kh);   // both issuers observe the tile half
+                if (kh) cnt1++; else cnt0++;
+                if (kmajor) StageLoop<true, 0, 0>::run(c, kh, wi, kh == nkh - 1);
+                else StageLoop<false, 0, 0>::run(c, kh, wi, kh == nkh - 1);
+            }
+            for (int kh = 0; kh < nkh; kh++) {
+                if (kmajor) StageLoop<true, 1, 0>::run(c, kh, wi, kh == nkh - 1);
+                else StageLoop<false, 1, 0>::run(c, kh, wi, kh == nkh - 1);
+            }
         }
+        // the last hand-over has no taker yet: the warp whose turn would be next consumes it
+        if (c.nstage > 0 && (c.nstage & 1) == c.parity) named_bar_sync(c.parity ? 1 : 2);
+        if (elect_one()) umma_commit(bar(B_DONE));
+        __syncwarp();
+        mbar_wait(bar(B_DONE), 0, P.fault, 0x600);
     } else if (warp >= 4 && warp < 12) {
         // ---- epilogue: 8 warps.  thread = output channel c (TMEM lane); warps 4-7 take cells x = 0..3
         // of a board row, warps 8-11 cells x = 4..6.  One TMEM load = the 16 boards of a cell = 2 x 16
@@ -971,18 +903,6 @@ size_t hz_tower_sched_bytes(int64_t n_boards, int n_blocks) {
     return sizeof(unsigned int) * ((size_t)(2 + 2 * (2 + 2 * n_blocks) * tiles) + hz::tower::MAILBOX_WORDS);   // + the optional head item per tile, + the pair-mode mailboxes
 }
 
-int hz_tower_forward(const void* x0_tiles, const void* const* w_tiles, const float* const* biases, int n_blocks, void* buf_a,
-                     void* buf_b, void* buf_c, void* sched, void** out_tiles, int64_t n_boards, unsigned int* fault, void* stream) {
-    return hz_tower_forward_active(x0_tiles, w_tiles, biases, n_blocks, buf_a, buf_b, buf_c, sched, out_tiles, n_boards, nullptr, fault, stream);
-}
-
-int hz_tower_forward_active(const void* x0_tiles, const void* const* w_tiles, const float* const* biases, int n_blocks, void* buf_a,
-                            void* buf_b, void* buf_c, void* sched, void** out_tiles, int64_t n_boards, const int32_t* n_active,
-                            unsigned int* fault, void* stream) {
-    return hz_tower_forward_heads(x0_tiles, w_tiles, biases, n_blocks, buf_a, buf_b, buf_c, sched, out_tiles, n_boards, n_active, nullptr,
-                                  nullptr, nullptr, fault, stream);
-}
-
 int hz_tower_forward_heads(const void* x0_tiles, const void* const* w_tiles, const float* const* biases, int n_blocks, void* buf_a,
                            void* buf_b, void* buf_c, void* sched, void** out_tiles, int64_t n_boards, const int32_t* n_active,
                            const void* w_head_tiles, const float* b_head, float* head_conv_tiled, unsigned int* fault, void* stream) {
@@ -1027,12 +947,8 @@ int hz_tower_forward_heads(const void* x0_tiles, const void* const* w_tiles, con
     P.n_active = n_active;
     if (out_tiles) *out_tiles = P.buf[cur];
     const int n_items = P.n_layers * P.n_tiles;
-    // pair mode (clusters of two CTAs sharing the weight stream by multicast) unless switched off or there is a single tile
-    static const bool no_pair = getenv("HZ_TOWER_NO_PAIR") != nullptr;
-    static const int want_c = getenv("HZ_TOWER_CLUSTER") ? atoi(getenv("HZ_TOWER_CLUSTER")) : 2;     // CTAs per cluster: 2 (default) or 4
-    int csz = (no_pair || want_c < 2) ? 0 : (want_c >= 4 ? 4 : 2);
-    while (csz >= 2 && (P.n_tiles < csz || grid_for(P.n_tiles) < csz)) csz >>= 1;
-    P.pair = csz >= 2 ? csz : 0;
+    // pair mode (clusters of two CTAs sharing the weight stream by multicast) unless there is a single tile or a single CTA
+    P.pair = grid_for(P.n_tiles) >= 2 ? 2 : 0;
     P.mailbox = P.sched + (2 + 2 * (size_t)MAX_LAYERS_SCHED(n_blocks) * P.n_tiles);
     k_sched_init<<<(2 + 2 * n_items + 255) / 256, 256, 0, (cudaStream_t)stream>>>(P.sched, P.n_tiles, P.n_layers, n_active, P.pair, P.mailbox);
     if (P.pair) {

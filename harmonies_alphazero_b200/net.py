@@ -89,6 +89,8 @@ def _fold(conv, bn):
 class InferenceNet:
     """Folded, channels-last inference copy of an AlphaZeroNet on one device."""
 
+    heads_in_tower = True   # the tile path runs the 1x1 head convolutions inside the tower launch; bench.py reads it
+
     def __init__(self, model, device="cuda", dtype=torch.bfloat16, fused=True, fused_heads=True, tower="auto"):
         """tower: "hand" = csrc/hz_tower.cu, the hand-written sm_100a tcgen05 tower (bf16 on CUDA
         with 128 filters and <= 64 input planes; it raises for anything else, there is no silent
@@ -107,8 +109,6 @@ class InferenceNet:
             raise ValueError("the hand-written tower is bf16 on CUDA only")
         self.tower = tower
         self.hand = None
-        self._hc = {}
-        self.heads_in_tower = True     # tile path: 1x1 head convolutions as a work item of the tower launch (False: k_head_conv_t16, the A/B switch)
         self.load(model)
 
     def load(self, model):
@@ -242,22 +242,12 @@ class InferenceNet:
         lib = _lib.load()
         glob = glob.contiguous()
         na = None if n_active is None else n_active.data_ptr()
-        fold = self.heads_in_tower and self.hand.fused_layers
-        if fold:
-            # the 1x1 head convolutions run inside the tower launch, as one more work item per tile
-            self.hand.forward_tiles(x0, n, n_active=n_active, tag=tag, heads=True)
-            hc = self.hand.head_conv(n, tag)
-        else:
-            hc = self._hc.get((n, tag))     # tag: callers running concurrently on different streams keep separate scratch
-            if hc is None:
-                hc = self._hc[(n, tag)] = torch.zeros((n, 105), dtype=torch.float32, device=self.device)
-            x_ptr = self.hand.forward_tiles(x0, n, n_active=n_active, tag=tag)
+        # the 1x1 head convolutions run inside the tower launch, as one more work item per tile
+        self.hand.forward_tiles(x0, n, n_active=n_active, tag=tag, heads=True)
+        hc = self.hand.head_conv(n, tag)
         with torch.cuda.device(self.device):
             st = torch.cuda.current_stream(self.device).cuda_stream
-            if not fold:
-                _lib.check(lib.hz_net_head_conv_t16_active(x_ptr, n, na, h["w_conv"].data_ptr(), h["b_conv"].data_ptr(), hc.data_ptr(), st),
-                           "hz_net_head_conv_t16")
-            _lib.check(lib.hz_net_heads_fc_active(hc.data_ptr(), glob.data_ptr(), n, na, 1 if fold else 0, h["H"], h["w_pol_t"].data_ptr(), h["b_pol"].data_ptr(),
+            _lib.check(lib.hz_net_heads_fc_active(hc.data_ptr(), glob.data_ptr(), n, na, h["H"], h["w_pol_t"].data_ptr(), h["b_pol"].data_ptr(),
                                                   h["w_v1_t"].data_ptr(), h["b_v1"].data_ptr(), h["w_v2"].data_ptr(), h["b_v2"],
                                                   logits.data_ptr(), value.data_ptr(), st), "hz_net_heads_fc")
         return logits, value

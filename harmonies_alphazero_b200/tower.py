@@ -76,7 +76,6 @@ class HandTower:
         self.blocks = [(conv(b.conv1, b.bn1), conv(b.conv2, b.bn2)) for b in model.residual_blocks]
         self._bufs = {}
         self.fault = None     # optional host-mapped fault word (tests)
-        self.fused_layers = True   # one persistent launch for all layers (False: one launch per layer)
         layers = [self.stem] + [cv for blk in self.blocks for cv in blk]
         self._w_ptrs = (ct.c_void_p * len(layers))(*[l[0].data_ptr() for l in layers])
         self._b_ptrs = (ct.c_void_p * len(layers))(*[l[1].data_ptr() for l in layers])
@@ -142,26 +141,16 @@ class HandTower:
         n_active: int32 device tensor (one element) = boards to compute, read on the device."""
         n_pad = (n + G - 1) // G * G
         buf = self._buffers(n_pad, tag)
-        x, y, z = buf["a"], buf["b"], buf["c"]
-        if self.fused_layers:
-            res = ct.c_void_p()
-            with torch.cuda.device(self.device):
-                hw = hb = hc = None
-                if heads:
-                    hw, hb, hc = self._head_w.data_ptr(), self._head_b.data_ptr(), self.head_conv(n, tag).data_ptr()
-                _lib.check(self.lib.hz_tower_forward_heads(
-                    x0.data_ptr(), self._w_ptrs, self._b_ptrs, len(self.blocks), x.data_ptr(), y.data_ptr(), z.data_ptr(),
-                    buf["sched"].data_ptr(), ct.byref(res), n_pad, None if n_active is None else n_active.data_ptr(),
-                    hw, hb, hc, self.fault, self._stream()), "hz_tower_forward")
-            return res.value
-        if n_active is not None or heads:
-            raise ValueError("n_active / heads need the fused all-layers launch")
-        self.conv(x0, 1, self.stem, None, x, n_pad, kmajor=True)
-        for c1, c2 in self.blocks:
-            self.conv(x, 2, c1, None, y, n_pad)
-            self.conv(y, 2, c2, x, z, n_pad)
-            x, z = z, x
-        return x.data_ptr()
+        res = ct.c_void_p()
+        with torch.cuda.device(self.device):
+            hw = hb = hc = None
+            if heads:
+                hw, hb, hc = self._head_w.data_ptr(), self._head_b.data_ptr(), self.head_conv(n, tag).data_ptr()
+            _lib.check(self.lib.hz_tower_forward_heads(
+                x0.data_ptr(), self._w_ptrs, self._b_ptrs, len(self.blocks), buf["a"].data_ptr(), buf["b"].data_ptr(), buf["c"].data_ptr(),
+                buf["sched"].data_ptr(), ct.byref(res), n_pad, None if n_active is None else n_active.data_ptr(),
+                hw, hb, hc, self.fault, self._stream()), "hz_tower_forward_heads")
+        return res.value
 
     @torch.no_grad()
     def forward(self, board, out=None):

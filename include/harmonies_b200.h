@@ -69,7 +69,7 @@
 extern "C" {
 #endif
 
-#define HZ_ABI_VERSION      5
+#define HZ_ABI_VERSION      6
 #define HZ_STATE_WORDS      32
 #define HZ_STATE_BYTES      128
 #define HZ_NUM_HEXES        23
@@ -340,24 +340,13 @@ int hz_net_heads(const void *x, const void *glob, int64_t n, int C, int H, const
                  const float *w_v1_t, const float *b_v1, const float *w_v2, float b_v2,
                  float *logits, float *value, void *stream);
 
-/* The same heads when the tower output is in T16 tiles (hz_tower_forward): first the 1x1 head
- * convolutions + BatchNorm + ReLU straight from the tiles (model.py:340-343,349-351) into
- * head_conv [n,105] fp32 = policy channel 0 [35 cells], policy channel 1 [35], value channel [35]
- * (w_conv [3][128], b_conv [3] as for hz_net_heads), then the FC layers (model.py:344-355; the
- * default network's shape only: 128 filters, H = 256). */
-int hz_net_head_conv_t16(const void *x_tiles, int64_t n, const float *w_conv, const float *b_conv,
-                         float *head_conv, void *stream);
-int hz_net_heads_fc(const float *head_conv, const void *glob, int64_t n, int H, const float *w_pol_t,
-                    const float *b_pol, const float *w_v1_t, const float *b_v1, const float *w_v2,
-                    float b_v2, float *logits, float *value, void *stream);
-/* The same with the row count taken from the device: rows min(n, *n_active) are evaluated
- * (n_active NULL = n; see hz_tree_set_active).  hc_tiled != 0: head_conv is in the layout
- * hz_tower_forward_heads writes: [tile of 16 boards][filter * 35 + cell][board in tile] fp32. */
-int hz_net_head_conv_t16_active(const void *x_tiles, int64_t n, const int32_t *n_active,
-                                const float *w_conv, const float *b_conv, float *head_conv,
-                                void *stream);
+/* The FC layers of the same heads (model.py:344-355; the default network's shape only: H = 256)
+ * when the 1x1 head convolutions + BatchNorm + ReLU are already evaluated by the head item of
+ * hz_tower_forward_heads: head_conv in the layout it writes, [tile of 16 boards][filter * 35 +
+ * cell][board in tile] fp32 (filters policy 0, policy 1, value).  Rows min(n, *n_active) are
+ * evaluated (n_active: a DEVICE int32, NULL = n; see hz_tree_set_active). */
 int hz_net_heads_fc_active(const float *head_conv, const void *glob, int64_t n,
-                           const int32_t *n_active, int hc_tiled, int H, const float *w_pol_t, const float *b_pol,
+                           const int32_t *n_active, int H, const float *w_pol_t, const float *b_pol,
                            const float *w_v1_t, const float *b_v1, const float *w_v2, float b_v2,
                            float *logits, float *value, void *stream);
 
@@ -380,7 +369,7 @@ size_t hz_tower_tile_bytes(int64_t n_boards, int channel_halves);
 int hz_tower_set_max_ctas(int max_ctas);
 /* Profiling switches of hz_tower_conv3x3 (0 = normal operation; results are WRONG otherwise):
  * 1 skip the MMAs, 2 skip the epilogue's memory traffic, 4 skip the weight copies, 8 skip the
- * activation copies; 32 = one MMA issuer warp instead of two (results stay right: A/B switch).
+ * activation copies.
  * Used by profiles/tower_bench.py to attribute the kernel's time. */
 int hz_tower_set_debug(int flags);
 /* Profiling: a device buffer of 4096 uint64 (or NULL to switch off) into which CTA 0 of every
@@ -416,27 +405,18 @@ int hz_tower_conv3x3(const void *x_tiles, int in_channel_halves, int in_kmajor, 
  * the (1 + 2*n_blocks) * n_boards/16 items from a ready queue in `sched` that starts with the
  * stem items and to which the completion of (l, t) appends (l+1, t) — no grid-wide
  * synchronisation, no dependency stalls, and the load balances to within one item per CTA
- * whatever the tile count. */
-size_t hz_tower_sched_bytes(int64_t n_boards, int n_blocks);
-int hz_tower_forward(const void *x0_tiles, const void *const *w_tiles, const float *const *biases,
-                     int n_blocks, void *buf_a, void *buf_b, void *buf_c, void *sched,
-                     void **out_tiles, int64_t n_boards, unsigned int *fault, void *stream);
-
-/* hz_tower_forward over the tiles that hold boards 0..min(n_boards, *n_active)-1 only (n_active: a
- * DEVICE int32, NULL = all; see hz_tree_set_active).  The launch geometry and every address are
- * those of n_boards, so one captured CUDA graph serves every active count. */
-int hz_tower_forward_active(const void *x0_tiles, const void *const *w_tiles,
-                            const float *const *biases, int n_blocks, void *buf_a, void *buf_b,
-                            void *buf_c, void *sched, void **out_tiles, int64_t n_boards,
-                            const int32_t *n_active, unsigned int *fault, void *stream);
-
-/* hz_tower_forward_active followed, in the same launch, by the 1x1 head convolutions + BatchNorm +
- * ReLU (model.py:340-343,349-351) as one more work item per tile: a single-tap tcgen05.mma pass
+ * whatever the tile count.
+ * Only the tiles that hold boards 0..min(n_boards, *n_active)-1 are computed (n_active: a DEVICE
+ * int32, NULL = all; see hz_tree_set_active).  The launch geometry and every address are those of
+ * n_boards, so one captured CUDA graph serves every active count.
+ * After the body, in the same launch, the 1x1 head convolutions + BatchNorm + ReLU
+ * (model.py:340-343,349-351) run as one more work item per tile: a single-tap tcgen05.mma pass
  * over the tile the last block just wrote.  w_head_tiles: [2 channel halves][128 rows][128 B]
  * K-major SWIZZLE_128B bf16 with rows 0..2 = high parts of the three head filters (policy 0,
  * policy 1, value), rows 3..5 = low parts (filter = hi + lo: fp32-weight accuracy), other rows
  * zero; b_head [3] fp32; head_conv_tiled: [n_boards/16][3*35][16] fp32 (read it with
- * hz_net_heads_fc_active(..., hc_tiled = 1)).  w_head_tiles == NULL: no head item. */
+ * hz_net_heads_fc_active).  w_head_tiles == NULL: no head item. */
+size_t hz_tower_sched_bytes(int64_t n_boards, int n_blocks);
 int hz_tower_forward_heads(const void *x0_tiles, const void *const *w_tiles,
                            const float *const *biases, int n_blocks, void *buf_a, void *buf_b,
                            void *buf_c, void *sched, void **out_tiles, int64_t n_boards,

@@ -113,9 +113,7 @@ def main():
     r["dense_equiv_tflops"] = dense_flop / r["us_min"] / 1e6
     out["cudnn_conv_warm"] = r
     # whole tower and whole forward (tower + heads), CUDA graph replay like self-play
-    hand_layers = hnet.InferenceNet(model, tower="hand")
-    hand_layers.hand.fused_layers = False
-    for name, net in (("hand", hand), ("hand_per_layer", hand_layers), ("cudnn", lib)):
+    for name, net in (("hand", hand), ("cudnn", lib)):
         logits = torch.zeros((B, 143), dtype=torch.float32, device="cuda")
         value = torch.zeros(B, dtype=torch.float32, device="cuda")
         s = torch.cuda.Stream()
@@ -144,7 +142,7 @@ def main():
     x0 = hand.hand.x0_buffer(B)
     hand.hand.to_tiles(board, 40, True, x0)
     fa = {}
-    for flags, name in ((0, "full"), (4, "no_weight_copies"), (8, "no_act_copies"), (2, "no_epilogue_mem"), (12, "no_copies"), (14, "mma_only"), (1, "no_mma"), (32, "single_issuer")):
+    for flags, name in ((0, "full"), (4, "no_weight_copies"), (8, "no_act_copies"), (2, "no_epilogue_mem"), (12, "no_copies"), (14, "mma_only"), (1, "no_mma")):
         ht.lib.hz_tower_set_debug(flags)
         fa[name] = timeit(lambda: hand.hand.forward_tiles(x0, B), a.iters)["us_min"]
     ht.lib.hz_tower_set_debug(0)

@@ -41,7 +41,7 @@ def test_library_exports_every_declared_symbol(built_lib):
     # the Python binding declares a signature for each of them, and nothing else
     assert sorted(_lib.SIGNATURES) == syms
     loaded = _lib.load()
-    assert loaded.hz_abi_version() == 5
+    assert loaded.hz_abi_version() == 6
     assert loaded.hz_status_string(-4).decode().startswith("workspace")
     assert loaded.hz_launch_count() == 0
     assert loaded.hz_tree_workspace_bytes(4096, 100, 0, 1) > 4096 * 6901 * 128
@@ -159,7 +159,7 @@ def test_network_is_the_reference_model():
 
 
 def test_tower_weight_images_follow_the_documented_layout():
-    """tower.pack_conv_weight / pack_head_weight (host side of hz_tower_forward*): element (tap, out o, in i) of the folded
+    """tower.pack_conv_weight / pack_head_weight (host side of hz_tower_forward_heads): element (tap, out o, in i) of the folded
     weights sits where include/harmonies_b200.h says the K-major SWIZZLE_128B tile keeps it — half i // 64, row o of 128
     bytes, 16-byte group ((i % 64) // 8) ^ (o & 7), element i % 8 — and the head filters are split into bf16 high + low rows
     whose sum reproduces the fp32 filter to 2^-16 relative."""

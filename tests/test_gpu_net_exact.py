@@ -13,25 +13,19 @@ The reference is the module's own layers in float64, with bf16 round-to-nearest-
 kernel does.  It asserts its own preconditions (``reference``), so a change of recipe that stops exercising the rounding
 or leaves the exact range fails loudly instead of passing quietly.
 
-The same exact network runs through every inference path, batch size, active prefix, grid size, tower depth and
-environment switch.  Exact data cannot see a kernel that drops the low part of a bf16 hi + lo split: with integer weights
+The same exact network runs through every inference path, batch size, active prefix, grid size and tower depth.
+Exact data cannot see a kernel that drops the low part of a bf16 hi + lo split: with integer weights
 every low part is zero.  The split-precision tests use real-valued weights with large low parts, and a scale-free bound
 derived in ``split_bound``.  Host-side negative controls show that the bound catches one dropped low product.  The last
 test bounds the fused softmax of ``hz_tree_expand_backup`` per edge against fp64.
 """
 
 import ctypes as ct
-import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
-
-from tests.conftest import ROOT
 
 SIZES = (1, 15, 16, 17, 33, 203, 4096, 4103, 16384)
 N_MAX = max(SIZES)
@@ -236,7 +230,7 @@ def test_recipe_folds_exactly_and_meets_its_preconditions():
 
 
 # ---- the exact network through every path ------------------------------------------------------------------------------
-PATHS = ("forward", "tiles_heads_in_tower", "tiles_head_conv_t16", "layer_by_layer")
+PATHS = ("forward", "tiles")
 
 
 class Runner:
@@ -261,18 +255,11 @@ class Runner:
 
     def run(self, path, b40, x0, gl, n_active=None, out=None):
         inf, B = self.inf, gl.shape[0]
-        try:
-            if path == "forward":                    # hand tower + hz_net_heads (k_heads_p)
-                res = inf(b40, gl, out=out)
-            elif path == "layer_by_layer":           # one hz_tower_conv3x3 launch per layer + k_heads_p
-                inf.hand.fused_layers = False
-                res = inf(b40, gl, out=out)
-            else:                                    # the tile path: head item in the tower, or k_head_conv_t16
-                inf.heads_in_tower = path == "tiles_heads_in_tower"
-                res = inf.forward_tiles(x0, gl, B, out=out, n_active=n_active)
-            torch.cuda.synchronize()
-        finally:
-            inf.hand.fused_layers, inf.heads_in_tower = True, True
+        if path == "forward":                    # hand tower + hz_net_heads (k_heads_p)
+            res = inf(b40, gl, out=out)
+        else:                                    # the tile path: head item in the tower, then k_heads_fc_mma
+            res = inf.forward_tiles(x0, gl, B, out=out, n_active=n_active)
+        torch.cuda.synchronize()
         assert int(self.fault[0]) == 0, f"{path}: barrier time-out {int(self.fault[0]):#x}"
         return tuple(t.clone() for t in res)
 
@@ -307,18 +294,16 @@ def test_every_path_is_exact(exact8, B):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("B", [203, 4103])
-@pytest.mark.parametrize("heads_in_tower", [True, False])
-def test_active_prefix_is_exact_and_leaves_the_rest(exact8, B, heads_in_tower):
+@pytest.mark.parametrize("B", [33, 203, 4103, 16384])
+def test_active_prefix_is_exact_and_leaves_the_rest(exact8, B):
     run, ref = exact8["run"], exact8["ref"]
     b40, x0, gl = run.inputs(exact8["board"][:B], exact8["glob"][:B])
     na = torch.zeros(1, dtype=torch.int32, device="cuda")
-    path = "tiles_heads_in_tower" if heads_in_tower else "tiles_head_conv_t16"
     for k in (0, 1, 16, 17, 31, 32, 33, B - 1, B):
         na.fill_(k)
         out = (torch.full((B, 143), SENTINEL, device="cuda"), torch.full((B,), SENTINEL, device="cuda"))
-        logits, value = run.run(path, b40, x0, gl, n_active=na, out=out)
-        assert_exact((logits, value), ref, k, f"{path}, {B} boards, n_active {k}")
+        logits, value = run.run("tiles", b40, x0, gl, n_active=na, out=out)
+        assert_exact((logits, value), ref, k, f"tiles, {B} boards, n_active {k}")
         assert bool((logits[k:] == SENTINEL).all()) and bool((value[k:] == SENTINEL).all()), k
 
 
@@ -333,7 +318,7 @@ def test_small_grids_are_exact(exact8, ctas):
 def test_mailbox_slot_and_tag_wrap(exact8):
     """One cluster (max_ctas = 2) at 8,192 boards: 256 pairs of tiles x 18 items = 4,608 items through one mailbox, so
     both the slot index (k & 63) and the tag (k % 4095 + 1) wrap; 4,352 without the head item."""
-    _check_paths(exact8["run"], exact8["board"], exact8["glob"], exact8["ref"], [8192], paths=("tiles_heads_in_tower", "forward"), ctas=2)
+    _check_paths(exact8["run"], exact8["board"], exact8["glob"], exact8["ref"], [8192], paths=("tiles", "forward"), ctas=2)
 
 
 @pytest.mark.gpu
@@ -363,7 +348,7 @@ def test_ten_blocks_are_refused():
     from harmonies_alphazero_b200 import _lib
 
     with pytest.raises(_lib.HarmoniesLibraryError):
-        run.run("tiles_heads_in_tower", b40, x0, gl)
+        run.run("tiles", b40, x0, gl)
 
 
 @pytest.mark.gpu
@@ -381,41 +366,6 @@ def test_generic_heads_kernel_on_the_test_size_net(B):
     got = inf._fused_heads(x, glob.cuda().to(torch.bfloat16), None)
     torch.cuda.synchronize()
     assert_exact(got, ref, B, f"k_heads, {B} boards")
-
-
-# ---- environment switches: read once per process, so each runs in a process of its own -------------------------------
-SWITCHES = {"HZ_FC_FMA": "1", "HZ_HEADS_GENERIC": "1", "HZ_TOWER_NO_PAIR": "1", "HZ_TOWER_CLUSTER": "4"}
-
-
-def _switch_main(path):
-    """child process: the exact check of every path at a few sizes, the last one wrapping the mailbox where there is one"""
-    data = torch.load(path)
-    ref = {k: v.cuda() for k, v in data["ref"].items()}
-    board, glob = data["board"].cuda().float(), data["glob"].cuda()
-    run = Runner(exact_model())
-    _check_paths(run, board, glob, ref, [17, 4103, N_MAX])
-    if os.environ.get("HZ_TOWER_CLUSTER") == "4":
-        _check_paths(run, board, glob, ref, [N_MAX], ctas=4)     # one cluster of four: 256 units x 18 = 4,608 items
-    else:
-        _check_paths(run, board, glob, ref, [8192], ctas=2)
-    print(json.dumps({"ok": True}))
-
-
-@pytest.fixture(scope="module")
-def exact8_file(exact8, tmp_path_factory):
-    path = tmp_path_factory.mktemp("exact8") / "exact8.pt"
-    ref = {k: exact8["ref"][k].cpu() for k in ("logits", "value")}
-    torch.save(dict(board=exact8["board"].to(torch.uint8).cpu(), glob=exact8["glob"].cpu(), ref=ref), path)
-    return path
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("switch", sorted(SWITCHES))
-def test_environment_switches_are_exact(exact8_file, switch):
-    env = dict(os.environ, **{switch: SWITCHES[switch]})
-    code = "import sys; from tests.test_gpu_net_exact import _switch_main; _switch_main(sys.argv[1])"
-    r = subprocess.run([sys.executable, "-c", code, str(exact8_file)], capture_output=True, text=True, timeout=900, cwd=ROOT, env=env)
-    assert r.returncode == 0 and '"ok": true' in r.stdout, (r.stdout[-2000:], r.stderr[-3000:])
 
 
 # ---- split precision: real-valued weights with large low parts -------------------------------------------------------
@@ -518,7 +468,7 @@ def test_head_item_and_tensor_core_fc_meet_the_split_bound(exact8):
     run = Runner(model)
     B = 203
     b40, x0, gl = run.inputs(exact8["board"][:B], exact8["glob"][:B])
-    logits, _ = run.run("tiles_heads_in_tower", b40, x0, gl)
+    logits, _ = run.run("tiles", b40, x0, gl)
     hc = run.inf.hand.head_conv(B).view(-1, 3, 35, 16).permute(0, 3, 1, 2).reshape(-1, 3, 35)[:B].double()
     x = exact8["ref"]["tower"][:B]
     wd, bd = w.double().cuda(), b.double().cuda()

@@ -152,9 +152,11 @@ def test_conv_random_values_bf16_tolerance(tw):
 
 def test_fused_launch_equals_layer_by_layer(tw):
     """The persistent all-layers launch (each CTA carries its tiles through the 17 layers) must
-    reproduce the one-launch-per-layer result bit for bit — with one tile per CTA, several tiles per
-    CTA, and all ten tiles through a single CTA (the ready queue hands it every item of every layer)."""
+    reproduce the one-launch-per-layer result (hz_tower_conv3x3 chained here) bit for bit — with one tile
+    per CTA, several tiles per CTA, and all ten tiles through a single CTA (the ready queue hands it every
+    item of every layer)."""
     from harmonies_alphazero_b200 import net as hnet
+    from harmonies_alphazero_b200 import tower as htower
 
     torch.manual_seed(2)
     model = hnet.AlphaZeroNet.from_config(hnet.DEFAULT_MODEL_CONFIG).eval()
@@ -164,9 +166,16 @@ def test_fused_launch_equals_layer_by_layer(tw):
     g = torch.Generator().manual_seed(4)
     b40 = torch.zeros((B, 40, 5, 7), dtype=torch.bfloat16, device="cuda").contiguous(memory_format=torch.channels_last)
     b40[:, :38] = (torch.rand((B, 38, 5, 7), generator=g) < 0.2).to(torch.bfloat16).cuda()
-    ht.fused_layers = False
-    want = ht.forward(b40).clone()
-    ht.fused_layers = True
+    n_pad = (B + 15) // 16 * 16
+    x0 = ht.x0_buffer(B)
+    ht.to_tiles(b40, 40, True, x0)
+    x, y, z = (torch.zeros(n_pad // 16 * 2 * htower.KH_BYTES, dtype=torch.uint8, device="cuda") for _ in range(3))
+    ht.conv(x0, 1, ht.stem, None, x, n_pad, kmajor=True)
+    for c1, c2 in ht.blocks:
+        ht.conv(x, 2, c1, None, y, n_pad)
+        ht.conv(y, 2, c2, x, z, n_pad)
+        x, z = z, x
+    want = ht.from_tiles(x, n_pad)[:B].view(B, 5, 7, 128).permute(0, 3, 1, 2)
     try:
         for ctas in (0, 4, 1):       # 10 tiles: one per CTA / up to 3 per CTA / all 10 in one CTA
             ht.lib.hz_tower_set_max_ctas(ctas)
@@ -294,7 +303,7 @@ def test_self_play_runs_on_the_hand_written_tower(tw):
 
 
 def test_active_prefix_of_the_tile_path(tw):
-    """hz_tower_forward_active / hz_net_*_active: with a device-side row count the evaluated prefix is
+    """hz_tower_forward_heads / hz_net_heads_fc_active: with a device-side row count the evaluated prefix is
     bit-identical to the full evaluation and the rows beyond the last active tile are left untouched."""
     from harmonies_alphazero_b200 import net as hnet
 
@@ -379,43 +388,6 @@ def test_search_is_a_function_of_the_priors_whichever_tower_produced_them(tw):
     N1, W1, P1, _ = t1.root_edges(); N2, W2, P2, _ = t2.root_edges()
     assert torch.equal(N1, N2) and torch.equal(W1, W2) and torch.equal(P1, P2)
     assert worst < 0.03          # same leaves, two towers: bf16-level agreement of priors and values
-
-
-def test_head_convolutions_as_a_tower_work_item(tw):
-    """hz_tower_forward_heads: the 1x1 head convolutions run as one more work item per tile inside the tower
-    launch (single-tap tcgen05.mma, filters split into bf16 high + low parts) and must agree with the separate
-    fp32-FMA kernel (k_head_conv_t16) on the same tower output: 1e-4 absolute on O(1) logits — also with a
-    device-side active count and for a board count that is not a multiple of 16."""
-    from harmonies_alphazero_b200 import net as hnet
-
-    torch.manual_seed(5)
-    model = hnet.AlphaZeroNet.from_config(hnet.DEFAULT_MODEL_CONFIG).eval()
-    for mod in model.modules():
-        if isinstance(mod, torch.nn.BatchNorm2d):
-            mod.running_mean.normal_(0, 0.2); mod.running_var.uniform_(0.6, 1.4)
-            mod.weight.data.uniform_(0.6, 1.4); mod.bias.data.normal_(0, 0.2)
-    hand = hnet.InferenceNet(model, device="cuda", tower="hand")
-    assert hand.heads_in_tower
-    B = 203
-    g = torch.Generator().manual_seed(12)
-    b40 = torch.zeros((B, 40, 5, 7), dtype=torch.bfloat16, device="cuda").contiguous(memory_format=torch.channels_last)
-    b40[:, :38] = (torch.rand((B, 38, 5, 7), generator=g) < 0.2).to(torch.bfloat16).cuda()
-    glob = torch.rand((B, 42), generator=g).to(torch.bfloat16).cuda()
-    x0 = hand.hand.x0_buffer(B)
-    hand.hand.to_tiles(b40, 40, True, x0)
-    l_in, v_in = (t.clone() for t in hand.forward_tiles(x0, glob, B))
-    hand.heads_in_tower = False
-    l_out, v_out = (t.clone() for t in hand.forward_tiles(x0, glob, B))
-    hand.heads_in_tower = True
-    torch.cuda.synchronize()
-    assert float(l_out.abs().max()) > 0.05                      # the logits are not trivially zero
-    assert float((l_in - l_out).abs().max()) <= 1e-4 and float((v_in - v_out).abs().max()) <= 1e-4
-    na = torch.tensor([77], dtype=torch.int32, device="cuda")
-    out = (torch.full((B, 143), -7.0, device="cuda"), torch.full((B,), -7.0, device="cuda"))
-    hand.forward_tiles(x0, glob, B, out=out, n_active=na)
-    torch.cuda.synchronize()
-    assert torch.equal(out[0][:77], l_in[:77]) and torch.equal(out[1][:77], v_in[:77])
-    assert bool((out[0][77:] == -7.0).all())
 
 
 def test_reloaded_weights_take_effect_under_the_captured_graph(tw):
