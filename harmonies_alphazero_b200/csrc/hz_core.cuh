@@ -931,9 +931,45 @@ __device__ __forceinline__ uint32_t channel_mask(const uint32_t* w, int c) {
     uint32_t ph = (m >> 1) & 7u;
     return (ph >= 1 && ph <= 3) ? VALID : 0u;                        // :74-81 (phase 0 and game_over -> 0)
 }
+// the 38 channel bits of the cell at hex hx (0 for the padding cells, hx >= 23): a cell holds at most 3+3 tiles, so
+// each (player p, level l) sets the bit p*18 + (code-1)*3 + l of its tile code instead of probing 38 masks; bit 36 is
+// player 1, bit 37 phase 1-3
+__device__ __forceinline__ uint64_t cell_bits(const uint32_t* w, int hx) {
+    if (hx >= 23) return 0;
+    uint64_t bits = 0;
+#pragma unroll
+    for (int pl = 0; pl < 6; pl++) {
+        uint32_t code = ((w[pl * 3] >> hx) & 1u) | (((w[pl * 3 + 1] >> hx) & 1u) << 1) | (((w[pl * 3 + 2] >> hx) & 1u) << 2);
+        int p = pl / 3, l = pl - 3 * p;
+        if (code) bits |= 1ull << (p * 18 + ((int)code - 1) * 3 + l);
+    }
+    uint32_t m = w[HZ_W_BAG1META] >> 24, ph = (m >> 1) & 7u;
+    if (m & 1u) bits |= 1ull << 36;
+    if (ph >= 1 && ph <= 3) bits |= 1ull << 37;
+    return bits;
+}
+// fp32(k / 3.0) for k = 0..3 by selects (a local array would live in local memory); 1 for k > 3
+__device__ __forceinline__ float third(uint32_t k) {
+    return k == 0 ? 0.0f : k == 1 ? (float)(1.0 / 3.0) : k == 2 ? (float)(2.0 / 3.0) : 1.0f;
+}
+// the value of the phase plane (channel 37) where it is set, i.e. in phases 1-3: the reference's phase / 3.0
+__device__ __forceinline__ float phase_value(const uint32_t* w) { return third((w[HZ_W_BAG1META] >> 25) & 7u); }
+// the one-hot table of the vector stores: VEC = 16 / sizeof(T) bits -> 16 bytes of T 0.0 / 1.0 (16 entries for fp32,
+// 256 for bf16), built by the whole block (not unrolled: with a blockDim.x stride that would cost a trip-count division)
+template <typename T>
+__device__ __forceinline__ void build_onehot_lut(uint4* lut) {
+    constexpr int VEC = 16 / (int)sizeof(T);
+#pragma unroll 1
+    for (int i = threadIdx.x; i < (1 << VEC); i += blockDim.x) {
+        uint32_t o[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+            o[j] = VEC == 4 ? (((i >> j) & 1) ? 0x3F800000u : 0u)
+                            : (((i >> (2 * j)) & 1) ? 0x3F80u : 0u) | (((i >> (2 * j + 1)) & 1) ? 0x3F800000u : 0u);
+        lut[i] = make_uint4(o[0], o[1], o[2], o[3]);
+    }
+}
 __device__ __forceinline__ float global_feature(const uint32_t* w, int g) {
-    // fp32(k / 3.0) for k = 0..3 by selects (a local array would live in local memory)
-    auto third = [](uint32_t k) { return k == 0 ? 0.0f : k == 1 ? (float)(1.0 / 3.0) : k == 2 ? (float)(2.0 / 3.0) : 1.0f; };
     if (g < 30) {                                                    // :98-107
         int i = g / 6, t = g - 6 * i;
         uint32_t np = (w[HZ_W_BAG1META] >> 16) & 0xFFu;
@@ -948,6 +984,27 @@ __device__ __forceinline__ float global_feature(const uint32_t* w, int g) {
     // the two small integers gives the same bits: c/init is exact or has a binary period of at
     // most 22 bits (init <= 23), so its 53-bit rounding can never land on an fp32 midpoint.
     return __fdiv_rn((float)cnt, (float)INIT_BAG[t]);
+}
+
+// ---- warp-level state encoding: one warp per record, one scalar store per element ------------
+// LAYOUT: HZ_LAYOUT_NCHW, HZ_LAYOUT_NHWC, or HZ_LAYOUT_NHWC40 (channel stride 40, channels 38
+// and 39 written as zero: the stem convolution then needs no cuDNN input-padding kernel)
+template <int LAYOUT> struct RowElems { static constexpr int value = LAYOUT == HZ_LAYOUT_NHWC40 ? 1400 : 1330; };   // (T16K never takes the generic path)
+template <typename T, int LAYOUT>
+__device__ __forceinline__ void warp_encode(const uint32_t* w, uint32_t* smask, T* board, T* glob, int lane) {
+    for (int c = lane; c < 40; c += 32) smask[c] = c < 38 ? channel_mask(w, c) : 0u;
+    __syncwarp();
+    float phase_val = phase_value(w);
+    for (int e = lane; e < RowElems<LAYOUT>::value; e += 32) {
+        int c, cell;
+        if (LAYOUT == HZ_LAYOUT_NHWC40) { cell = e / 40; c = e - 40 * cell; }
+        else if (LAYOUT == HZ_LAYOUT_NHWC) { cell = e / 38; c = e - 38 * cell; }
+        else { c = e / 35; cell = e - 35 * c; }
+        uint32_t bit = (smask[c] >> CELL_HEX[cell]) & 1u;
+        board[e] = cvt<T>(bit ? (c == 37 ? phase_val : 1.0f) : 0.0f);
+    }
+    for (int g = lane; g < 42; g += 32) glob[g] = cvt<T>(global_feature(w, g));
+    __syncwarp();
 }
 
 

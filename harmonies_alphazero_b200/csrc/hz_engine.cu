@@ -4,9 +4,10 @@
 //
 // Mapping: one thread per game, state held in registers (7 x LDG.128 in, 8 x STG.128 out),
 // hex-parallel work done as 23-bit bit-board arithmetic; the neighbour expansion LUT lives in
-// 3 KB of shared memory per block.  hz_encode is write-bound (5.5 KB out per 128 B in): a warp
-// renders a group of records as a bit stream and stores 16-byte vectors through a lookup table
-// (k_encode_w); hz_greedy_actions is warp-per-game with one lane per legal move.
+// 3 KB of shared memory per block.  hz_encode is write-bound (5.5 KB out per 128 B in) and one
+// launch of k_encode: a warp renders a group of records as a bit stream and stores 16-byte vectors
+// through a lookup table, and encodes the records outside whole aligned groups one by one with
+// scalar stores (warp_encode); hz_greedy_actions is warp-per-game with one lane per legal move.
 #include "hz_common.cuh"
 #include "hz_core.cuh"
 
@@ -307,187 +308,33 @@ __global__ void __launch_bounds__(PTPB, 7) k_playout(void* states, int64_t n, in
 }
 
 // ---- encode (process_game_state.py:15-137) ------------------------------------------------------
-constexpr int ENC_S = 8;      // states per block iteration
-constexpr int ENC_TPB = 256;
+// One WARP renders a group of G records (G*1330 elements = 665 16-byte vectors: G = 2 for fp32,
+// 4 for bf16) with no block-level barrier at all — each warp has its own staging area and only
+// __syncwarp()s, so the SM always has other warps to issue from.  The tensor is ~94 % zeros and
+// every non-zero is 1.0 except the phase plane, so the group is first rendered as a BIT stream in
+// output order (1 bit per element) and a store is then one table lookup: VEC bits -> 16 bytes of
+// 0.0/1.0 (then the phase patch).  The records outside whole groups at a 16-byte-aligned board
+// (the n mod G last ones, or all of them when the board is not aligned) are work items of the same
+// loop, one warp per record with scalar stores (warp_encode).
+constexpr int ENC_WARPS = 8;
 template <typename T, bool NHWC>
-__global__ void __launch_bounds__(ENC_TPB) k_encode(const void* states, int64_t n, T* board, T* glob, int vec_ok) {
-    __shared__ uint32_t smask[ENC_S][40];
-    __shared__ float sphase[ENC_S];
-    __shared__ float sglob[ENC_S][42];
-    __shared__ uint8_t scell[36];   // shared copy: per-lane indices into __constant__ would serialise
-    __shared__ uint8_t shex[24];
-    __shared__ __align__(16) uint32_t sw[ENC_S][32];
-    // The tensor is ~94 % zeros and every non-zero is 1.0 except the phase plane, so the chunk
-    // is first rendered as a BIT stream in output order (1 bit per element, 10,640 bits) and a
-    // store is then one table lookup: VEC bits -> 16 bytes of 0.0/1.0 (then the phase patch).
-    constexpr int VEC = 16 / (int)sizeof(T);
-    __shared__ uint32_t stream[ENC_S * 1330 / 32 + 4], pstream[ENC_S * 1330 / 32 + 4];
-    __shared__ uint64_t perm[3][256];   // hex-order byte -> cell-order bits (NCHW rows)
-    __shared__ uint4 vlut[1 << VEC];
-    __shared__ uint32_t sphase_bits[ENC_S];
-    if (threadIdx.x < 35) scell[threadIdx.x] = CELL_HEX[threadIdx.x];
-    if (threadIdx.x < 23) shex[threadIdx.x] = HEX_CELL[threadIdx.x];
-    for (int i = threadIdx.x; i < (1 << VEC); i += ENC_TPB) {
-        uint32_t o[4];
-        if (VEC == 4) {
-#pragma unroll
-            for (int j = 0; j < 4; j++) o[j] = ((i >> j) & 1) ? 0x3F800000u : 0u;
-        } else {
-#pragma unroll
-            for (int j = 0; j < 4; j++) o[j] = (((i >> (2 * j)) & 1) ? 0x3F80u : 0u) | (((i >> (2 * j + 1)) & 1) ? 0x3F800000u : 0u);
-        }
-        vlut[i] = make_uint4(o[0], o[1], o[2], o[3]);
-    }
-    if (!NHWC) {
-        for (int e = threadIdx.x; e < 768; e += ENC_TPB) {
-            int c = e >> 8, v = e & 255;
-            uint64_t m = 0;
-            for (int b = 0; b < 8; b++) {
-                int i = c * 8 + b;
-                if (((v >> b) & 1) && i < 23) m |= 1ull << HEX_CELL[i];
-            }
-            perm[c][v] = m;
-        }
-    }
-    const uint32_t* W = reinterpret_cast<const uint32_t*>(states);
-    int64_t n_chunks = (n + ENC_S - 1) / ENC_S;
-    for (int64_t chunk = blockIdx.x; chunk < n_chunks; chunk += gridDim.x) {
-        int64_t base = chunk * ENC_S;
-        int cnt = (int)min((int64_t)ENC_S, n - base);
-        for (int i = threadIdx.x; i < ENC_S * 1330 / 32 + 4; i += ENC_TPB) { stream[i] = 0; pstream[i] = 0; }
-        // stage the chunk's records (1 KB) in shared memory with one coalesced 16-byte load per
-        // thread: the 640 mask/feature tasks below each read 1-3 words of a record
-        if (threadIdx.x < cnt * 8)
-            reinterpret_cast<uint4*>(&sw[0][0])[threadIdx.x] = reinterpret_cast<const uint4*>(W)[base * 8 + threadIdx.x];
-        __syncthreads();
-        for (int item = threadIdx.x; item < cnt * 80; item += ENC_TPB) {
-            int s = item / 80, c = item - 80 * s;
-            const uint32_t* w = sw[s];
-            if (c < 38) {
-                smask[s][c] = channel_mask(w, c);
-                if (c == 37) sphase[s] = (float)((double)((w[HZ_W_BAG1META] >> 25) & 7u) / 3.0);
-            } else {
-                sglob[s][c - 38] = global_feature(w, c - 38);
-            }
-        }
-        __syncthreads();
-        // Write-bound part: every thread emits one 16-byte vector (4 fp32 / 8 bf16) per store.
-        // A chunk of 8 states is 8*1330 elements = a whole number of vectors and starts
-        // 16-byte aligned; a ragged last chunk falls back to scalar stores.
-        T* bout = board + base * 1330;
-        int total = cnt * 1330;
-        int nvec = (cnt == ENC_S && vec_ok) ? total / VEC : 0;
-        if (nvec) {
-            // ---- render the bit stream: one task per (state, channel) [NCHW] or (state, cell) [NHWC]
-            if (threadIdx.x < ENC_S) {
-                float pv = sphase[threadIdx.x];
-                sphase_bits[threadIdx.x] = VEC == 4 ? __float_as_uint(pv) : (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(pv));
-            }
-            constexpr int ROWS = NHWC ? 35 : 38, ROW_BITS = NHWC ? 38 : 35;
-            for (int item = threadIdx.x; item < ENC_S * ROWS; item += ENC_TPB) {
-                int s = item / ROWS, row = item - ROWS * s;
-                uint64_t bits = 0;
-                if (NHWC) {
-                    int hx = scell[row];
-                    if (hx < 23) {
-                        // a cell has at most 3+3 tiles: read the tile code of each (player, level)
-                        // and set its channel bit (p*18 + type*3 + level) instead of probing 38 masks
-                        const uint32_t* w = sw[s];
-#pragma unroll
-                        for (int pl = 0; pl < 6; pl++) {
-                            uint32_t code = ((w[pl * 3] >> hx) & 1u) | (((w[pl * 3 + 1] >> hx) & 1u) << 1) | (((w[pl * 3 + 2] >> hx) & 1u) << 2);
-                            int p = pl / 3, l = pl - 3 * p;
-                            if (code) bits |= 1ull << (p * 18 + ((int)code - 1) * 3 + l);
-                        }
-                        bits |= (uint64_t)((smask[s][36] >> hx) & 1u) << 36;
-                        bits |= (uint64_t)((smask[s][37] >> hx) & 1u) << 37;
-                    }
-                } else {
-                    uint32_t m = smask[s][row];                      // hex order -> cell order: 3 table lookups
-                    bits = perm[0][m & 255] | perm[1][(m >> 8) & 255] | perm[2][(m >> 16) & 127];
-                }
-                if (bits) {
-                    int off = s * 1330 + row * ROW_BITS, wd = off >> 5, sh = off & 31;
-                    uint64_t lo = bits << sh;
-                    uint32_t hi = sh ? (uint32_t)(bits >> (64 - sh)) : 0u;
-                    if ((uint32_t)lo) atomicOr(&stream[wd], (uint32_t)lo);
-                    if ((uint32_t)(lo >> 32)) atomicOr(&stream[wd + 1], (uint32_t)(lo >> 32));
-                    if (hi) atomicOr(&stream[wd + 2], hi);
-                    // second stream: the set elements of the phase plane (channel 37, value k/3)
-                    uint64_t pbits = NHWC ? (bits & (1ull << 37)) : (row == 37 ? bits : 0ull);
-                    if (pbits) {
-                        uint64_t plo = pbits << sh;
-                        uint32_t phi = sh ? (uint32_t)(pbits >> (64 - sh)) : 0u;
-                        if ((uint32_t)plo) atomicOr(&pstream[wd], (uint32_t)plo);
-                        if ((uint32_t)(plo >> 32)) atomicOr(&pstream[wd + 1], (uint32_t)(plo >> 32));
-                        if (phi) atomicOr(&pstream[wd + 2], phi);
-                    }
-                }
-            }
-            __syncthreads();
-        }
-        for (int v = threadIdx.x; v < nvec; v += ENC_TPB) {
-            int e0 = v * VEC;
-            uint32_t nib = (stream[e0 >> 5] >> (e0 & 31)) & ((1u << VEC) - 1u);   // VEC divides 32: never straddles
-            uint32_t pm = (pstream[e0 >> 5] >> (e0 & 31)) & ((1u << VEC) - 1u);
-            uint4 o = vlut[nib];
-            while (pm) {                                             // rare: phase-plane elements hold k/3, not 1.0
-                int j = __ffs(pm) - 1;
-                pm &= pm - 1;
-                uint32_t pb = sphase_bits[(e0 + j) / 1330];
-                int wi = VEC == 4 ? j : (j >> 1);
-                uint32_t cur = wi == 0 ? o.x : wi == 1 ? o.y : wi == 2 ? o.z : o.w;
-                uint32_t nw = VEC == 4 ? pb : ((j & 1) ? ((cur & 0x0000FFFFu) | (pb << 16)) : ((cur & 0xFFFF0000u) | pb));
-                o.x = wi == 0 ? nw : o.x; o.y = wi == 1 ? nw : o.y; o.z = wi == 2 ? nw : o.z; o.w = wi == 3 ? nw : o.w;
-            }
-            reinterpret_cast<uint4*>(bout)[v] = o;
-        }
-        for (int e = nvec * VEC + threadIdx.x; e < total; e += ENC_TPB) {
-            int s = e / 1330, r = e - 1330 * s;
-            int c, cell;
-            if (NHWC) { cell = r / 38; c = r - 38 * cell; } else { c = r / 35; cell = r - 35 * c; }
-            uint32_t bit = (smask[s][c] >> scell[cell]) & 1u;
-            bout[e] = cvt<T>(bit ? (c == 37 ? sphase[s] : 1.0f) : 0.0f);
-        }
-        T* gout = glob + base * 42;
-        for (int e = threadIdx.x; e < cnt * 42; e += ENC_TPB) gout[e] = cvt<T>(sglob[e / 42][e % 42]);
-        __syncthreads();
-    }
-}
-
-// Fast path of hz_encode: one WARP renders a group of G records (G*1330 elements = 665 16-byte
-// vectors: G = 2 for fp32, 4 for bf16) with no block-level barrier at all — each warp has its
-// own staging area and only __syncwarp()s, so the SM always has other warps to issue from.
-// Same bit-stream + table-lookup scheme as k_encode (which remains the tail / unaligned path).
-constexpr int ENCW_WARPS = 8;
-template <typename T, bool NHWC>
-__global__ void __launch_bounds__(ENCW_WARPS * 32) k_encode_w(const void* states, int64_t n_groups, T* board, T* glob) {
+__global__ void __launch_bounds__(ENC_WARPS * 32) k_encode(const void* states, int64_t n, T* board, T* glob) {
     constexpr int VEC = 16 / (int)sizeof(T);
     constexpr int G = VEC / 2;                       // 2 (fp32) or 4 (bf16) records per group
     constexpr int NV = G * 1330 / VEC;               // 665 vectors per group
     constexpr int SWORDS = (G * 1330 + 31) / 32 + 3;
     constexpr int ROWS = NHWC ? 35 : 38, ROW_BITS = NHWC ? 38 : 35;
-    __shared__ __align__(16) uint32_t sw[ENCW_WARPS][G][32];
-    __shared__ uint32_t smask[ENCW_WARPS][G][40];
-    __shared__ uint32_t stream[ENCW_WARPS][SWORDS], pstream[ENCW_WARPS][SWORDS];
-    __shared__ uint32_t sphase_bits[ENCW_WARPS][G];
-    __shared__ uint64_t perm[3][256];
+    __shared__ __align__(16) uint32_t sw[ENC_WARPS][G][32];
+    __shared__ uint32_t smask[ENC_WARPS][G][40];
+    __shared__ uint32_t stream[ENC_WARPS][SWORDS], pstream[ENC_WARPS][SWORDS];
+    __shared__ uint32_t sphase_bits[ENC_WARPS][G];
+    __shared__ uint64_t perm[3][256];   // hex-order byte -> cell-order bits (NCHW rows)
     __shared__ uint4 vlut[1 << VEC];
-    __shared__ uint8_t scell[36];
+    __shared__ uint8_t scell[36];       // shared copy: per-lane indices into __constant__ would serialise
     if (threadIdx.x < 35) scell[threadIdx.x] = CELL_HEX[threadIdx.x];
-    for (int i = threadIdx.x; i < (1 << VEC); i += ENCW_WARPS * 32) {
-        uint32_t o[4];
-        if (VEC == 4) {
-#pragma unroll
-            for (int j = 0; j < 4; j++) o[j] = ((i >> j) & 1) ? 0x3F800000u : 0u;
-        } else {
-#pragma unroll
-            for (int j = 0; j < 4; j++) o[j] = (((i >> (2 * j)) & 1) ? 0x3F80u : 0u) | (((i >> (2 * j + 1)) & 1) ? 0x3F800000u : 0u);
-        }
-        vlut[i] = make_uint4(o[0], o[1], o[2], o[3]);
-    }
+    build_onehot_lut<T>(vlut);
     if (!NHWC) {
-        for (int e = threadIdx.x; e < 768; e += ENCW_WARPS * 32) {
+        for (int e = threadIdx.x; e < 768; e += ENC_WARPS * 32) {
             int c = e >> 8, v = e & 255;
             uint64_t m = 0;
             for (int b = 0; b < 8; b++) {
@@ -501,45 +348,42 @@ __global__ void __launch_bounds__(ENCW_WARPS * 32) k_encode_w(const void* states
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint32_t* my_stream = stream[warp];
     uint32_t* my_pstream = pstream[warp];
-    const int64_t n_warps = (int64_t)gridDim.x * ENCW_WARPS;
-    for (int64_t grp = (int64_t)blockIdx.x * ENCW_WARPS + warp; grp < n_groups; grp += n_warps) {
-        const int64_t base = grp * G;
+    const int64_t n_warps = (int64_t)gridDim.x * ENC_WARPS;
+    const int64_t n_groups = ((uintptr_t)board & 15) == 0 ? n / G : 0;   // the vector stores need an aligned base
+    const int64_t n_items = n - n_groups * (G - 1);   // the groups, then one item per remaining record
+    for (int64_t item = (int64_t)blockIdx.x * ENC_WARPS + warp; item < n_items; item += n_warps) {
+        if (item >= n_groups) {
+            const int64_t r = item + n_groups * (G - 1);
+            sw[warp][0][lane] = reinterpret_cast<const uint32_t*>(states)[r * 32 + lane];
+            __syncwarp();
+            warp_encode<T, NHWC ? HZ_LAYOUT_NHWC : HZ_LAYOUT_NCHW>(sw[warp][0], smask[warp][0], board + r * 1330, glob + r * 42, lane);
+            continue;
+        }
+        const int64_t base = item * G;
         for (int i = lane; i < G * 8; i += 32)
             reinterpret_cast<uint4*>(&sw[warp][0][0])[i] = reinterpret_cast<const uint4*>(states)[base * 8 + i];
         for (int i = lane; i < SWORDS; i += 32) { my_stream[i] = 0; my_pstream[i] = 0; }
         __syncwarp();
-        // channel masks (hex order) and the 42 global features of each record
-        for (int item = lane; item < G * 80; item += 32) {
-            int s = item / 80, c = item - 80 * s;
+        // channel masks (hex order, NCHW rows) and the 42 global features of each record
+        for (int it = lane; it < G * 80; it += 32) {
+            int s = it / 80, c = it - 80 * s;
             const uint32_t* w = sw[warp][s];
-            if (c < 38) smask[warp][s][c] = channel_mask(w, c);
-            else glob[(base + s) * 42 + (c - 38)] = cvt<T>(global_feature(w, c - 38));
+            if (c >= 38) glob[(base + s) * 42 + (c - 38)] = cvt<T>(global_feature(w, c - 38));
+            else if (!NHWC) smask[warp][s][c] = channel_mask(w, c);
         }
         if (lane < G) {
-            uint32_t ph = (sw[warp][lane][HZ_W_BAG1META] >> 25) & 7u;
-            float pv = ph == 1 ? (float)(1.0 / 3.0) : ph == 2 ? (float)(2.0 / 3.0) : ph == 3 ? 1.0f : 0.0f;
+            float pv = phase_value(sw[warp][lane]);
             sphase_bits[warp][lane] = VEC == 4 ? __float_as_uint(pv) : (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(pv));
         }
         __syncwarp();
-        // bit streams in output order
-        for (int item = lane; item < G * ROWS; item += 32) {
-            int s = item / ROWS, row = item - ROWS * s;
-            uint64_t bits = 0;
+        // bit streams in output order: one task per (record, cell) [NHWC] or (record, channel) [NCHW]
+        for (int it = lane; it < G * ROWS; it += 32) {
+            int s = it / ROWS, row = it - ROWS * s;
+            uint64_t bits;
             if (NHWC) {
-                int hx = scell[row];
-                if (hx < 23) {
-                    const uint32_t* w = sw[warp][s];
-#pragma unroll
-                    for (int pl = 0; pl < 6; pl++) {
-                        uint32_t code = ((w[pl * 3] >> hx) & 1u) | (((w[pl * 3 + 1] >> hx) & 1u) << 1) | (((w[pl * 3 + 2] >> hx) & 1u) << 2);
-                        int p = pl / 3, l = pl - 3 * p;
-                        if (code) bits |= 1ull << (p * 18 + ((int)code - 1) * 3 + l);
-                    }
-                    bits |= (uint64_t)((smask[warp][s][36] >> hx) & 1u) << 36;
-                    bits |= (uint64_t)((smask[warp][s][37] >> hx) & 1u) << 37;
-                }
+                bits = cell_bits(sw[warp][s], scell[row]);
             } else {
-                uint32_t m = smask[warp][s][row];
+                uint32_t m = smask[warp][s][row];                      // hex order -> cell order: 3 table lookups
                 bits = perm[0][m & 255] | perm[1][(m >> 8) & 255] | perm[2][(m >> 16) & 127];
             }
             if (bits) {
@@ -549,6 +393,7 @@ __global__ void __launch_bounds__(ENCW_WARPS * 32) k_encode_w(const void* states
                 if ((uint32_t)lo) atomicOr(&my_stream[wd], (uint32_t)lo);
                 if ((uint32_t)(lo >> 32)) atomicOr(&my_stream[wd + 1], (uint32_t)(lo >> 32));
                 if (hi) atomicOr(&my_stream[wd + 2], hi);
+                // second stream: the set elements of the phase plane (channel 37, value k/3)
                 uint64_t pbits = NHWC ? (bits & (1ull << 37)) : (row == 37 ? bits : 0ull);
                 if (pbits) {
                     uint64_t plo = pbits << sh;
@@ -563,7 +408,7 @@ __global__ void __launch_bounds__(ENCW_WARPS * 32) k_encode_w(const void* states
         uint4* out = reinterpret_cast<uint4*>(board + base * 1330);   // G*1330*sizeof(T) is a multiple of 16
         for (int v = lane; v < NV; v += 32) {
             int e0 = v * VEC;
-            uint32_t nib = (my_stream[e0 >> 5] >> (e0 & 31)) & ((1u << VEC) - 1u);
+            uint32_t nib = (my_stream[e0 >> 5] >> (e0 & 31)) & ((1u << VEC) - 1u);   // VEC divides 32: never straddles
             uint32_t pm = (my_pstream[e0 >> 5] >> (e0 & 31)) & ((1u << VEC) - 1u);
             uint4 o = vlut[nib];
             while (pm) {                                             // phase-plane elements hold k/3, not 1.0
@@ -647,44 +492,19 @@ int hz_encode(const void* states, int64_t n, void* board, void* glob, int dtype,
     if (!states || !board || !glob || n < 0) return HZ_ERR_ARG;
     if (dtype != HZ_DTYPE_F32 && dtype != HZ_DTYPE_BF16) return HZ_ERR_ARG;
     if (layout != HZ_LAYOUT_NCHW && layout != HZ_LAYOUT_NHWC) return HZ_ERR_ARG;
-    if (n == 0) return HZ_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    int vec_ok = ((uintptr_t)board & 15) == 0;   // 16-byte vector stores need an aligned base
-    // fast path: whole groups of 2 (fp32) / 4 (bf16) records, one warp per group, no block barriers
-    int G = dtype == HZ_DTYPE_F32 ? 2 : 4;
-    int64_t n_groups = vec_ok ? n / G : 0, done = n_groups * G;
-    int launches = 0;
-    if (n_groups) {
-        int64_t blocks = (n_groups + ENCW_WARPS - 1) / ENCW_WARPS;
-        int grid = (int)(blocks < 148 * 6 ? blocks : 148 * 6);
-        if (dtype == HZ_DTYPE_F32) {
-            if (layout == HZ_LAYOUT_NCHW) k_encode_w<float, false><<<grid, ENCW_WARPS * 32, 0, st>>>(states, n_groups, (float*)board, (float*)glob);
-            else k_encode_w<float, true><<<grid, ENCW_WARPS * 32, 0, st>>>(states, n_groups, (float*)board, (float*)glob);
-        } else {
-            if (layout == HZ_LAYOUT_NCHW) k_encode_w<__nv_bfloat16, false><<<grid, ENCW_WARPS * 32, 0, st>>>(states, n_groups, (__nv_bfloat16*)board, (__nv_bfloat16*)glob);
-            else k_encode_w<__nv_bfloat16, true><<<grid, ENCW_WARPS * 32, 0, st>>>(states, n_groups, (__nv_bfloat16*)board, (__nv_bfloat16*)glob);
-        }
-        launches++;
+    // work items of one warp each: whole groups of G records at an aligned board, then the remaining records
+    int64_t G = dtype == HZ_DTYPE_F32 ? 2 : 4, n_groups = ((uintptr_t)board & 15) == 0 ? n / G : 0;
+    int64_t blocks = (n - n_groups * (G - 1) + ENC_WARPS - 1) / ENC_WARPS;
+    int grid = (int)(blocks < 148 * 6 ? blocks : 148 * 6);
+    if (dtype == HZ_DTYPE_F32) {
+        if (layout == HZ_LAYOUT_NCHW) k_encode<float, false><<<grid, ENC_WARPS * 32, 0, st>>>(states, n, (float*)board, (float*)glob);
+        else k_encode<float, true><<<grid, ENC_WARPS * 32, 0, st>>>(states, n, (float*)board, (float*)glob);
+    } else {
+        if (layout == HZ_LAYOUT_NCHW) k_encode<__nv_bfloat16, false><<<grid, ENC_WARPS * 32, 0, st>>>(states, n, (__nv_bfloat16*)board, (__nv_bfloat16*)glob);
+        else k_encode<__nv_bfloat16, true><<<grid, ENC_WARPS * 32, 0, st>>>(states, n, (__nv_bfloat16*)board, (__nv_bfloat16*)glob);
     }
-    if (done < n) {   // tail (or unaligned output): the block kernel, scalar stores
-        int64_t m = n - done;
-        const char* sp = (const char*)states + done * 128;
-        size_t esz = dtype == HZ_DTYPE_F32 ? 4 : 2;
-        char* bp = (char*)board + (size_t)done * 1330 * esz;
-        char* gp = (char*)glob + (size_t)done * 42 * esz;
-        int64_t chunks = (m + ENC_S - 1) / ENC_S;
-        int grid = (int)(chunks < 148 * 8 ? chunks : 148 * 8);
-        int tail_vec = ((uintptr_t)bp & 15) == 0;
-        if (dtype == HZ_DTYPE_F32) {
-            if (layout == HZ_LAYOUT_NCHW) k_encode<float, false><<<grid, ENC_TPB, 0, st>>>(sp, m, (float*)bp, (float*)gp, tail_vec);
-            else k_encode<float, true><<<grid, ENC_TPB, 0, st>>>(sp, m, (float*)bp, (float*)gp, tail_vec);
-        } else {
-            if (layout == HZ_LAYOUT_NCHW) k_encode<__nv_bfloat16, false><<<grid, ENC_TPB, 0, st>>>(sp, m, (__nv_bfloat16*)bp, (__nv_bfloat16*)gp, tail_vec);
-            else k_encode<__nv_bfloat16, true><<<grid, ENC_TPB, 0, st>>>(sp, m, (__nv_bfloat16*)bp, (__nv_bfloat16*)gp, tail_vec);
-        }
-        launches++;
-    }
-    return hz_launched(launches);
+    return hz_launched(1);
 }
 
 int hz_canon_hash(const void* states, int64_t n, int key_mode, uint64_t* hashes, void* stream) {

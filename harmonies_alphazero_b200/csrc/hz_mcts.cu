@@ -112,27 +112,6 @@ __global__ void __launch_bounds__(TTPB) k_tree_reset(hz_tree T, const uint4* roo
     T.search_key[t] = keys ? keys[t] : rand64(key_of(s) ^ HZ_SEARCH_SALT, (uint64_t)s.w[HZ_W_MOVES]);
 }
 
-// ---- warp-level state encoding (shared with hz_encode's definition of the tensors) -----------
-// LAYOUT: HZ_LAYOUT_NCHW, HZ_LAYOUT_NHWC, or HZ_LAYOUT_NHWC40 (channel stride 40, channels 38
-// and 39 written as zero: the stem convolution then needs no cuDNN input-padding kernel)
-template <int LAYOUT> struct RowElems { static constexpr int value = LAYOUT == HZ_LAYOUT_NHWC40 ? 1400 : 1330; };   // (T16K never takes the generic path)
-template <typename T, int LAYOUT>
-__device__ __forceinline__ void warp_encode(const uint32_t* w, uint32_t* smask, T* board, T* glob, int lane) {
-    for (int c = lane; c < 40; c += 32) smask[c] = c < 38 ? channel_mask(w, c) : 0u;
-    __syncwarp();
-    float phase_val = (float)((double)((w[HZ_W_BAG1META] >> 25) & 7u) / 3.0);
-    for (int e = lane; e < RowElems<LAYOUT>::value; e += 32) {
-        int c, cell;
-        if (LAYOUT == HZ_LAYOUT_NHWC40) { cell = e / 40; c = e - 40 * cell; }
-        else if (LAYOUT == HZ_LAYOUT_NHWC) { cell = e / 38; c = e - 38 * cell; }
-        else { c = e / 35; cell = e - 35 * c; }
-        uint32_t bit = (smask[c] >> CELL_HEX[cell]) & 1u;
-        board[e] = cvt<T>(bit ? (c == 37 ? phase_val : 1.0f) : 0.0f);
-    }
-    for (int g = lane; g < 42; g += 32) glob[g] = cvt<T>(global_feature(w, g));
-    __syncwarp();
-}
-
 // Fast leaf encoder for the self-play layout (bf16, NHWC40): the 40 channels of a cell are
 // 5 bytes of bits (<= 3+3 tile codes + player + phase), and 8 bits expand to a 16-byte vector
 // of bf16 0.0/1.0 by one table lookup: 35 cells x 5 vectors = 175 16-byte stores per leaf
@@ -143,27 +122,13 @@ __device__ __forceinline__ void warp_encode(const uint32_t* w, uint32_t* smask, 
 template <bool T16K>
 __device__ __forceinline__ void warp_encode_fast40(const uint32_t* w, uint8_t* sbytes, const uint4* vlut8,
                                                    const uint8_t* scell, __nv_bfloat16* board, size_t row, __nv_bfloat16* glob, int lane) {
-    uint32_t m = w[HZ_W_BAG1META] >> 24, ph = (m >> 1) & 7u;
-    bool player1 = (m & 1u) != 0, phase_on = ph >= 1 && ph <= 3;
     for (int cell = lane; cell < 35; cell += 32) {
-        int hx = scell[cell];
-        uint64_t bits = 0;
-        if (hx < 23) {
-#pragma unroll
-            for (int pl = 0; pl < 6; pl++) {
-                uint32_t code = ((w[pl * 3] >> hx) & 1u) | (((w[pl * 3 + 1] >> hx) & 1u) << 1) | (((w[pl * 3 + 2] >> hx) & 1u) << 2);
-                int p = pl / 3, l = pl - 3 * p;
-                if (code) bits |= 1ull << (p * 18 + ((int)code - 1) * 3 + l);
-            }
-            if (player1) bits |= 1ull << 36;
-            if (phase_on) bits |= 1ull << 37;
-        }
+        uint64_t bits = cell_bits(w, scell[cell]);
 #pragma unroll
         for (int k = 0; k < 5; k++) sbytes[cell * 5 + k] = (uint8_t)(bits >> (8 * k));
     }
     __syncwarp();
-    float pv = ph == 1 ? (float)(1.0 / 3.0) : ph == 2 ? (float)(2.0 / 3.0) : 1.0f;
-    uint32_t pb = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(pv));
+    uint32_t pb = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(phase_value(w)));
     uint4* out = reinterpret_cast<uint4*>(board + row * 1400);
     uint8_t* tile = reinterpret_cast<uint8_t*>(board) + (row >> 4) * (size_t)(560 * 128);
     const int leaf = (int)(row & 15);
@@ -193,12 +158,7 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
     __shared__ uint8_t sbytes[FAST40 ? WPB : 1][176];
     __shared__ uint8_t scell[36];
     if (FAST40) {
-        for (int i = threadIdx.x; i < 256; i += TTPB) {
-            uint32_t o[4];
-#pragma unroll
-            for (int j = 0; j < 4; j++) o[j] = (((i >> (2 * j)) & 1) ? 0x3F80u : 0u) | (((i >> (2 * j + 1)) & 1) ? 0x3F800000u : 0u);
-            vlut8[i] = make_uint4(o[0], o[1], o[2], o[3]);
-        }
+        build_onehot_lut<__nv_bfloat16>(vlut8);
         if (threadIdx.x < 35) scell[threadIdx.x] = CELL_HEX[threadIdx.x];
         __syncthreads();
     }

@@ -103,6 +103,90 @@ def test_golden_encode_fp32_bit_exact(hb):
         assert torch.equal(b3.contiguous(), b.to(torch.bfloat16)) and torch.equal(gl3, gl.to(torch.bfloat16))
 
 
+# hz_encode renders whole 16-byte-aligned groups of 2 (fp32) / 4 (bf16) records with vector stores and every other
+# record (the ragged tail, or all of them when the board is not aligned) with scalar ones.  The sizes cover fewer
+# records than a group, one record past a group and, at 30,001, more groups than the 148*6 blocks x 8 warps of the
+# grid-stride loop hold (28,416 bf16 / 14,208 fp32 records), so that it wraps.
+ENCODE_SIZES = (1, 2, 3, 4, 5, 7, 9, 37, 4099, 30001)
+ENCODE_KINDS = [(d, cl) for d in (torch.float32, torch.bfloat16) for cl in (False, True)]
+SENTINEL = -7.0
+
+
+def _offsets(dtype):
+    """output offsets in elements: aligned, one element off, 8 bytes off"""
+    return (0, 1, 8 // torch.empty(0, dtype=dtype).element_size())
+
+
+@pytest.fixture(scope="module")
+def encode_pool(hb):
+    """32,524 records in a fixed shuffled order: games 0..49 actions deep (every phase, both players), games played
+    to the end, the weird goldens and the encode goldens"""
+    n, groups = 20000, 50
+    st = hb.init_states(n, seed=606)
+    per = n // groups
+    for d in range(1, groups):
+        hb.playout(st[d * per:(d + 1) * per], max_steps=d if d < groups - 1 else 1000)
+    words = np.concatenate([host(st), load_golden("weird")["states"], load_golden("encode")["states"]])
+    words = words[np.random.default_rng(606).permutation(len(words))]
+    meta = words[:, 22] >> 24
+    assert set((meta & 1).tolist()) == {0, 1} and set(((meta >> 1) & 7).tolist()) >= {0, 1, 2, 3, 4}
+    return words
+
+
+def _encode_into(hb, st, dtype, cl, off):
+    """hz_encode into views at element offset `off` of sentinel-filled buffers; returns (board, glob, bbuf, gbuf)"""
+    n = st.shape[0]
+    bbuf = torch.full((off + n * 1330 + 64,), SENTINEL, dtype=dtype, device="cuda")
+    gbuf = torch.full((off + n * 42 + 64,), SENTINEL, dtype=dtype, device="cuda")
+    flat = bbuf[off:off + n * 1330]
+    board = flat.view(n, 5, 7, 38).permute(0, 3, 1, 2) if cl else flat.view(n, 38, 5, 7)
+    glob = gbuf[off:off + n * 42].view(n, 42)
+    hb.encode(st, dtype=dtype, channels_last=cl, board=board, glob=glob)
+    return board, glob, bbuf, gbuf
+
+
+@pytest.mark.parametrize("dtype,cl", ENCODE_KINDS)
+def test_encode_every_size_and_alignment_vs_oracle(hb, oracle, encode_pool, dtype, cl):
+    """hz_encode == oracle.encode at every size and at outputs aligned, 1 element off and 8 bytes off: fp32 bit for
+    bit, bf16 the round-to-nearest-even of the oracle's fp32, channels-last the same logical tensor; no byte outside
+    the n records is written"""
+    bits = torch.int32 if dtype == torch.float32 else torch.int16
+    for n in ENCODE_SIZES:
+        words = encode_pool[:n]
+        st = dev(words)
+        outs = []
+        for off in _offsets(dtype):
+            board, glob, bbuf, gbuf = _encode_into(hb, st, dtype, cl, off)
+            for buf, end in ((bbuf, off + n * 1330), (gbuf, off + n * 42)):
+                assert bool((buf[:off] == SENTINEL).all()) and bool((buf[end:] == SENTINEL).all()), (n, off)
+            outs.append((board, glob))
+        board, glob = outs[0]
+        for b, g in outs[1:]:
+            assert torch.equal(b.view(bits), board.view(bits)) and torch.equal(g.view(bits), glob.view(bits)), n
+        for lo in range(0, n, 4096):
+            hi = min(n, lo + 4096)
+            ob, og = oracle.encode(words[lo:hi])
+            want_b, want_g = torch.from_numpy(ob).to(dtype).view(bits), torch.from_numpy(og).to(dtype).view(bits)
+            assert torch.equal(board[lo:hi].contiguous().view(bits).cpu(), want_b), (n, lo)
+            assert torch.equal(glob[lo:hi].view(bits).cpu(), want_g), (n, lo)
+
+
+@pytest.mark.parametrize("dtype,cl", ENCODE_KINDS)
+def test_encode_is_one_launch(hb, encode_pool, dtype, cl):
+    """hz_encode is one kernel launch for every non-empty batch, whatever its size and the output's alignment"""
+    before = hb.launch_count()
+    hb.encode(dev(encode_pool[:0]), dtype=dtype, channels_last=cl)
+    assert hb.launch_count() == before
+    launches = {}
+    for n in ENCODE_SIZES:
+        st = dev(encode_pool[:n])
+        for off in _offsets(dtype):
+            before = hb.launch_count()
+            _encode_into(hb, st, dtype, cl, off)
+            launches[(n, off)] = hb.launch_count() - before
+    assert launches == {k: 1 for k in launches}
+
+
 def test_golden_weird_states(hb):
     """non-standard states the reference accepts through initial_state: ragged piles, leftover
     hands, nearly empty bags (partial piles, multi-pile replenish, bag-empty end), stray flags"""

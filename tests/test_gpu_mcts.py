@@ -160,21 +160,19 @@ def test_select_outputs_leaf_encoding(mods, oracle):
     value = torch.empty(n, device="cuda")
     leaf = torch.empty((n, 32), dtype=torch.int32, device="cuda")
     for s in range(sims):
-        for dtype, cl in ((torch.float32, False), (torch.bfloat16, True)):
-            board = torch.empty((n, 38, 5, 7), dtype=dtype, device="cuda",
-                                memory_format=torch.channels_last if cl else torch.contiguous_format)
-            glob = torch.empty((n, 42), dtype=dtype, device="cuda")
-            t.select(2.0, board, glob, leaf, dtype=dtype, channels_last=cl)
-            b2, g2 = hb.encode(leaf, dtype=dtype, channels_last=cl)
-            assert torch.equal(board, b2) and torch.equal(glob, g2)
-            if dtype == torch.float32:
-                ob, og = oracle.encode(leaf.cpu().numpy().view(np.uint32))
-                assert np.array_equal(board.cpu().numpy(), ob) and np.array_equal(glob.cpu().numpy(), og)
-        # 40-channel padded NHWC variant (two zero channels) used by the self-play stem
-        b40 = torch.full((n, 40, 5, 7), 7.0, dtype=torch.bfloat16, device="cuda").contiguous(memory_format=torch.channels_last)
-        g40 = torch.empty((n, 42), dtype=torch.bfloat16, device="cuda")
-        t.select(2.0, b40, g40, leaf, dtype=torch.bfloat16, channels_last=True, pad40=True)
-        assert torch.equal(b40[:, :38].contiguous(), board.contiguous()) and (b40[:, 38:] == 0).all() and torch.equal(g40, glob)
+        # every (dtype, layout) but T16K (test_leaf_encoder_writes_the_stem_image); pad40 is the 40-channel NHWC
+        # layout (channels 38 and 39 written as zero) that the self-play stem reads
+        for dtype in (torch.float32, torch.bfloat16):
+            for cl, pad40 in ((False, False), (True, False), (True, True)):
+                board = torch.full((n, 40 if pad40 else 38, 5, 7), 7.0, dtype=dtype, device="cuda").contiguous(
+                    memory_format=torch.channels_last if cl else torch.contiguous_format)
+                glob = torch.empty((n, 42), dtype=dtype, device="cuda")
+                t.select(2.0, board, glob, leaf, dtype=dtype, channels_last=cl, pad40=pad40)
+                b2, g2 = hb.encode(leaf, dtype=dtype, channels_last=cl)
+                assert torch.equal(board[:, :38], b2) and (board[:, 38:] == 0).all() and torch.equal(glob, g2)
+                if dtype == torch.float32:
+                    ob, og = oracle.encode(leaf.cpu().numpy().view(np.uint32))
+                    assert np.array_equal(board[:, :38].cpu().numpy(), ob) and np.array_equal(glob.cpu().numpy(), og)
         t.fake_eval(policy, value)
         # synthetic evaluator == packed.fake_eval of the leaf's exact hash
         if s == 3:
