@@ -75,10 +75,14 @@ __host__ __device__ __forceinline__ uint64_t rand64(uint64_t key, uint64_t ctr) 
 }
 // The inner mix depends on the counter only, and counters are small (move numbers < 200, draw
 // events*8+k < 400): a per-block shared table of the first RTAB_N inner values halves the cost
-// of every random number in the fused playout.  RandTab() computes it.
+// of every random number in the fused playout.  The values are a compile-time table (RAND_TAB_G, gen_tables.py); a block
+// copies them to shared memory with coalesced 16-byte loads (4 per thread at 64 threads) instead of computing 512 mix64.
 constexpr int RTAB_N = 512;
-__device__ __forceinline__ void build_rand_table(uint64_t* rtab) {
-    for (int i = threadIdx.x; i < RTAB_N; i += blockDim.x) rtab[i] = mix64((uint64_t)i + 0x9E3779B97F4A7C15ull);
+static_assert(sizeof(RAND_TAB_G) == RTAB_N * sizeof(uint64_t), "hz_tables.inc: RAND_TAB_G has RTAB_N entries");
+__device__ __forceinline__ void build_rand_table(uint64_t* rtab) {   // rtab: 16-byte aligned
+    const uint4* src = reinterpret_cast<const uint4*>(RAND_TAB_G);
+    uint4* dst = reinterpret_cast<uint4*>(rtab);
+    for (int e = threadIdx.x; e < RTAB_N / 2; e += blockDim.x) dst[e] = src[e];
 }
 // The table is handed around as its 32-bit shared-window address (0: no table, compute): through a generic pointer the
 // compiler rebuilds the window address (S2R SR_CgaCtaId + LEA) in front of every lookup.
@@ -260,28 +264,21 @@ __device__ __forceinline__ void legal_words(const Legal& L, uint32_t out[5]) {
     out[2] = (uint32_t)mid; out[3] = (uint32_t)(mid >> 32);
     out[4] = hi;
 }
-__host__ __device__ constexpr uint32_t nib_sel(int k) {
-    uint32_t t = 0;
-    for (uint32_t y = 0; y < 16; y++) {
-        int c = 0;
-        for (uint32_t b = 0; b < 4; b++)
-            if ((y >> b) & 1u) { if (c == k) t |= b << (2 * y); c++; }
-    }
-    return t;
-}
-// position of the k-th (0-based) set bit of m; k < popc(m)
+// position of the k-th (0-based) set bit of a 23-bit mask m; k < popc(m)
 __device__ __forceinline__ int nth_set_bit(uint32_t m, int k) {
-    int pos = 0, c;
-    c = __popc(m & 0xFFFFu); if (k >= c) { k -= c; pos += 16; m >>= 16; }
-    c = __popc(m & 0xFFu);   if (k >= c) { k -= c; pos += 8;  m >>= 8; }
+    // the byte by cumulative counts (the trick of draw_tile): bytes 1 and 2 of e hold the set bits of bytes 0 and 0..1, and
+    // bit 7 of each byte of d says k reached that count (all counts and k are < 128: no borrow between bytes)
+    const uint32_t e = (uint32_t)__popc(m & 0xFFu) * 0x100u + (uint32_t)__popc(m & 0xFFFFu) * 0x10000u;
+    const uint32_t d = (((uint32_t)k * 0x01010100u) | 0x80808000u) - e;
+    const uint32_t j = __popc(d & 0x00808000u);
+    k -= (int)__byte_perm(e, 0u, j);                                   // byte j of e: the set bits below byte j (byte 0 is 0)
+    int pos = 8 * (int)j, c;
+    m >>= pos;
     c = __popc(m & 0xFu);    if (k >= c) { k -= c; pos += 4;  m >>= 4; }
-    // the last nibble by table: NIB_SEL(k) holds, 2 bits per nibble value, the position of its k-th set bit
-    constexpr uint32_t S0 = nib_sel(0), S1 = nib_sel(1), S2 = nib_sel(2), S3 = nib_sel(3);
-    uint32_t tab;   // S[k] by three selects (written as selp: the compiler turns the ternary chain into a jump table)
-    asm("{\n\t.reg .pred p1, p2, p3;\n\tsetp.eq.s32 p1, %1, 1;\n\tsetp.eq.s32 p2, %1, 2;\n\tsetp.eq.s32 p3, %1, 3;\n\t"
-        "selp.u32 %0, %3, %2, p1;\n\tselp.u32 %0, %4, %0, p2;\n\tselp.u32 %0, %5, %0, p3;\n\t}"
-        : "=&r"(tab) : "r"(k), "n"(S0), "n"(S1), "n"(S2), "n"(S3));
-    return pos + (int)((tab >> (2u * (m & 0xFu))) & 3u);
+    // in the last nibble the same way: byte i of pre = set bits of the nibble's bits 0..i (the multiply by 0x204081 moves
+    // bit i to bit 8i without carries), and the k-th set bit is at the number of those counts <= k
+    const uint32_t pre = (((m & 0xFu) * 0x204081u) & 0x01010101u) * 0x01010101u;
+    return pos + __popc(((((uint32_t)k * 0x01010101u) | 0x80808080u) - pre) & 0x80808080u);
 }
 // k-th legal action in ascending action-index order; k < legal_count(L)
 __device__ __forceinline__ int kth_action(const Legal& L, int k) {
@@ -705,28 +702,36 @@ __device__ __forceinline__ uint32_t place_random(uint32_t* b, uint32_t& hand, ui
     const uint32_t T0 = b[3] | (b[0] & ~t.occ1), T1 = b[4] | (b[1] & ~t.occ1), T2 = b[5] | (b[2] & ~t.occ1);
     const uint32_t x1 = T0 & T1 & ~T2 & ~t.occ2, x3 = ~T0 & ~T1 & T2 & ~t.occ2;                 // wood / stone top, h <= 2: :183, :186
     const uint32_t x4 = ((b[0] & b[1] & ~b[2]) | (~b[1] & b[2])) & ~t.occ1;                     // wood, stone or building at h == 1: :190-192
-    const uint32_t m0 = (hand & 0x003) ? empty : 0, m1 = (hand & 0x00C) ? (empty | x1) : 0, m2 = (hand & 0x030) ? empty : 0;
-    const uint32_t m3 = (hand & 0x0C0) ? (empty | x3) : 0, m4 = (hand & 0x300) ? (empty | x4) : 0, m5 = (hand & 0xC00) ? empty : 0;
-    const int c0 = __popc(m0), c1 = c0 + __popc(m1), c2 = c1 + __popc(m2), c3 = c2 + __popc(m3), c4 = c3 + __popc(m4);
-    const int n = c4 + __popc(m5);
-    const int k = (int)__umulhi(rh, (uint32_t)n);
-    // the type whose cumulative count covers k: the five comparisons are monotone, each one moves (type, mask, base) on
-    int tile = 0, below = 0;
-    uint32_t m = m0;
-    if (k >= c0) { tile = 1; m = m1; below = c0; }
-    if (k >= c1) { tile = 2; m = m2; below = c1; }
-    if (k >= c2) { tile = 3; m = m3; below = c2; }
-    if (k >= c3) { tile = 4; m = m4; below = c3; }
-    if (k >= c4) { tile = 5; m = m5; below = c4; }
+    // Type t's legal set is m_t = empty | x_t (x_0 = x_2 = x_5 = 0) if the hand holds t, else empty.  x1, x3 and x4 lie
+    // inside occ0 because records are gap-free (level l + 1 is occupied only where level l is; the stacking masks above
+    // assume it too), so popc(m_t) = h_t * (popc(empty) + popc(x_t)): four popcounts, and the counts are summed as bytes
+    // by multiplications.  Byte t of clo is the count of types 0..t, cum4 and n those of types 0..4 and 0..5 (n <= 138).
+    const uint32_t pe = __popc(empty);
+    const uint32_t hf = (hand | (hand >> 1)) & 0x555u;                    // bit 2t: the hand holds type t
+    const uint32_t f03 = ((hf & 0x55u) * 0x41041u) & 0x01010101u;         // byte t: h_t, t = 0..3
+    const uint32_t f45 = ((hf >> 8) * 0x41u) & 0x0101u;                   // byte t - 4: h_t, t = 4, 5
+    const uint32_t clo = ((f03 * 0xFFu) & (pe * 0x01010101u + (uint32_t)__popc(x1) * 0x100u + (uint32_t)__popc(x3) * 0x1000000u)) * 0x01010101u;
+    const uint32_t c45 = (f45 * 0xFFu) & (pe * 0x0101u + (uint32_t)__popc(x4));
+    const uint32_t cum4 = (clo >> 24) + (c45 & 0xFFu), n = cum4 + (c45 >> 8);
+    const uint32_t k = __umulhi(rh, n);
+    // the type whose cumulative count covers k: the number of counts <= k, four of them at once as bytes (they are <= 92;
+    // k is capped at 127 so that bit 7 of each byte of the difference says count <= k, with no borrow between bytes)
+    const uint32_t d = ((min(k, 127u) * 0x01010101u) | 0x80808080u) - clo;
+    const uint32_t tile = __popc(d & 0x80808080u) + (k >= cum4 ? 1u : 0u);
+    // the types before it: byte `tile` of (cum4, cum3 | cum2, cum1, cum0, 0)
+    const uint32_t below = __byte_perm(clo << 8, __byte_perm(clo, cum4, 0x43u), tile);
+    const uint32_t m = empty | (tile == 1u ? x1 : 0u) | (tile == 3u ? x3 : 0u) | (tile == 4u ? x4 : 0u);
     const uint32_t any = n != 0;                                      // shifts, not selects: a select here becomes a branch
-    const uint32_t bit = any << nth_set_bit(m, k - below);
-    // place the tile on level h of the hex (:257,275)
-    const uint32_t code = (uint32_t)tile + 1u;
-    const uint32_t lvl1 = t.occ0 & ~t.occ1;
+    const uint32_t bit = any << nth_set_bit(m, (int)(k - below));
+    // place the tile on level h of the hex (:257,275): the hex's bit goes into the planes of the code's set bits.  The hex
+    // is free at level h (it is not in occ2: x1 and x3 exclude it, x4 excludes occ1), so adding the bit is or-ing it, and
+    // the multiply-adds run on the FMA pipe
+    const uint32_t code = tile + 1u;
+    const uint32_t at[3] = {bit & empty, bit & t.occ0 & ~t.occ1, bit & t.occ1};
 #pragma unroll
     for (int q = 0; q < 3; q++) {
-        const uint32_t bq = (code & (1u << q)) ? bit : 0u;            // the hex in the planes of the code's set bits
-        b[q] |= bq & ~t.occ0; b[3 + q] |= bq & lvl1; b[6 + q] |= bq & t.occ1;
+        const uint32_t cq = (code >> q) & 1u;
+        b[q] += at[0] * cq; b[3 + q] += at[1] * cq; b[6 + q] += at[2] * cq;
     }
     hand -= any << (2 * tile);                                        // hand.remove, :250
     return bit;

@@ -264,7 +264,7 @@ __global__ void __launch_bounds__(PTPB, 7) k_playout(void* states, int64_t n, in
                                                   unsigned long long* total_steps, const uint64_t* keys,
                                                   uint64_t seed, uint64_t first_id, uint32_t* results) {
     __shared__ NbrLut lut;
-    __shared__ uint64_t rtab_s[RTAB_N];
+    __shared__ __align__(16) uint64_t rtab_s[RTAB_N];
     __shared__ WaterQueue<2 * PTPB, 2 * PTPB> wq;
     build_nbr_lut(&lut);
     build_rand_table(rtab_s);

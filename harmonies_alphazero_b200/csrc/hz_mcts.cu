@@ -526,7 +526,7 @@ __global__ void __launch_bounds__(RTPB, 7) k_tree_rollout_eval(hz_tree T, int lo
     const int64_t rows = (int64_t)active_trees(T) * T.leaves;
     if ((int64_t)blockIdx.x * RTPB >= (rows << log2r)) return;      // the whole block lies past the active rows
     __shared__ NbrLut lut;
-    __shared__ uint64_t rtab_s[RTAB_N];
+    __shared__ __align__(16) uint64_t rtab_s[RTAB_N];
     __shared__ WaterQueue<2 * RTPB, 2 * RTPB> wq;
     __shared__ int warp_sum[RTPB / 32];
     build_nbr_lut(&lut);
