@@ -481,8 +481,10 @@ __device__ __forceinline__ uint32_t draw_tile(uint32_t& lo, uint32_t& hi, uint32
     uint32_t r = (x * total) >> 21;                                  // 21+7 bits < 32
     uint32_t clo = lo * 0x01010101u;                                 // byte k = sum of bytes 0..k (totals <= 255: no carries)
     uint32_t c4 = (clo >> 24) + (hi & 0xFFu);
-    uint32_t rr = r * 0x01010101u;
-    int t = __popc(__vcmpleu4(clo, rr) & 0x01010101u) + (c4 <= r ? 1 : 0);
+    // types 0..3 whose cumulative count is <= r, four at once: bit 7 of each byte of the difference is set exactly there (a
+    // bag holds at most 120 tiles, so r and the counts are < 128 and no byte borrows; __vcmpleu4 is emulated on sm_100a)
+    uint32_t rr = (r * 0x01010101u) | 0x80808080u;
+    int t = __popc((rr - clo) & 0x80808080u) + (c4 <= r ? 1 : 0);
     lo -= shl_clamped(1u, 8u * (uint32_t)t);                         // t >= 4: shifted out
     hi -= shl_clamped(1u, 8u * (uint32_t)t - 32u);                   // t < 4: the count wraps to >= 32, shifted out
     return 1u << (2 * t);
@@ -720,7 +722,10 @@ __device__ __forceinline__ uint32_t place_random(uint32_t* b, uint32_t& hand, ui
     const uint32_t tile = __popc(d & 0x80808080u) + (k >= cum4 ? 1u : 0u);
     // the types before it: byte `tile` of (cum4, cum3 | cum2, cum1, cum0, 0)
     const uint32_t below = __byte_perm(clo << 8, __byte_perm(clo, cum4, 0x43u), tile);
-    const uint32_t m = empty | (tile == 1u ? x1 : 0u) | (tile == 3u ? x3 : 0u) | (tile == 4u ? x4 : 0u);
+    // the type's legal set: empty plus its stacking set, picked by the flags (tile == 1, 3, 4) as byte `tile` of three
+    // constants (tile <= 5); the sets are disjoint from empty and one flag at most is set, so multiply-adds do the or-ing
+    const uint32_t m = empty + x1 * __byte_perm(0x100u, 0u, tile) + x3 * __byte_perm(0x1000000u, 0u, tile) +
+                       x4 * __byte_perm(0u, 1u, tile);
     const uint32_t any = n != 0;                                      // shifts, not selects: a select here becomes a branch
     const uint32_t bit = any << nth_set_bit(m, (int)(k - below));
     // place the tile on level h of the hex (:257,275): the hex's bit goes into the planes of the code's set bits.  The hex
