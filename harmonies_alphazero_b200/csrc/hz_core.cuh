@@ -474,15 +474,15 @@ __device__ __forceinline__ uint32_t shl_clamped(uint32_t v, uint32_t n) {   // v
     asm("shl.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
     return r;
 }
-// draw j (0..2) of a pile from a bag of `total` > 0 tiles, the bag as two 32-bit halves (types 0..3 | 4,5): the
+// draw j (0..2) of a pile from a bag of 0 < `total` <= 127 tiles, the bag as two 32-bit halves (types 0..3 | 4,5): the
 // cumulative counts and the decrement stay 32-bit operations.  Returns the tile's increment of the pile code.
 __device__ __forceinline__ uint32_t draw_tile(uint32_t& lo, uint32_t& hi, uint32_t total, uint64_t z, int j) {
     uint32_t x = (uint32_t)(z >> (21 * j)) & 0x1FFFFFu;
     uint32_t r = (x * total) >> 21;                                  // 21+7 bits < 32
     uint32_t clo = lo * 0x01010101u;                                 // byte k = sum of bytes 0..k (totals <= 255: no carries)
     uint32_t c4 = (clo >> 24) + (hi & 0xFFu);
-    // types 0..3 whose cumulative count is <= r, four at once: bit 7 of each byte of the difference is set exactly there (a
-    // bag holds at most 120 tiles, so r and the counts are < 128 and no byte borrows; __vcmpleu4 is emulated on sm_100a)
+    // types 0..3 whose cumulative count is <= r, four at once: bit 7 of each byte of the difference is set exactly there
+    // (total <= 127, so r and the counts are < 128 and no byte borrows; __vcmpleu4 is emulated on sm_100a)
     uint32_t rr = (r * 0x01010101u) | 0x80808080u;
     int t = __popc((rr - clo) & 0x80808080u) + (c4 <= r ? 1 : 0);
     lo -= shl_clamped(1u, 8u * (uint32_t)t);                         // t >= 4: shifted out
@@ -492,6 +492,20 @@ __device__ __forceinline__ uint32_t draw_tile(uint32_t& lo, uint32_t& hi, uint32
 __device__ __forceinline__ uint32_t draw_pile(uint64_t& bag, uint64_t z) {
     uint32_t lo = (uint32_t)bag, hi = (uint32_t)(bag >> 32), code = 0;
     int total = bag_total(bag);
+    if (total > 127) {
+        // A game's bag never holds more than 120 tiles, but a record may carry up to 255 of each type (pack_fields): past
+        // draw_tile's range, three draws by the plain cumulative loop of the specification (x * total < 2^21 * 1530 < 2^32).
+#pragma unroll
+        for (int j = 0; j < 3; j++, total--) {
+            const uint32_t r = (((uint32_t)(z >> (21 * j)) & 0x1FFFFFu) * (uint32_t)total) >> 21;
+            int t = 0;
+            uint32_t cum = (uint32_t)bag & 0xFFu;                    // count of types 0..t
+            while (t < 5 && cum <= r) cum += (uint32_t)(bag >> (8 * ++t)) & 0xFFu;
+            bag -= 1ull << (8 * t);
+            code += 1u << (2 * t);
+        }
+        return code;
+    }
 #pragma unroll
     for (int j = 0; j < 3; j++) {
         if (total > 0) {
@@ -502,7 +516,7 @@ __device__ __forceinline__ uint32_t draw_pile(uint64_t& bag, uint64_t z) {
     bag = (uint64_t)lo | ((uint64_t)hi << 32);
     return code;
 }
-// draw_pile from a bag of total >= 3 tiles: always three draws, no branch
+// draw_pile from a bag of 3 <= total <= 127 tiles: always three draws, no branch
 __device__ __forceinline__ uint32_t draw_pile3(uint32_t& lo, uint32_t& hi, uint32_t total, uint64_t z) {
     uint32_t code = draw_tile(lo, hi, total, z, 0);                  // (three statements: each draw sees the bag the last left)
     code += draw_tile(lo, hi, total - 1u, z, 1);
@@ -785,7 +799,8 @@ __device__ __forceinline__ bool playout_step(State& s, const NbrLut* lut, RandTa
 // hand from the first chain.  playout_round() is one straight-line body over registers that the compiler can interleave,
 // and writes the record once; playout_step runs them one after the other with a branch on phase and player per action.
 // The straight line covers the regular round: every placement has a legal hex and each top-up draws three tiles from a
-// bag of >= 3.  Anything else returns false with s untouched, and the caller plays the round with playout_step.
+// bag of 3..127 (draw_pile3's range; a game's bag never holds more than 120).  Anything else returns false with s
+// untouched, and the caller plays the round with playout_step.
 // Same draws, same result as eight playout_step<P, true> calls; the final scoring is left to the caller as there.
 __device__ __forceinline__ bool round_ready(const State& s) {
     // the rand table covers every counter of the round (moves+7, (ev+1)*8 < RTAB_N)
@@ -812,7 +827,7 @@ __device__ __forceinline__ bool playout_round(State& s, RandTab rtab) {
     uint32_t b0[9], b1[9];
 #pragma unroll
     for (int q = 0; q < 9; q++) { b0[q] = s.w[q]; b1[q] = s.w[9 + q]; }
-    bool ok = total >= 6u;
+    bool ok = total - 6u <= 127u - 6u;                               // 6 <= total <= 127
 #pragma unroll
     for (int i = 1; i <= 3; i++) {
         ok &= place_random(b0, hand0, rh[i]) != 0u;

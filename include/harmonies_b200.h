@@ -44,6 +44,19 @@
  *  w[27]      number of actions applied so far (game_move_count, trainer.py:466,509)
  *  w[28..31]  reserved, zero
  *
+ *  What the kernels assume of a record (packed.pack_fields produces nothing else):
+ *   - stacks without gaps: level l+1 of a hex holds a tile only where level l does.  Every
+ *     kernel that reads a board assumes it (the stacking masks, place_random's counts); a
+ *     gapped record is outside the format, not a supported input.  pack_fields builds the
+ *     planes from stack lists, so it cannot produce one.
+ *   - piles and hand: 2-bit counts (at most 3 tiles of a type).  The engine kernels take any
+ *     such code; pack_fields also caps a pile and the hand at 3 tiles in all.
+ *   - bag: any count 0..255 per type (pack_fields accepts exactly that range).  Every draw
+ *     (hz_apply, hz_end_turn, hz_replenish_piles, hz_draw_tiles, in-tree expansion, the fused
+ *     playouts) follows the rule below for any such bag; a game's bag never holds more than
+ *     120 tiles, and the fused playout's whole-round path takes bags of 6..127 tiles only.
+ *   - counters: w[26] and w[27] may take any uint32 value and wrap modulo 2^32.
+ *
  *  Canonical identity (get_canonical_tuple, harmonies_engine.py:81-110) = words 0..22 with
  *  the ending flag and winner bits masked out (meta & 0x0F).
  *
