@@ -614,12 +614,39 @@ static int tree_find_or_add(otree *t, const uint32_t *w, uint64_t h, int *was_ne
     return id;
 }
 
+/* Whole-tree copy of a finished search (tests compare it node for node with the device arenas).
+ * Caller-owned arrays of cap_nodes / cap_edges entries; nodes in creation order, edges in
+ * append order, so ids are the tree's own.  Entries past the caps are not copied. */
+typedef struct {
+    int cap_nodes, cap_edges;
+    uint32_t *words;                                   /* [cap_nodes * 32] */
+    uint64_t *hash;                                    /* tree key */
+    int32_t *first_edge, *n_edges, *player;
+    int32_t *child, *N, *action, *mover, *V;
+    double *W;
+    float *P;
+} hzo_tree_dump;
+
+static void dump_tree(const otree *t, hzo_tree_dump *d) {
+    if (!d) return;
+    for (int i = 0; i < t->n_nodes && i < d->cap_nodes; i++) {
+        const onode *nd = &t->nodes[i];
+        memcpy(d->words + (size_t)i * 32, nd->w, sizeof nd->w);
+        d->hash[i] = nd->hash; d->first_edge[i] = nd->first_edge; d->n_edges[i] = nd->n_edges; d->player[i] = nd->player;
+    }
+    for (int i = 0; i < t->n_edges && i < d->cap_edges; i++) {
+        const oedge *e = &t->edges[i];
+        d->child[i] = e->child; d->N[i] = e->N; d->W[i] = e->W; d->P[i] = e->P;
+        d->action[i] = e->action; d->mover[i] = e->mover; d->V[i] = e->V;
+    }
+}
+
 /* One full search = get_best_action_and_pi (MCTS.py:272-381) up to the root statistics.
- * Outputs (each [143], indexed by action, nullable): N, W, P, child.  Returns 0 or -1 on
- * arena overflow. */
+ * Outputs (each [143], indexed by action, nullable): N, W, P, child; `dump` (nullable) receives
+ * the whole tree.  Returns 0 or -1 on arena overflow. */
 int hzo_search(const uint32_t *root, uint64_t search_key, int sims, double cpuct, int key_mode,
                const float *noise, double eps, hzo_eval_fn eval, void *user, int32_t *outN, double *outW, float *outP,
-               int32_t *out_child, int32_t *out_nodes, int32_t *out_edges) {
+               int32_t *out_child, int32_t *out_nodes, int32_t *out_edges, hzo_tree_dump *dump) {
     geometry();
     if (!eval) eval = fake_eval;
     otree t;
@@ -716,6 +743,7 @@ int hzo_search(const uint32_t *root, uint64_t search_key, int sims, double cpuct
     }
     if (out_nodes) *out_nodes = t.n_nodes;
     if (out_edges) *out_edges = t.n_edges;
+    dump_tree(&t, dump);
     free(t.nodes); free(t.edges); free(t.table); free(path);
     return rc;
 }
@@ -731,7 +759,7 @@ int hzo_search(const uint32_t *root, uint64_t search_key, int sims, double cpuct
  * hzo_search (the reference's sequential search). */
 int hzo_search_vl(const uint32_t *root, uint64_t search_key, int steps, int leaves, double cpuct, int key_mode,
                   const float *noise, double eps, hzo_eval_fn eval, void *user, int32_t *outN, double *outW,
-                  float *outP, int32_t *out_child, int32_t *out_nodes, int32_t *out_edges) {
+                  float *outP, int32_t *out_child, int32_t *out_nodes, int32_t *out_edges, hzo_tree_dump *dump) {
     geometry();
     if (!eval) eval = fake_eval;
     int sims = steps * leaves;
@@ -840,6 +868,7 @@ int hzo_search_vl(const uint32_t *root, uint64_t search_key, int steps, int leav
     }
     if (out_nodes) *out_nodes = t.n_nodes;
     if (out_edges) *out_edges = t.n_edges;
+    dump_tree(&t, dump);
     free(t.nodes); free(t.edges); free(t.table); free(path); free(depth); free(leafs);
     return rc;
 }
@@ -869,7 +898,7 @@ static void *search_worker(void *arg) {
     search_job *j = (search_job *)arg;
     for (int64_t g = j->lo; g < j->hi; g++)
         hzo_search(j->roots + g * 32, j->keys[g], j->sims, j->cpuct, HZ_KEY_REFERENCE, NULL, 0.0, NULL, NULL,
-                   j->N ? j->N + g * HZ_ACTION_SIZE : NULL, NULL, NULL, NULL, NULL, NULL);
+                   j->N ? j->N + g * HZ_ACTION_SIZE : NULL, NULL, NULL, NULL, NULL, NULL, NULL);
     return NULL;
 }
 /* many independent searches with the synthetic evaluator, for CPU-baseline timing */

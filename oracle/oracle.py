@@ -125,9 +125,24 @@ def playout(states, max_steps=1000, n_threads=1):
     return s, steps, int(total)
 
 
-def search(root, search_key, sims, cpuct, noise=None, eps=0.0, eval_fn=None, key_mode=1, leaves=1):
+class _TreeDump(C.Structure):
+    _fields_ = [("cap_nodes", C.c_int), ("cap_edges", C.c_int)] + [
+        (f, C.c_void_p) for f in ("words", "hash", "first_edge", "n_edges", "player", "child", "N", "action", "mover", "V", "W", "P")
+    ]
+
+
+_DUMP_TYPES = {"words": (np.uint32, 32), "hash": (np.uint64, 0), "first_edge": (np.int32, 0), "n_edges": (np.int32, 0),
+               "player": (np.int32, 0), "child": (np.int32, 0), "N": (np.int32, 0), "action": (np.int32, 0),
+               "mover": (np.int32, 0), "V": (np.int32, 0), "W": (np.float64, 0), "P": (np.float32, 0)}
+_NODE_FIELDS = ("words", "hash", "first_edge", "n_edges", "player")
+
+
+def search(root, search_key, sims, cpuct, noise=None, eps=0.0, eval_fn=None, key_mode=1, leaves=1, tree=False, vl=None):
     """One reference-semantics search.  eval_fn(words[32]) -> (p[143] float32, v float) or
-    None for the synthetic evaluator.  Returns dict(N, W, P, child, n_nodes, n_edges, rc)."""
+    None for the synthetic evaluator.  Returns dict(N, W, P, child, n_nodes, n_edges, rc).
+    leaves > 1 (or vl=True) runs the virtual-loss schedule (hzo_search_vl, sims // leaves rounds).
+    tree=True adds "tree": the whole arena as numpy arrays, nodes in creation order (words [n, 32],
+    hash, first_edge, n_edges, player) and edges in append order (child, N, W, P, action, mover, V)."""
     r = np.ascontiguousarray(root, dtype=np.uint32).reshape(32)
     N = np.zeros(143, dtype=np.int32)
     W = np.zeros(143, dtype=np.float64)
@@ -145,18 +160,30 @@ def search(root, search_key, sims, cpuct, noise=None, eps=0.0, eval_fn=None, key
             vp[0] = float(v)
 
         cb = EVAL_FN(_cb)
-    if leaves == 1:
+    dump, arrays = None, {}
+    if tree:   # the oracle's arena capacities (hzo_search)
+        caps = (1 + 69 * sims, 69 * sims + 1)
+        for f, (dt, w) in _DUMP_TYPES.items():
+            cap = caps[0] if f in _NODE_FIELDS else caps[1]
+            arrays[f] = np.zeros((cap, w) if w else cap, dtype=dt)
+        dump = _TreeDump(caps[0], caps[1], *(arrays[f].ctypes.data for f, _ in _TreeDump._fields_[2:]))
+    pd = None if dump is None else C.byref(dump)
+    if not (leaves > 1 if vl is None else vl):
+        assert leaves == 1
         rc = lib().hzo_search(
             _p(r), C.c_uint64(int(search_key)), C.c_int(sims), C.c_double(cpuct), C.c_int(key_mode), _p(nz), C.c_double(eps),
-            cb, None, _p(N), _p(W), _p(P), _p(child), C.byref(nn), C.byref(ne),
+            cb, None, _p(N), _p(W), _p(P), _p(child), C.byref(nn), C.byref(ne), pd,
         )
     else:   # virtual-loss mode: sims must be a multiple of leaves (sims // leaves rounds)
         assert sims % leaves == 0
         rc = lib().hzo_search_vl(
             _p(r), C.c_uint64(int(search_key)), C.c_int(sims // leaves), C.c_int(leaves), C.c_double(cpuct), C.c_int(key_mode),
-            _p(nz), C.c_double(eps), cb, None, _p(N), _p(W), _p(P), _p(child), C.byref(nn), C.byref(ne),
+            _p(nz), C.c_double(eps), cb, None, _p(N), _p(W), _p(P), _p(child), C.byref(nn), C.byref(ne), pd,
         )
-    return {"N": N, "W": W, "P": P, "child": child, "n_nodes": nn.value, "n_edges": ne.value, "rc": rc}
+    out = {"N": N, "W": W, "P": P, "child": child, "n_nodes": nn.value, "n_edges": ne.value, "rc": rc}
+    if tree:
+        out["tree"] = {f: a[: nn.value if f in _NODE_FIELDS else ne.value] for f, a in arrays.items()}
+    return out
 
 
 def choose(N, u=0.0, exploratory=False):
