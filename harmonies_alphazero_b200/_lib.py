@@ -31,11 +31,15 @@ SIGNATURES = {
     "hz_greedy_actions": (_i, [_vp, _i64, _vp, _vp]),
     "hz_playout": (_i, [_vp, _i64, _i, _vp, _vp, _vp]),
     "hz_playout_keys": (_i, [_vp, _i64, _u64, _u64, _i, _vp, _vp, _vp]),
+    "hz_sym_states": (_i, [_vp, _i64, _vp, _vp, _vp]),
+    "hz_sym_actions": (_i, [_vp, _i64, _i, _vp, _vp, _i, _vp, _vp]),
     "hz_tree_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i]),
     "hz_tree_create": (_i, [C.POINTER(_vp), _vp, C.c_size_t, _i, _i, _i, _i, _i]),
     "hz_tree_destroy": (_i, [_vp]),
     "hz_tree_reset": (_i, [_vp, _vp, _vp, _vp]),
     "hz_tree_set_active": (_i, [_vp, _vp]),
+    "hz_tree_set_symmetry": (_i, [_vp, _i]),
+    "hz_tree_leaf_frames": (_i, [_vp, _vp, _vp]),
     "hz_tree_select": (_i, [_vp, _f, _vp, _vp, _vp, _i, _i, _vp]),
     "hz_tree_expand_backup": (_i, [_vp, _vp, _vp, _i, _vp, _d, _vp]),
     "hz_tree_fake_eval": (_i, [_vp, _vp, _vp, _vp]),

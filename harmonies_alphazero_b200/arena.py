@@ -39,13 +39,16 @@ def _search(tree, net, states, sims, cpuct, bufs):
 GREEDY = "greedy"   # pass as either side to play the 1-ply greedy agent of evaluation.py instead of a network
 
 
-def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cuda", seed=0, key_mode=hb.KEY_REFERENCE, leaves=1):
+def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cuda", seed=0, key_mode=hb.KEY_REFERENCE, leaves=1,
+               symmetry=None):
     """Returns dict(candidate_wins, best_wins, draws, win_rate, games).  Each side is an
     InferenceNet on ``device``, ``arena.GREEDY`` (run_tournament of evaluation.py:7-65:
     AlphaZero vs the greedy agent, sides alternating by game index) or a
     ``selfplay.RolloutEvaluator`` (a network-free search of the same simulation count).  leaves > 1 switches the
     searches to the virtual-loss mode (K simulations in flight per tree): not the reference's
-    visit counts any more, but a 30-game match then fills the network batch K times better."""
+    visit counts any more, but a 30-game match then fills the network batch K times better.
+    symmetry: None, "board" or "full": both sides' networks see every leaf in a random symmetry frame
+    (BatchedMCTS.set_symmetry)."""
     dev = torch.device(device)
     sims, cpuct = int(mcts_config_eval["num_simulations"]), float(mcts_config_eval["cpuct"])
     # group 0: candidate is player 0 (even game indices); group 1: candidate is player 1
@@ -63,6 +66,7 @@ def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cud
         tree = bufs = None
         if searchers:                                                # greedy vs greedy needs no search arena
             tree = BatchedMCTS(n, sims, device=dev, key_mode=key_mode, leaves=leaves)
+            tree.set_symmetry(symmetry)
             rows = n * leaves
             both_tiles = all(x not in nets or getattr(x, "wants_tiles", False) for x in (candidate_net, best_net))
             if anynet is None:                   # rollouts only: priors and values, no leaf encoding

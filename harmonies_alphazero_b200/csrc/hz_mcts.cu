@@ -18,6 +18,7 @@
 
 #include "hz_common.cuh"
 #include "hz_core.cuh"
+#include "hz_sym.cuh"
 
 struct hz_tree {
     int n_trees, max_sims, max_nodes, max_edges, table_size, key_mode;
@@ -25,7 +26,7 @@ struct hz_tree {
     uint4* node_state;      // [n_trees * max_nodes * 8]
     uint64_t* node_hash;    // [n_trees * max_nodes]
     uint32_t* node_edge0;   // [n_trees * max_nodes]
-    uint32_t* node_info;    // [n_trees * max_nodes]  n_edges | player << 8
+    uint32_t* node_info;    // [n_trees * max_nodes]  n_edges | player << 8 (| frame << 16 under hz_tree_set_symmetry)
     uint32_t* edge_child;   // [n_trees * max_edges]
     int32_t* edge_N;
     double* edge_W;
@@ -45,6 +46,8 @@ struct hz_tree {
     uint64_t* search_key;
     size_t table_bytes;
     const int32_t* n_active;   // device word (nullable): only trees 0..*n_active-1 take part in reset / select / evaluate / expand
+    int sym_mode;           // HZ_SYM_* of the launches that follow (hz_tree_set_symmetry)
+    int frames_on;          // host side: the last hz_tree_select ran with a mode on
 };
 
 namespace hz {
@@ -148,7 +151,8 @@ __device__ __forceinline__ void warp_encode_fast40(const uint32_t* w, uint8_t* s
 }
 
 // ---- select: move_to_leaf (MCTS.py:63-149) + create_state_tensors(leaf) (MCTS.py:299) ---------
-template <typename OT, int LAYOUT>
+// G = order of the symmetry group of the leaf frames (0: off, the reference's select)
+template <typename OT, int LAYOUT, int G>
 __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, uint4* leaf_states, OT* board, OT* glob) {
     __shared__ uint32_t sm_words[WPB][32];
     __shared__ uint32_t sm_mask[WPB][40];
@@ -252,6 +256,21 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
         size_t row = (size_t)t * K + j;
         warp_load_words(sm_words[warp], v.node_state, node, lane);      // (__syncwarp inside: V updates are visible to the next descent)
         if (leaf_states) reinterpret_cast<uint32_t*>(leaf_states + row * 8)[lane] = sm_words[warp][lane];
+        if constexpr (G != 0) {                                          // the network sees T_g(leaf); the tree keeps its frame
+            const uint32_t* w = sm_words[warp];
+            const int g = sym_frame(w, T.search_key[t], G);
+            const uint32_t w22 = w[HZ_W_BAG1META], own = w[lane];
+            const uint32_t m = (w22 >> 16) & 0xFFu;
+            // the frame is a function of the node within a search: kept in the node's info word, bits 16..27 =
+            // g | n_piles << 9 (OR of the same value when the node is reached again; a new search creates new nodes)
+            if (lane == 0) atomicOr(&v.node_info[node], ((uint32_t)g | ((m < 5u ? m : 5u) << 9)) << 16);
+            if (board) {
+                const uint32_t nw = warp_sym_word(own, g, lane);
+                __syncwarp();
+                sm_words[warp][lane] = nw;
+                __syncwarp();
+            }
+        }
         if (board) {
             if constexpr (FAST40)
                 warp_encode_fast40<LAYOUT == HZ_LAYOUT_T16K>(sm_words[warp], sbytes[warp], vlut8, scell, (__nv_bfloat16*)board, row,
@@ -311,6 +330,14 @@ __device__ __forceinline__ void table_insert(const hz_tree& T, const TreeView& v
 #ifndef HZ_EXPAND_MIN_BLOCKS
 #define HZ_EXPAND_MIN_BLOCKS 4
 #endif
+// row entry of action a in the evaluator's frame fr (g | n_piles << 9, from the leaf's info word): sigma_g(a)
+__device__ __forceinline__ int frame_action(int a, uint32_t fr) {
+    const int g = (int)(fr & 0x1FFu), m = (int)(fr >> 9);
+    return sym_action(a, g & 3, m, a < m ? sym_pile_perm(g, m, false) : 0u, SYM_HEX_G);
+}
+
+// SYM: the leaf rows are in the frames of k_tree_select (hz_tree_set_symmetry); false = the reference's expansion
+template <bool SYM>
 __global__ void __launch_bounds__(TTPB, HZ_EXPAND_MIN_BLOCKS) k_tree_expand_backup(hz_tree T, const float* policy, const float* value,
                                                              int is_logits, const float* noise, double eps) {
     __shared__ uint32_t sm_words[WPB][32];
@@ -334,11 +361,17 @@ __global__ void __launch_bounds__(TTPB, HZ_EXPAND_MIN_BLOCKS) k_tree_expand_back
     const uint32_t* path = v.path + (size_t)j * (T.max_sims + 1);
     const float* prow = policy + row * HZ_ACTION_SIZE;
     float pl[5];
+    // SYM: the row is loaded through sigma_g (frame in the leaf's info word), so every lane holds what it holds with the mode off
+    uint32_t leaf_info = SYM ? v.node_info[leaf] : 0u;
+    const uint32_t fr = SYM ? leaf_info >> 16 : 0u;
 #pragma unroll
-    for (int i = 0; i < 5; i++) pl[i] = lane + 32 * i < HZ_ACTION_SIZE ? prow[lane + 32 * i] : -INFINITY;
+    for (int i = 0; i < 5; i++) {
+        const int a = lane + 32 * i;
+        pl[i] = a < HZ_ACTION_SIZE ? prow[SYM ? frame_action(a, fr) : a] : -INFINITY;
+    }
     const float val_f = value[row];
     const uint32_t pe = lane < depth ? path[lane] : 0u;
-    const uint32_t leaf_info = v.node_info[leaf];
+    if (!SYM) leaf_info = v.node_info[leaf];
     const uint64_t leaf_hash = v.node_hash[leaf];
     const uint64_t skey = T.search_key[t];
     int n_nodes = T.n_nodes[t];
@@ -442,7 +475,7 @@ __global__ void __launch_bounds__(TTPB, HZ_EXPAND_MIN_BLOCKS) k_tree_expand_back
                 int e = e0 + n_new_edges + __popc(valid_mask & ((1u << lane) - 1u));
                 HZ_BOUND(e, T.max_edges, 302);
                 HZ_BOUND(a, HZ_ACTION_SIZE, 303);
-                float p = prow[a];
+                float p = prow[SYM ? frame_action(a, fr) : a];
                 if (is_logits) p = expf(p - mx) * inv_sum;
                 if (mix) {
                     float keep = one_minus * p;                      // np.float32 product, :323
@@ -461,7 +494,7 @@ __global__ void __launch_bounds__(TTPB, HZ_EXPAND_MIN_BLOCKS) k_tree_expand_back
         }
         if (lane == 0 && !overflow && expand) {
             v.node_edge0[leaf] = (uint32_t)e0;
-            v.node_info[leaf] = (uint32_t)n_new_edges | ((uint32_t)leaf_player << 8);
+            v.node_info[leaf] = (uint32_t)n_new_edges | ((uint32_t)leaf_player << 8) | (SYM ? (leaf_info & 0xFFFF0000u) : 0u);
             T.n_nodes[t] = n_nodes;
             T.n_edges[t] = e0 + n_new_edges;
         }
@@ -493,6 +526,8 @@ __global__ void __launch_bounds__(TTPB, HZ_EXPAND_MIN_BLOCKS) k_tree_expand_back
 }
 
 // ---- synthetic evaluator (stands in for ModelManager.predict in tests / tree-only benches) -----
+// SYM: entry sigma_g(a) of the row gets what entry a gets with the mode off (the frame of k_tree_select)
+template <bool SYM>
 __global__ void __launch_bounds__(TTPB) k_tree_fake_eval(hz_tree T, float* policy, float* value) {
     __shared__ uint32_t sm_words[WPB][32];
     int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -505,8 +540,9 @@ __global__ void __launch_bounds__(TTPB) k_tree_fake_eval(hz_tree T, float* polic
         State s;
         state_from_words(s, sm_words[warp]);
         uint64_t h = canon_hash(s, HZ_KEY_EXACT);
+        const uint32_t fr = SYM ? v.node_info[T.leaf[row]] >> 16 : 0u;
         for (int a = lane; a < HZ_ACTION_SIZE; a += 32)
-            policy[row * HZ_ACTION_SIZE + a] = (float)(mix64(h ^ (uint64_t)(a + 1)) >> 40) * 0x1p-24f;
+            policy[row * HZ_ACTION_SIZE + (SYM ? frame_action(a, fr) : a)] = (float)(mix64(h ^ (uint64_t)(a + 1)) >> 40) * 0x1p-24f;
         if (lane == 0) value[row] = (float)((double)(mix64(h ^ 0x5EEDull) >> 40) * 0x1p-23 - 1.0);
         __syncwarp();
     }
@@ -520,6 +556,8 @@ __global__ void __launch_bounds__(TTPB) k_tree_fake_eval(hz_tree T, float* polic
 // 64-thread blocks under (64, 7) for the reason given at k_playout: the register cap leaves the round path room.
 constexpr int RTPB = 64;
 constexpr int ROLLOUT_MAX_STEPS = 1000;
+// SYM: the priors go into the frame of k_tree_select (entry sigma_g(a) gets what entry a gets with the mode off)
+template <bool SYM>
 __global__ void __launch_bounds__(RTPB, 7) k_tree_rollout_eval(hz_tree T, int log2r, float* policy, float* value,
                                                                unsigned long long* total_steps) {
     const int R = 1 << log2r;
@@ -553,10 +591,11 @@ __global__ void __launch_bounds__(RTPB, 7) k_tree_rollout_eval(hz_tree T, int lo
             uint32_t lw[5];
             legal_words(L, lw);
             const float p = n ? 1.0f / (float)n : 0.0f;
+            const uint32_t fr = SYM ? T.node_info[(size_t)t * T.max_nodes + leaf] >> 16 : 0u;
             for (int a = r; a < HZ_ACTION_SIZE; a += R) {
                 const int i = a >> 5;   // selects, not lw[i]: a dynamic index would put lw in local memory
                 const uint32_t w = i == 0 ? lw[0] : i == 1 ? lw[1] : i == 2 ? lw[2] : i == 3 ? lw[3] : lw[4];
-                policy[row * HZ_ACTION_SIZE + a] = ((w >> (a & 31)) & 1u) ? p : 0.0f;
+                policy[row * HZ_ACTION_SIZE + (SYM ? frame_action(a, fr) : a)] = ((w >> (a & 31)) & 1u) ? p : 0.0f;
             }
         }
         if (!leaf_over) {
@@ -589,6 +628,14 @@ __global__ void __launch_bounds__(RTPB, 7) k_tree_rollout_eval(hz_tree T, int lo
         for (int o = 16; o > 0; o >>= 1) steps += __shfl_xor_sync(FULL, steps, o);
         if ((threadIdx.x & 31) == 0 && steps) atomicAdd(total_steps, (unsigned long long)steps);
     }
+}
+
+// ---- frames of the last select (hz_tree_leaf_frames) ------------------------------------------------
+__global__ void __launch_bounds__(TTPB) k_tree_leaf_frames(hz_tree T, int on, uint16_t* frames) {
+    const int64_t row = (int64_t)blockIdx.x * TTPB + threadIdx.x;
+    if (row >= (int64_t)T.n_trees * T.leaves) return;
+    const int64_t t = row / T.leaves;
+    frames[row] = on ? (uint16_t)((T.node_info[t * T.max_nodes + T.leaf[row]] >> 16) & 0x1FFu) : (uint16_t)0;
 }
 
 // ---- root statistics (MCTS.py:355-381) and move choice (MCTS.py:394-441) -------------------------
@@ -732,6 +779,8 @@ int hz_tree_create(hz_tree** out, void* workspace, size_t workspace_bytes, int n
     t->table_hash = (uint64_t*)(b + L.off[19]); t->edge_cinfo = (uint32_t*)(b + L.off[20]);
     t->table_bytes = (size_t)n_trees * L.table_size * 4;
     t->n_active = nullptr;
+    t->sym_mode = HZ_SYM_OFF;
+    t->frames_on = 0;
     *out = t;
     return HZ_OK;
 }
@@ -745,6 +794,18 @@ int hz_tree_set_active(hz_tree* t, const int32_t* n_active) {
     if (!t || ((uintptr_t)n_active & 3)) return HZ_ERR_ARG;
     t->n_active = n_active;
     return HZ_OK;
+}
+
+int hz_tree_set_symmetry(hz_tree* t, int mode) {
+    if (!t || (mode != HZ_SYM_OFF && mode != HZ_SYM_BOARD && mode != HZ_SYM_FULL)) return HZ_ERR_ARG;
+    t->sym_mode = mode;
+    return HZ_OK;
+}
+
+int hz_tree_leaf_frames(hz_tree* t, uint16_t* frames, void* stream) {
+    if (!t || !frames) return HZ_ERR_ARG;
+    k_tree_leaf_frames<<<tree_blocks(t->n_trees * t->leaves, TTPB), TTPB, 0, (cudaStream_t)stream>>>(*t, t->frames_on, frames);
+    return hz_launched(1);
 }
 
 int hz_tree_reset(hz_tree* t, const void* root_states, const uint64_t* search_keys, void* stream) {
@@ -763,7 +824,10 @@ int hz_tree_select(hz_tree* t, float cpuct, void* leaf_states, void* board, void
     uint4* ls = (uint4*)leaf_states;
     if (layout != HZ_LAYOUT_NCHW && layout != HZ_LAYOUT_NHWC && layout != HZ_LAYOUT_NHWC40 && layout != HZ_LAYOUT_T16K) return HZ_ERR_ARG;
     if (layout == HZ_LAYOUT_T16K && dtype != HZ_DTYPE_BF16) return HZ_ERR_ARG;
-#define HZ_SELECT(T, L) k_tree_select<T, L><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob)
+#define HZ_SELECT(T, L)                                                                                    \
+    (t->sym_mode == HZ_SYM_FULL    ? k_tree_select<T, L, 480><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob) \
+     : t->sym_mode == HZ_SYM_BOARD ? k_tree_select<T, L, 4><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob)   \
+                                   : k_tree_select<T, L, 0><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob))
     if (dtype == HZ_DTYPE_F32) {
         if (layout == HZ_LAYOUT_NHWC40) HZ_SELECT(float, HZ_LAYOUT_NHWC40);
         else if (layout == HZ_LAYOUT_NHWC) HZ_SELECT(float, HZ_LAYOUT_NHWC);
@@ -777,19 +841,26 @@ int hz_tree_select(hz_tree* t, float cpuct, void* leaf_states, void* board, void
         return HZ_ERR_ARG;
     }
 #undef HZ_SELECT
+    t->frames_on = t->sym_mode != HZ_SYM_OFF;
     return hz_launched(1);
 }
 
 int hz_tree_expand_backup(hz_tree* t, const float* policy, const float* value, int is_logits, const float* noise,
                           double eps, void* stream) {
     if (!t || !policy || !value) return HZ_ERR_ARG;
-    k_tree_expand_backup<<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value, is_logits, noise, eps);
+    if (t->sym_mode != HZ_SYM_OFF)
+        k_tree_expand_backup<true><<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value, is_logits, noise, eps);
+    else
+        k_tree_expand_backup<false><<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value, is_logits, noise, eps);
     return hz_launched(1);
 }
 
 int hz_tree_fake_eval(hz_tree* t, float* policy, float* value, void* stream) {
     if (!t || !policy || !value) return HZ_ERR_ARG;
-    k_tree_fake_eval<<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value);
+    if (t->sym_mode != HZ_SYM_OFF)
+        k_tree_fake_eval<true><<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value);
+    else
+        k_tree_fake_eval<false><<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value);
     return hz_launched(1);
 }
 
@@ -799,8 +870,11 @@ int hz_tree_rollout_eval(hz_tree* t, int rollouts, float* policy, float* value, 
     int log2r = 0;
     while ((1 << log2r) < rollouts) log2r++;
     int64_t threads = (int64_t)t->n_trees * t->leaves * rollouts;
-    k_tree_rollout_eval<<<(unsigned)((threads + RTPB - 1) / RTPB), RTPB, 0, (cudaStream_t)stream>>>(*t, log2r, policy, value,
-                                                                                                   total_steps);
+    const unsigned grid = (unsigned)((threads + RTPB - 1) / RTPB);
+    if (t->sym_mode != HZ_SYM_OFF)
+        k_tree_rollout_eval<true><<<grid, RTPB, 0, (cudaStream_t)stream>>>(*t, log2r, policy, value, total_steps);
+    else
+        k_tree_rollout_eval<false><<<grid, RTPB, 0, (cudaStream_t)stream>>>(*t, log2r, policy, value, total_steps);
     return hz_launched(1);
 }
 

@@ -47,30 +47,46 @@ class ReplayRing:
             return torch.arange(self.size, device=self.device)
         return (self.head + torch.arange(self.capacity, device=self.device)) % self.capacity
 
-    def sample(self, batch_size, generator=None, dtype=torch.float32):
+    def sample(self, batch_size, generator=None, dtype=torch.float32, augment=None):
         """A training batch (board [B,38,5,7], global [B,42], pi [B,143], z [B,1]) on the
-        device: uniform sampling with replacement + hz_encode of the packed states."""
+        device: uniform sampling with replacement + hz_encode of the packed states.
+        augment: None, "board" or "full": every row is mapped by its own uniform group element g
+        (drawn from ``generator`` after the indices): encode(T_g(state)), T_g(visits) normalised, z."""
         if self.size == 0:
             raise ValueError("replay ring is empty")
         idx = torch.randint(0, self.size, (batch_size,), device=self.device, generator=generator)
         if self.size == self.capacity:
             idx = (self.head + idx) % self.capacity
-        return self._batch(idx, dtype)
+        return self._batch(idx, dtype, self._elements(idx.numel(), augment, generator))
 
-    def _batch(self, idx, dtype=torch.float32):
-        board, glob = hb.encode(self.states[idx].contiguous(), dtype=dtype)
-        v = self.visits[idx].to(torch.float64)
+    def _elements(self, n, augment, generator):
+        if augment is None:                      # no draw: the generator advances exactly as without augmentation
+            return None
+        from .symmetry import random_elements
+
+        return random_elements(n, augment, device=self.device, generator=generator)
+
+    def _batch(self, idx, dtype=torch.float32, sym=None):
+        states, visits = self.states[idx].contiguous(), self.visits[idx]
+        if sym is not None:
+            from .symmetry import transform_actions, transform_states
+
+            visits = transform_actions(visits.contiguous(), sym, states)
+            transform_states(states, sym, out=states)
+        board, glob = hb.encode(states, dtype=dtype)
+        v = visits.to(torch.float64)
         pi = (v / v.sum(dim=1, keepdim=True).clamp_min(1)).to(torch.float32)      # trainer.py:535
         return board, glob, pi, self.z[idx].view(-1, 1)
 
-    def epoch(self, batch_size, shuffle=True, generator=None):
+    def epoch(self, batch_size, shuffle=True, generator=None, augment=None):
         """Iterate once over the whole buffer in batches (DataLoader(ReplayBufferDataset(...),
-        shuffle=True), trainer.py:146-153)."""
+        shuffle=True), trainer.py:146-153).  augment: as for ``sample`` (one element per row and batch)."""
         order = self._ordered_index()
         if shuffle:
             order = order[torch.randperm(order.numel(), device=self.device, generator=generator)]
         for i in range(0, order.numel(), batch_size):
-            yield self._batch(order[i:i + batch_size])
+            part = order[i:i + batch_size]
+            yield self._batch(part, sym=self._elements(part.numel(), augment, generator))
 
     def to_reference_buffer(self):
         """deque(maxlen=capacity) of (board, global, pi, z) CPU tensors, oldest first — the

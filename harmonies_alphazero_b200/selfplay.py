@@ -43,6 +43,7 @@ class SelfPlayConfig:
     max_nodes: int = 0             # per-tree node arena; 0 = worst case 1 + 69*sims
     max_moves: int = 200           # hard cap per game (structural maximum is 160 actions)
     compact_live: bool = True      # play(): keep the live games in a dense slot prefix and search only those (the game tail costs what it uses)
+    eval_symmetry: str = None      # None, "board" or "full": the network sees each leaf in a random symmetry frame (hz_tree_set_symmetry)
 
     @classmethod
     def from_mcts_config(cls, mcts_config, **kw):
@@ -97,6 +98,18 @@ class Trajectories:
         fn = torch.from_numpy
         return [tuple(fn(f[i].copy()) for f in fields) for i in range(n - lo)]
 
+    def transform(self, sym):
+        """A copy with every example mapped by a group element (symmetry.py): states T_g(state), visits
+        x'[sigma_g(a)] = x[a], z and the ids unchanged.  sym: int or int[M] (0..479)."""
+        from .symmetry import transform_actions, transform_states
+
+        if len(self) == 0:
+            return Trajectories(self.states.clone(), self.visits.clone(), self.z.clone(), self.game_id.clone(),
+                                self.move_no.clone(), dict(self.stats))
+        states = self.states.contiguous()
+        return Trajectories(transform_states(states, sym), transform_actions(self.visits.contiguous(), sym, states),
+                            self.z.clone(), self.game_id.clone(), self.move_no.clone(), dict(self.stats))
+
     def to(self, device):
         return Trajectories(self.states.to(device), self.visits.to(device), self.z.to(device),
                             self.game_id.to(device), self.move_no.to(device), dict(self.stats))
@@ -150,6 +163,7 @@ class _Group:
         if cfg.num_simulations % K:
             raise ValueError("num_simulations must be a multiple of leaves_per_step")
         self.tree = BatchedMCTS(n, cfg.num_simulations, device=dev, key_mode=cfg.key_mode, max_nodes=cfg.max_nodes, leaves=K)
+        self.tree.set_symmetry(cfg.eval_symmetry)     # before any capture: a graph keeps the mode it was captured with
         rows = n * K                  # the network sees K leaves per tree and step
         dt, cl = net.dtype, owner.channels_last
         self.tiles = bool(getattr(net, "wants_tiles", False))   # leaves go straight into the hand-written tower's input image

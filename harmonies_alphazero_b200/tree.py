@@ -53,6 +53,21 @@ class BatchedMCTS:
         self._n_active = n_active
         _lib.check(self.lib.hz_tree_set_active(self.handle, _ptr(n_active)), "hz_tree_set_active")
 
+    def set_symmetry(self, mode):
+        """Random-frame leaf evaluation (hz_tree_set_symmetry): None / "board" / "full".  With a mode on, the evaluator sees
+        every leaf in a frame T_g drawn from the leaf and the search key, and its policy row is read back through sigma_g;
+        the tree does not change.  Acts on the calls that follow; a captured CUDA graph keeps the mode of its capture."""
+        from .symmetry import mode_code
+
+        _lib.check(self.lib.hz_tree_set_symmetry(self.handle, mode_code(mode)), "hz_tree_set_symmetry")
+
+    def leaf_frames(self):
+        """int64[rows]: the frame g of every leaf row of the last ``select`` (0 when it ran with the mode off)."""
+        out = torch.empty(self.rows, dtype=torch.int16, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.hz_tree_leaf_frames(self.handle, _ptr(out), self._stream()), "hz_tree_leaf_frames")
+        return out.to(torch.int64)
+
     def reset(self, root_states, search_keys=None):
         """New search per tree (no tree reuse, MCTS.py:288-289).  search_keys int64[n] or None
         (derived per (game, move) from the root's own rng key and move counter)."""

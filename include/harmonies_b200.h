@@ -135,9 +135,11 @@ extern "C" {
 #define HZ_MOVE_BAD_PHASE     6  /* :296 */
 #define HZ_MOVE_BAD_DRAW      7  /* explicit replay draw not available in the bag */
 
-/* encode dtypes / layouts */
+/* encode dtypes / layouts (HZ_DTYPE_I16 / HZ_DTYPE_I32: hz_sym_actions only) */
 #define HZ_DTYPE_F32  0
 #define HZ_DTYPE_BF16 1
+#define HZ_DTYPE_I16  2
+#define HZ_DTYPE_I32  3
 #define HZ_LAYOUT_NCHW 0
 #define HZ_LAYOUT_NHWC 1
 #define HZ_LAYOUT_NHWC40 2  /* hz_tree_select only: [n,5,7,40], channels 38,39 = 0 (8-aligned C for the stem conv) */
@@ -240,6 +242,38 @@ int hz_playout_keys(const uint64_t *keys, int64_t n, uint64_t seed, uint64_t fir
                     int max_steps, uint32_t *results, unsigned long long *total_steps,
                     void *stream);
 
+/* ---- game symmetries --------------------------------------------------------------------
+ * The 23-hex board has exactly four automorphisms of its neighbour graph, all maps of the hex
+ * lattice (axial coordinates): b = 0 identity, b = 1 (q,r) -> (q+r,-r), b = 2 (q,r) -> (-q-r,r),
+ * b = 3 (q,r) -> (-q,-r) (hex i -> 22-i).  They form a Klein four-group (b1 o b2 = b1 ^ b2).  The
+ * order of the piles carries no information either (pop(i) shifts the later piles, new ones are
+ * appended).  Every rule (legality, the five scoring terms, the end-of-game trigger) reads only
+ * stacks and adjacency, so a position and its image have the same value and the same legal moves
+ * up to the action permutation below.
+ *  element g (0..479, uint16): board part b = g & 3, pile part c = g >> 2 (0..119).
+ *  T_g(state): the content of hex i moves to hex tau_b(i) in all 18 plane words; with m = n_piles,
+ *           pi = itertools.permutations(range(m))[c mod m!], the pile at position i < m moves to
+ *           position pi[i] (positions >= m stay put).  Hand, bag, meta, scores, rng key and the
+ *           counters are unchanged.  m! divides 120, so a uniform g gives a uniform permutation.
+ *  sigma_g(a): pi[a] for a < m; a for m <= a < 5; 5 + 23t + tau_b(h) for a = 5 + 23t + h.
+ *           A policy, visit or mask row x transforms as x'[sigma_g(a)] = x[a].
+ * The tables (tau_b, its inverse, the permutations) are generated from constants.py's geometry by
+ * gen_tables.py into csrc/hz_tables.inc; harmonies_alphazero_b200/symmetry.py mirrors them. */
+#define HZ_SYM_OFF   0   /* no symmetry (the default of a tree: reference-exact) */
+#define HZ_SYM_BOARD 1   /* the 4 board symmetries (pile part 0) */
+#define HZ_SYM_FULL  2   /* board x pile order: 480 elements */
+#define HZ_SYMMETRY_SALT 0x53594D4D45545259ull   /* leaf frames of the search, see hz_tree_set_symmetry */
+
+/* out[i] = T_{sym[i]}(states[i]).  out == states works (in place); other overlap does not.
+ * Words 28..31 are copied unchanged. */
+int hz_sym_states(const void *states, int64_t n, const uint16_t *sym, void *out, void *stream);
+
+/* Rows x [n,143] of dtype HZ_DTYPE_F32, HZ_DTYPE_I16 or HZ_DTYPE_I32: out[i][sigma(a)] = x[i][a] with
+ * sigma = sigma_{sym[i]} (inverse == 0) or sigma_{sym[i]}^-1 (inverse != 0).  n_piles is read from
+ * states[i] (it is the same in either frame).  out must not overlap x. */
+int hz_sym_actions(const void *x, int64_t n, int dtype, const uint16_t *sym, const void *states,
+                   int inverse, void *out, void *stream);
+
 /* ---- search tree (MCTS.py) ---------------------------------------------------------- */
 
 typedef struct hz_tree hz_tree;   /* opaque: n_trees independent DAGs in flat arrays */
@@ -276,6 +310,29 @@ int hz_tree_reset(hz_tree *t, const void *root_states, const uint64_t *search_ke
  * of a step then costs only the live rows.  The reference has no counterpart (one process per
  * game, trainer.py:104-107). */
 int hz_tree_set_active(hz_tree *t, const int32_t *n_active);
+
+/* Random-frame leaf evaluation (AlphaGo Zero's random rotation of the network's view): mode
+ * HZ_SYM_OFF (the default, reference-exact), HZ_SYM_BOARD (G = 4) or HZ_SYM_FULL (G = 480).  With a
+ * mode on, leaf row r of every following step gets one frame
+ *   z = rand(sk ^ HZ_SYMMETRY_SALT, canon_hash(leaf, HZ_KEY_EXACT)),  g_r = ((z >> 32) * G) >> 32
+ * (leaf = the node's stored words, sk = the tree's search key): it depends on the leaf and the search
+ * key only, so two virtual-loss rows that reach one leaf share it.  The tree itself never changes frame:
+ *  - hz_tree_select writes (board, glob) of T_{g_r}(leaf) in every layout; leaf_states stay untransformed;
+ *  - hz_tree_expand_backup takes policy[r][sigma_{g_r}(a)] as the prior of action a (the fused softmax,
+ *    its sums and the root Dirichlet mix run in the tree's order, as with the mode off);
+ *  - hz_tree_fake_eval and hz_tree_rollout_eval write their result into the frame (entry sigma_{g_r}(a)
+ *    gets what entry a gets with the mode off; values unchanged), so a search with them is the same
+ *    with the mode on or off.
+ * A leaf's frame is kept in the tree's node record for the rest of the search.  The mode acts on the
+ * launches that follow the call; a captured CUDA graph keeps the mode it was captured with.  Set the
+ * mode before hz_tree_reset: one search runs in one mode (switching it on after steps with the mode off
+ * is fine; switching between HZ_SYM_BOARD and HZ_SYM_FULL inside a search is not). */
+int hz_tree_set_symmetry(hz_tree *t, int mode);
+
+/* frames[n_trees * leaves] (uint16): g_r of every leaf row of the last hz_tree_select (0 for all rows
+ * when that select ran with the mode off).  Rows of trees beyond the active prefix keep the frames of
+ * the last select that included them. */
+int hz_tree_leaf_frames(hz_tree *t, uint16_t *frames, void *stream);
 
 /* move_to_leaf (MCTS.py:63-149) for every tree, then create_state_tensors of the leaf
  * (MCTS.py:299) into board/glob (see hz_encode).  cpuct is applied as fp32(cpuct)*P in fp32
