@@ -48,6 +48,13 @@ SIGNATURES = {
     "hz_tree_choose": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "hz_tree_stats": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "hz_tree_root_edges": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "hz_evalcache_bytes": (C.c_size_t, [_i64, _i]),
+    "hz_evalcache_create": (_i, [C.POINTER(_vp), _vp, C.c_size_t, _i64, _i]),
+    "hz_evalcache_destroy": (_i, [_vp]),
+    "hz_evalcache_clear": (_i, [_vp, _vp]),
+    "hz_evalcache_stats": (_i, [_vp, _vp, _vp]),
+    "hz_tree_select_cached": (_i, [_vp, _vp, _f, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "hz_evalcache_fill": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hz_net_heads": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp]),
     "hz_net_heads_fc_active": (_i, [_vp, _vp, _i64, _vp, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp]),
     "hz_tower_tile_bytes": (C.c_size_t, [_i64, _i]),

@@ -12,11 +12,11 @@ excludes draws (trainer.py:338-342).
 import torch
 
 from . import batched as hb
-from .selfplay import RolloutEvaluator
-from .tree import BatchedMCTS
+from .selfplay import RolloutEvaluator, check_cacheable
+from .tree import BatchedMCTS, EvalCache
 
 
-def _search(tree, net, states, sims, cpuct, bufs):
+def _search(tree, net, states, sims, cpuct, bufs, cache=None, cbufs=None):
     board, glob, logits, value = bufs
     tree.reset(states)
     if isinstance(net, RolloutEvaluator):
@@ -28,6 +28,17 @@ def _search(tree, net, states, sims, cpuct, bufs):
     tiles = board.dtype == torch.uint8
     pad40 = not tiles and board.shape[1] == 40
     for _ in range(sims // tree.leaves):
+        if cache is not None:        # only the missed leaves go through the network (tree.EvalCache)
+            net_logits, net_value, eval_rows, n_eval = cbufs
+            tree.select_cached(cache, cpuct, board, glob, logits, value, eval_rows, n_eval, dtype=net.dtype, channels_last=True,
+                               pad40=pad40, tiles=tiles)
+            if tiles:
+                net.forward_tiles(board, glob, glob.shape[0], out=(net_logits, net_value), n_active=n_eval)
+            else:
+                net(board, glob, out=(net_logits, net_value))
+            cache.fill(net_logits, net_value, eval_rows, n_eval, logits, value)
+            tree.expand_backup(logits, value, is_logits=True)
+            continue
         tree.select(cpuct, board, glob, dtype=net.dtype, channels_last=True, pad40=pad40, tiles=tiles)
         if tiles:
             net.forward_tiles(board, glob, glob.shape[0], out=(logits, value))
@@ -40,7 +51,7 @@ GREEDY = "greedy"   # pass as either side to play the 1-ply greedy agent of eval
 
 
 def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cuda", seed=0, key_mode=hb.KEY_REFERENCE, leaves=1,
-               symmetry=None):
+               symmetry=None, eval_cache=0):
     """Returns dict(candidate_wins, best_wins, draws, win_rate, games).  Each side is an
     InferenceNet on ``device``, ``arena.GREEDY`` (run_tournament of evaluation.py:7-65:
     AlphaZero vs the greedy agent, sides alternating by game index) or a
@@ -48,8 +59,15 @@ def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cud
     searches to the virtual-loss mode (K simulations in flight per tree): not the reference's
     visit counts any more, but a 30-game match then fills the network batch K times better.
     symmetry: None, "board" or "full": both sides' networks see every leaf in a random symmetry frame
-    (BatchedMCTS.set_symmetry)."""
+    (BatchedMCTS.set_symmetry).
+    eval_cache: entries of a leaf evaluation cache per side (tree.EvalCache), 0 = off.  One player makes all four actions
+    of a turn, so a side's searches reuse its own earlier evaluations; the results are unchanged.  Network sides must be
+    row-invariant; a rollout side raises ValueError."""
     dev = torch.device(device)
+    if eval_cache:
+        for side in (candidate_net, best_net):
+            if side is not GREEDY:
+                check_cacheable(side)
     sims, cpuct = int(mcts_config_eval["num_simulations"]), float(mcts_config_eval["cpuct"])
     # group 0: candidate is player 0 (even game indices); group 1: candidate is player 1
     sizes = [(num_games + 1) // 2, num_games // 2]
@@ -82,6 +100,11 @@ def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cud
                     torch.zeros((rows, 143), dtype=torch.float32, device=dev),
                     torch.zeros(rows, dtype=torch.float32, device=dev),
                 )
+        caches = cbufs = None
+        if eval_cache and nets:
+            caches = [None if side is GREEDY else EvalCache(eval_cache, rows, device=dev) for side in (candidate_net, best_net)]
+            cbufs = (torch.zeros((rows, 143), dtype=torch.float32, device=dev), torch.zeros(rows, dtype=torch.float32, device=dev),
+                     torch.zeros(rows, dtype=torch.int32, device=dev), torch.zeros(1, dtype=torch.int32, device=dev))
         for _ in range(200):
             over, oc = hb.outcome(states)
             if bool(over.all()):
@@ -93,11 +116,12 @@ def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cud
             mover = int(movers[0].item())
             if not bool((movers == mover).all()):
                 raise RuntimeError("arena games of one group are out of lockstep (different players to move)")
-            net = candidate_net if mover == g else best_net
+            side = 0 if mover == g else 1
+            net = (candidate_net, best_net)[side]
             if net is GREEDY:                                        # evaluation.py:137-196, one kernel
                 actions = hb.greedy_actions(states)
             else:
-                _search(tree, net, states, sims, cpuct, bufs)
+                _search(tree, net, states, sims, cpuct, bufs, None if caches is None else caches[side], cbufs)
                 actions = tree.choose()                              # first max N: testing=True
             actions = torch.where(live, actions, torch.full_like(actions, -1))
             hb.apply(states, actions)

@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libharmonies_b200.so")
-SOURCES = ["hz_abi.cu", "hz_engine.cu", "hz_mcts.cu", "hz_symmetry.cu", "hz_heads.cu", "hz_tower.cu"]
+SOURCES = ["hz_abi.cu", "hz_engine.cu", "hz_mcts.cu", "hz_evalcache.cu", "hz_symmetry.cu", "hz_heads.cu", "hz_tower.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

@@ -933,6 +933,13 @@ __device__ __forceinline__ uint64_t canon_hash(const State& s, int mode) {
     key_words(s, mode, k);
     return hash_key_words(k);
 }
+// canon_hash(leaf, HZ_KEY_EXACT) of 32 staged words (any memory space the caller can read uniformly)
+__device__ __forceinline__ uint64_t exact_key_of_words(const uint32_t* w) {
+    uint64_t h = 0x9E3779B97F4A7C15ull;
+#pragma unroll
+    for (int i = 0; i < HZ_CANON_WORDS; i++) h = hash_step(h, i == HZ_W_BAG1META ? (w[i] & 0x0FFFFFFFu) : w[i]);
+    return mix64(h);
+}
 
 // ---- state tensors (process_game_state.py:15-137): per-channel hex masks + global features ----
 __constant__ uint8_t CELL_HEX[35] = {31, 31, 4, 9, 14, 19, 22, 31, 31, 5, 10, 15, 20, 31, 31, 1, 6, 11,

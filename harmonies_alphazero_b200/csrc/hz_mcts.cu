@@ -18,6 +18,7 @@
 
 #include "hz_common.cuh"
 #include "hz_core.cuh"
+#include "hz_evalcache.cuh"
 #include "hz_sym.cuh"
 
 struct hz_tree {
@@ -150,10 +151,52 @@ __device__ __forceinline__ void warp_encode_fast40(const uint32_t* w, uint8_t* s
     __syncwarp();
 }
 
+// ---- evaluation cache, select side (hz_tree_select_cached) ---------------------------------------------------------
+// Leaf row `row` with staged words w, exact key `key` and frame fr.  Returns whether the leaf needs the network:
+//  - terminal: no row anywhere (k_tree_expand_backup uses the outcome);
+//  - hit: the stored row goes to EC.policy[row], EC.value[row] and the entry's stamp is refreshed;
+//  - miss: network row m = atomicAdd(n_eval) (erow = m), eval_rows[m] = row, and (key, frame) wait there for the fill.
+__device__ __forceinline__ bool cache_row(const EvalCacheArgs& EC, const uint32_t* w, uint64_t key, uint32_t fr, size_t row,
+                                          size_t& erow, unsigned long long& n_hit, unsigned long long& n_terminal, int lane) {
+    const hz_evalcache& c = EC.c;
+    HZ_BOUND(row, c.max_rows, 602);
+    if (words_over(w)) {
+        n_terminal++;
+        return false;
+    }
+    const int64_t e = ec_probe(c, key, fr, w, lane);
+    if (e >= 0) {
+        const float* src = c.row + e * EC_ROW;
+        for (int a = lane; a < HZ_ACTION_SIZE; a += 32) EC.policy[row * HZ_ACTION_SIZE + a] = src[a];
+        if (lane == 0) {
+            EC.value[row] = src[HZ_ACTION_SIZE];
+            c.stamp[e] = c.clock[0] + 1u;
+        }
+        n_hit++;
+        return false;
+    }
+    int m = 0;
+    if (lane == 0) m = atomicAdd(EC.n_eval, 1);                  // one row per miss: the warp is one tree
+    m = __shfl_sync(FULL, m, 0);
+    HZ_BOUND(m, c.max_rows, 603);
+    if (lane == 0) {
+        EC.eval_rows[m] = (int32_t)row;
+        c.pend_key[m] = key;
+        c.pend_frame[m] = fr;
+    }
+    if (HZ_TREE_FULL_COMPARE && lane < HZ_CANON_WORDS)
+        c.pend_words[(size_t)m * HZ_CANON_WORDS + lane] = lane == HZ_W_BAG1META ? (w[lane] & 0x0FFFFFFFu) : w[lane];
+    erow = (size_t)m;
+    return true;
+}
+
 // ---- select: move_to_leaf (MCTS.py:63-149) + create_state_tensors(leaf) (MCTS.py:299) ---------
 // G = order of the symmetry group of the leaf frames (0: off, the reference's select)
-template <typename OT, int LAYOUT, int G>
-__global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, uint4* leaf_states, OT* board, OT* glob) {
+// CACHE: look every leaf up in the evaluation cache EC (hz_tree_select_cached); only misses are encoded, into the dense
+// network rows handed out by EC.n_eval.  EC is the last parameter, so the cache-off kernels' parameters keep their offsets.
+template <typename OT, int LAYOUT, int G, bool CACHE>
+__global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, uint4* leaf_states, OT* board, OT* glob,
+                                                      EvalCacheArgs EC) {
     __shared__ uint32_t sm_words[WPB][32];
     __shared__ uint32_t sm_mask[WPB][40];
     constexpr bool FAST40 = (LAYOUT == HZ_LAYOUT_NHWC40 || LAYOUT == HZ_LAYOUT_T16K) && sizeof(OT) == 2;
@@ -171,6 +214,7 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
     if (t >= active_trees(T)) return;
     TreeView v = view_of(T, t);
     const int K = T.leaves;
+    [[maybe_unused]] unsigned long long n_hit = 0, n_terminal = 0;
     // K descents per tree and step.  K == 1 is the reference's move_to_leaf.  For K > 1 every
     // edge of an already chosen path carries an in-flight visit V: N' = N + V, W' = W - V
     // (a provisional loss for the mover), so the later descents of the step spread out.
@@ -256,29 +300,43 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
         size_t row = (size_t)t * K + j;
         warp_load_words(sm_words[warp], v.node_state, node, lane);      // (__syncwarp inside: V updates are visible to the next descent)
         if (leaf_states) reinterpret_cast<uint32_t*>(leaf_states + row * 8)[lane] = sm_words[warp][lane];
+        size_t erow = row;                                               // the row the leaf is encoded into
+        [[maybe_unused]] bool encode = true;                             // CACHE: the leaf needs the network
+        [[maybe_unused]] uint64_t ekey = 0;
+        if constexpr (CACHE) ekey = exact_key_of_words(sm_words[warp]);
         if constexpr (G != 0) {                                          // the network sees T_g(leaf); the tree keeps its frame
             const uint32_t* w = sm_words[warp];
-            const int g = sym_frame(w, T.search_key[t], G);
+            const int g = CACHE ? sym_frame_of_key(ekey, T.search_key[t], G) : sym_frame(w, T.search_key[t], G);
             const uint32_t w22 = w[HZ_W_BAG1META], own = w[lane];
             const uint32_t m = (w22 >> 16) & 0xFFu;
             // the frame is a function of the node within a search: kept in the node's info word, bits 16..27 =
             // g | n_piles << 9 (OR of the same value when the node is reached again; a new search creates new nodes)
             if (lane == 0) atomicOr(&v.node_info[node], ((uint32_t)g | ((m < 5u ? m : 5u) << 9)) << 16);
-            if (board) {
+            if constexpr (CACHE) encode = cache_row(EC, w, ekey, (uint32_t)g, row, erow, n_hit, n_terminal, lane);
+            if (board && encode) {
                 const uint32_t nw = warp_sym_word(own, g, lane);
                 __syncwarp();
                 sm_words[warp][lane] = nw;
                 __syncwarp();
             }
+        } else if constexpr (CACHE) {
+            encode = cache_row(EC, sm_words[warp], ekey, 0u, row, erow, n_hit, n_terminal, lane);
         }
-        if (board) {
+        if (board && encode) {
             if constexpr (FAST40)
-                warp_encode_fast40<LAYOUT == HZ_LAYOUT_T16K>(sm_words[warp], sbytes[warp], vlut8, scell, (__nv_bfloat16*)board, row,
-                                                             (__nv_bfloat16*)glob + row * 42, lane);
+                warp_encode_fast40<LAYOUT == HZ_LAYOUT_T16K>(sm_words[warp], sbytes[warp], vlut8, scell, (__nv_bfloat16*)board, erow,
+                                                             (__nv_bfloat16*)glob + erow * 42, lane);
             else
-                warp_encode<OT, LAYOUT>(sm_words[warp], sm_mask[warp], board + row * RowElems<LAYOUT>::value, glob + row * 42, lane);
+                warp_encode<OT, LAYOUT>(sm_words[warp], sm_mask[warp], board + erow * RowElems<LAYOUT>::value, glob + erow * 42, lane);
         }
         __syncwarp();
+    }
+    if constexpr (CACHE) {
+        if (lane == 0) {
+            atomicAdd(&EC.c.counters[0], (unsigned long long)K);
+            if (n_hit) atomicAdd(&EC.c.counters[1], n_hit);
+            if (n_terminal) atomicAdd(&EC.c.counters[2], n_terminal);
+        }
     }
 }
 
@@ -287,9 +345,6 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
 // (MCTS.py:185 looks `hash(state)` up in a dict of ids and never compares states); building
 // with -DHZ_TREE_FULL_COMPARE=1 additionally compares the 23 key words on a hash match, which
 // costs a dependent 128-byte gather per hit and only guards against a 2^-64 collision.
-#ifndef HZ_TREE_FULL_COMPARE
-#define HZ_TREE_FULL_COMPARE 0
-#endif
 __device__ __forceinline__ int table_find(const hz_tree& T, const TreeView& v, uint64_t h, const uint32_t* key) {
     uint32_t mask = (uint32_t)T.table_size - 1u;
     uint32_t slot = (uint32_t)h & mask;
@@ -817,17 +872,19 @@ int hz_tree_reset(hz_tree* t, const void* root_states, const uint64_t* search_ke
     return hz_launched(1);
 }
 
-int hz_tree_select(hz_tree* t, float cpuct, void* leaf_states, void* board, void* glob, int dtype, int layout, void* stream) {
-    if (!t || (board && !glob)) return HZ_ERR_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
+}  // extern "C"
+
+template <bool CACHE>
+static int launch_select(hz_tree* t, float cpuct, void* leaf_states, void* board, void* glob, int dtype, int layout,
+                         const EvalCacheArgs& ec, cudaStream_t st) {
     int grid = tree_blocks(t->n_trees, WPB);
     uint4* ls = (uint4*)leaf_states;
     if (layout != HZ_LAYOUT_NCHW && layout != HZ_LAYOUT_NHWC && layout != HZ_LAYOUT_NHWC40 && layout != HZ_LAYOUT_T16K) return HZ_ERR_ARG;
     if (layout == HZ_LAYOUT_T16K && dtype != HZ_DTYPE_BF16) return HZ_ERR_ARG;
-#define HZ_SELECT(T, L)                                                                                    \
-    (t->sym_mode == HZ_SYM_FULL    ? k_tree_select<T, L, 480><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob) \
-     : t->sym_mode == HZ_SYM_BOARD ? k_tree_select<T, L, 4><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob)   \
-                                   : k_tree_select<T, L, 0><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob))
+#define HZ_SELECT(T, L)                                                                                                         \
+    (t->sym_mode == HZ_SYM_FULL    ? k_tree_select<T, L, 480, CACHE><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec) \
+     : t->sym_mode == HZ_SYM_BOARD ? k_tree_select<T, L, 4, CACHE><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec)   \
+                                   : k_tree_select<T, L, 0, CACHE><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec))
     if (dtype == HZ_DTYPE_F32) {
         if (layout == HZ_LAYOUT_NHWC40) HZ_SELECT(float, HZ_LAYOUT_NHWC40);
         else if (layout == HZ_LAYOUT_NHWC) HZ_SELECT(float, HZ_LAYOUT_NHWC);
@@ -843,6 +900,23 @@ int hz_tree_select(hz_tree* t, float cpuct, void* leaf_states, void* board, void
 #undef HZ_SELECT
     t->frames_on = t->sym_mode != HZ_SYM_OFF;
     return hz_launched(1);
+}
+
+extern "C" {
+
+int hz_tree_select(hz_tree* t, float cpuct, void* leaf_states, void* board, void* glob, int dtype, int layout, void* stream) {
+    if (!t || (board && !glob)) return HZ_ERR_ARG;
+    return launch_select<false>(t, cpuct, leaf_states, board, glob, dtype, layout, EvalCacheArgs{}, (cudaStream_t)stream);
+}
+
+int hz_tree_select_cached(hz_tree* t, hz_evalcache* c, float cpuct, void* leaf_states, void* board, void* glob, int dtype,
+                          int layout, float* policy, float* value, int32_t* eval_rows, int32_t* n_eval, void* stream) {
+    if (!t || !c || !board || !glob || !policy || !value || !eval_rows || !n_eval || ((uintptr_t)n_eval & 3)) return HZ_ERR_ARG;
+    if ((int64_t)t->n_trees * t->leaves > c->max_rows) return HZ_ERR_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = cudaMemsetAsync(n_eval, 0, sizeof(int32_t), st);     // misses of this step count from 0
+    if (e != cudaSuccess) return hz_record_launch(0, e);
+    return launch_select<true>(t, cpuct, leaf_states, board, glob, dtype, layout, EvalCacheArgs{*c, policy, value, eval_rows, n_eval}, st);
 }
 
 int hz_tree_expand_backup(hz_tree* t, const float* policy, const float* value, int is_logits, const float* noise,

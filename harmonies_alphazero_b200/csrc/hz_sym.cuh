@@ -23,13 +23,13 @@ __device__ __forceinline__ int sym_action(int a, int b, int m, uint32_t pp, cons
 }
 
 // Frame of a leaf row: rand(sk ^ HZ_SYMMETRY_SALT, canon_hash(words, HZ_KEY_EXACT)) scaled to 0..G-1.
+__device__ __forceinline__ int sym_frame_of_key(uint64_t exact_key, uint64_t sk, int G) {
+    const uint64_t z = rand64(sk ^ HZ_SYMMETRY_SALT, exact_key);
+    return (int)(((z >> 32) * (uint64_t)G) >> 32);
+}
 // w: the 32 words (any memory space the caller can read uniformly).
 __device__ __forceinline__ int sym_frame(const uint32_t* w, uint64_t sk, int G) {
-    uint64_t h = 0x9E3779B97F4A7C15ull;
-#pragma unroll
-    for (int i = 0; i < HZ_CANON_WORDS; i++) h = hash_step(h, i == HZ_W_BAG1META ? (w[i] & 0x0FFFFFFFu) : w[i]);
-    const uint64_t z = rand64(sk ^ HZ_SYMMETRY_SALT, mix64(h));
-    return (int)(((z >> 32) * (uint64_t)G) >> 32);
+    return sym_frame_of_key(exact_key_of_words(w), sk, G);
 }
 
 // Pile words 18..20 of T_g (the hand in the high half of word 20 stays): new position j < m holds old pile pi^-1[j].

@@ -213,6 +213,13 @@ class InferenceNet:
         (hz_tree_select layout HZ_LAYOUT_T16K) and evaluated with ``forward_tiles``."""
         return self.hand is not None and self.heads is not None and self.use_fused_heads and self.heads["C"] == 128 and self.heads["H"] == 256
 
+    @property
+    def row_invariant(self):
+        """True when a board's outputs do not depend on its row, its neighbours in the batch or the active count (the
+        precondition of the leaf evaluation cache, tree.EvalCache): the tile path, whose tower and heads compute every
+        board on its own with a fixed schedule.  The cuDNN path picks kernels by batch shape and promises no such thing."""
+        return self.wants_tiles
+
     def leaf_buffers(self, rows):
         """(board, glob, logits, value) static buffers for ``rows`` leaves per step."""
         dev = self.device

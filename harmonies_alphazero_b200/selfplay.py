@@ -22,7 +22,7 @@ import numpy as np
 import torch
 
 from . import batched as hb
-from .tree import BatchedMCTS
+from .tree import BatchedMCTS, EvalCache
 
 
 @dataclass
@@ -44,6 +44,11 @@ class SelfPlayConfig:
     max_moves: int = 200           # hard cap per game (structural maximum is 160 actions)
     compact_live: bool = True      # play(): keep the live games in a dense slot prefix and search only those (the game tail costs what it uses)
     eval_symmetry: str = None      # None, "board" or "full": the network sees each leaf in a random symmetry frame (hz_tree_set_symmetry)
+    # Leaf evaluation cache (tree.EvalCache): entries per slot group, 0 = off.  Leaves that an earlier step of the game
+    # evaluated, and terminal leaves, skip the network; the trajectories stay bit-identical.  One search of every slot
+    # needs about n_slots * num_simulations entries (leaves_per_step rows per simulation step) at about 600 B each; fewer
+    # entries evict and cost hits, never correctness.  Needs a row-invariant network (InferenceNet on the tile path).
+    eval_cache: int = 0
 
     @classmethod
     def from_mcts_config(cls, mcts_config, **kw):
@@ -150,6 +155,15 @@ class RolloutEvaluator:
         raise RuntimeError("RolloutEvaluator is evaluated on the tree (hz_tree_rollout_eval), not on tensors")
 
 
+def check_cacheable(net):
+    """Raise ValueError unless ``net`` may sit behind the leaf evaluation cache: a network evaluator whose outputs are
+    row-invariant.  The synthetic and rollout evaluators run on the tree (rollout values depend on the search key)."""
+    if isinstance(net, (SyntheticEvaluator, RolloutEvaluator)) or getattr(net, "tree_eval", False):
+        raise ValueError("the leaf evaluation cache caches network rows: it does not apply to tree-side evaluators")
+    if not getattr(net, "row_invariant", False):
+        raise ValueError("the leaf evaluation cache needs a row-invariant evaluator (net.row_invariant): a hit must equal a fresh evaluation")
+
+
 class _Group:
     """A contiguous range of slots with its own trees, static network buffers, CUDA graph and
     stream.  Two groups on two streams let one group's tree kernels (HBM/latency-bound) run
@@ -179,6 +193,16 @@ class _Group:
             self.glob = torch.zeros((rows, 42), dtype=dt, device=dev)
             self.logits = torch.zeros((rows, 143), dtype=torch.float32, device=dev)
             self.value = torch.zeros(rows, dtype=torch.float32, device=dev)
+        self.cache = None
+        if cfg.eval_cache:
+            check_cacheable(net)
+            self.cache = EvalCache(cfg.eval_cache, rows, device=dev)
+            self.cache_version = None
+            # the network's compact output (rows 0..n_eval-1) and the leaf row of each of its rows
+            self.net_logits = torch.zeros((rows, 143), dtype=torch.float32, device=dev)
+            self.net_value = torch.zeros(rows, dtype=torch.float32, device=dev)
+            self.eval_rows = torch.zeros(rows, dtype=torch.int32, device=dev)
+            self.n_eval = torch.zeros(1, dtype=torch.int32, device=dev)
         self.noise = None if cfg.testing else torch.ones((n, 143), dtype=torch.float32, device=dev)
         self.alpha = None if cfg.testing else torch.full((n, 143), cfg.dirichlet_alpha, dtype=torch.float32, device=dev)
         self.graph = None
@@ -202,19 +226,32 @@ class _Group:
             t.rollout_eval(self.logits, self.value, o.net.rollouts)
             t.expand_backup(self.logits, self.value, is_logits=False, noise=self.noise, eps=o.cfg.dirichlet_epsilon)
             return
+        if self.cache is not None:     # select -> network on the n_eval missed rows -> fill -> expand+backup
+            t.select_cached(self.cache, o.cfg.cpuct, self.board, self.glob, self.logits, self.value, self.eval_rows, self.n_eval,
+                            dtype=o.net.dtype, channels_last=o.channels_last, pad40=o.pad40, tiles=self.tiles)
+            self._evaluate((self.net_logits, self.net_value), self.n_eval)
+            self.cache.fill(self.net_logits, self.net_value, self.eval_rows, self.n_eval, self.logits, self.value)
+            t.expand_backup(self.logits, self.value, is_logits=True, noise=self.noise, eps=o.cfg.dirichlet_epsilon)
+            return
         t.select(o.cfg.cpuct, self.board, self.glob, dtype=o.net.dtype, channels_last=o.channels_last, pad40=o.pad40, tiles=self.tiles)
         if getattr(o.net, "tree_eval", False):
             t.fake_eval(self.logits, self.value)       # priors, not logits
-        elif self.tiles:
-            o.net.forward_tiles(self.board, self.glob, self.glob.shape[0], out=(self.logits, self.value), n_active=self.n_active[1:2], tag=self.lo)
-        elif o._net_takes_out:        # InferenceNet writes straight into the static buffers
-            o.net(self.board, self.glob, out=(self.logits, self.value))
         else:
-            logits, value = o.net(self.board, self.glob)
-            self.logits.copy_(logits)
-            self.value.copy_(value)
+            self._evaluate((self.logits, self.value), self.n_active[1:2])
         t.expand_backup(self.logits, self.value, is_logits=not getattr(o.net, "tree_eval", False), noise=self.noise,
                         eps=o.cfg.dirichlet_epsilon)
+
+    def _evaluate(self, out, n_active):
+        """the network on the leaf buffers into ``out``; the tile path computes rows 0..n_active-1 only (a device word)"""
+        o = self.o
+        if self.tiles:
+            o.net.forward_tiles(self.board, self.glob, self.glob.shape[0], out=out, n_active=n_active, tag=self.lo)
+        elif o._net_takes_out:        # InferenceNet writes straight into the static buffers
+            o.net(self.board, self.glob, out=out)
+        else:
+            logits, value = o.net(self.board, self.glob)
+            out[0].copy_(logits)
+            out[1].copy_(value)
 
     def capture(self):
         """Warm up (cuDNN algorithm selection must happen outside capture) and capture one
@@ -278,12 +315,18 @@ class BatchedSelfPlay:
         main = torch.cuda.current_stream(self.device)
         for g in self.groups:
             g.prepare(states)
-            if g.graph is not None and g.graph_version != getattr(self.net, "version", 0):
+            version = getattr(self.net, "version", 0)
+            if g.cache is not None and g.cache_version != version:
+                g.cache.clear()                   # entries of other weights are stale
+                g.cache_version = version
+            if g.graph is not None and g.graph_version != version:
                 g.graph = None                    # the network was reloaded: the captured launches point at the old weights
             if cfg.use_cuda_graph and g.graph is None:
                 g.capture()
-                g.graph_version = getattr(self.net, "version", 0)
+                g.graph_version = version
                 g.tree.reset(states[g.lo:g.hi])   # the warm-up/capture advanced the trees
+                if g.cache is not None:
+                    g.cache.clear()               # its entries are valid, but its counters would count the warm-up
         for g in self.groups:
             if g.stream is not None:
                 g.stream.wait_stream(main)
@@ -329,6 +372,8 @@ class BatchedSelfPlay:
         compact = cfg.compact_live and self.n_groups == 1
         for g in self.groups:
             g.set_active(g.hi - g.lo)             # (a previous call that raised may have left a smaller active prefix)
+            if g.cache is not None:
+                g.cache.clear()                   # stats["eval_cache"] counts this call
         torch.cuda.synchronize(dev)
         t0 = time.perf_counter()
         step = 0
@@ -408,4 +453,10 @@ class BatchedSelfPlay:
         stats = {"sims": live_sims, "seconds": secs, "sims_per_s": live_sims / secs if secs > 0 else 0.0,
                  "games": int(finished.sum().item()), "examples": int(S.shape[0]), "move_steps": step,
                  "searched_slots": searched_slots}
+        if self.groups[0].cache is not None:
+            c = dict(zip(EvalCache.COUNTERS, torch.stack([g.cache.counters() for g in self.groups]).sum(dim=0).tolist()))
+            steps = step * (cfg.num_simulations // max(1, int(cfg.leaves_per_step)))
+            c.update(hit_rate=c["hits"] / max(1, c["looked_up"]), terminal_fraction=c["terminal"] / max(1, c["looked_up"]),
+                     net_rows_per_step=c["misses"] / max(1, steps), bytes=sum(g.cache.bytes for g in self.groups))
+            stats["eval_cache"] = c
         return Trajectories(S, V, z, G + cfg.first_game_id, M, stats)

@@ -95,6 +95,29 @@ class BatchedMCTS:
                 "hz_tree_select",
             )
 
+    def select_cached(self, cache, cpuct, board, glob, policy, value, eval_rows, n_eval, leaf_states=None, dtype=torch.float32,
+                      channels_last=False, pad40=False, tiles=False):
+        """``select`` through the leaf evaluation cache (hz_tree_select_cached): terminal leaves get no network row, hits
+        write their stored row into (policy, value), misses are encoded into the dense rows 0..n_eval-1 of (board, glob)
+        with eval_rows[m] = their leaf row.  n_eval: int32 device tensor with one element (zeroed by the call)."""
+        code = {torch.float32: F32, torch.bfloat16: BF16}[dtype]
+        layout = 3 if tiles else 2 if pad40 else (NHWC if channels_last else NCHW)
+        if tiles:
+            assert board.dtype == torch.uint8 and board.numel() >= (self.rows + 15) // 16 * 71680 and glob.shape[0] == self.rows
+        else:
+            assert board.shape[1] == (40 if pad40 else 38) and board.shape[0] == self.rows and glob.shape[0] == self.rows
+        assert policy.dtype == torch.float32 and policy.shape == (self.rows, 143) and policy.is_contiguous()
+        assert value.dtype == torch.float32 and value.numel() == self.rows and value.is_contiguous()
+        assert eval_rows.dtype == torch.int32 and eval_rows.numel() >= self.rows and n_eval.dtype == torch.int32
+        with torch.cuda.device(self.device):
+            _lib.check(
+                self.lib.hz_tree_select_cached(
+                    self.handle, cache.handle, float(cpuct), _ptr(leaf_states), _ptr(board), _ptr(glob), code, layout,
+                    _ptr(policy), _ptr(value), _ptr(eval_rows), _ptr(n_eval), self._stream(),
+                ),
+                "hz_tree_select_cached",
+            )
+
     def expand_backup(self, policy, value, is_logits=False, noise=None, eps=0.0):
         assert policy.dtype == torch.float32 and policy.shape == (self.rows, 143) and policy.is_contiguous()
         assert value.dtype == torch.float32 and value.numel() == self.rows and value.is_contiguous()
@@ -173,6 +196,61 @@ class BatchedMCTS:
             self.select(cpuct)
             self.fake_eval(policy, value)
             self.expand_backup(policy, value, noise=noise, eps=eps)
+
+
+class EvalCache:
+    """Leaf evaluation cache (hz_evalcache_*): ``entries`` stored evaluator rows (a multiple of 8, about 600 bytes each)
+    keyed by the leaf's exact canonical key and its evaluation frame, for trees of up to ``max_rows`` leaf rows per step.
+    A hit returns the bits the evaluator returned, so searches are unchanged, provided the evaluator is row-invariant
+    (a board's outputs do not depend on its row, its neighbours or the batch size).  Clear it when the weights change."""
+
+    COUNTERS = ("looked_up", "hits", "terminal", "misses", "inserts", "evictions")
+
+    def __init__(self, entries, max_rows, device="cuda"):
+        self.lib = _lib.load()
+        self.entries, self.max_rows, self.device = int(entries), int(max_rows), torch.device(device)
+        nbytes = self.lib.hz_evalcache_bytes(self.entries, self.max_rows)
+        if nbytes == 0:
+            raise ValueError("eval cache entries must be a positive multiple of 8 (and max_rows positive)")
+        self.workspace = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)   # zeroed: empty, counters at 0
+        h = C.c_void_p()
+        _lib.check(self.lib.hz_evalcache_create(C.byref(h), self.workspace.data_ptr(), nbytes, self.entries, self.max_rows),
+                   "hz_evalcache_create")
+        self.handle = h
+        self.bytes = nbytes
+
+    def __del__(self):
+        h, self.handle = getattr(self, "handle", None), None
+        if h:
+            self.lib.hz_evalcache_destroy(h)
+
+    def _stream(self):
+        return torch.cuda.current_stream(self.device).cuda_stream
+
+    def clear(self):
+        """Drop every entry and zero the counters (after a weight reload)."""
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.hz_evalcache_clear(self.handle, self._stream()), "hz_evalcache_clear")
+
+    def counters(self):
+        """int64[6] device tensor of the counters since the last clear (order: ``COUNTERS``)."""
+        out = torch.empty(6, dtype=torch.int64, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.hz_evalcache_stats(self.handle, _ptr(out), self._stream()), "hz_evalcache_stats")
+        return out
+
+    def stats(self):
+        """dict of the counters since the last clear: looked_up, hits, terminal, misses, inserts, evictions."""
+        return dict(zip(self.COUNTERS, self.counters().tolist()))
+
+    def fill(self, net_logits, net_value, eval_rows, n_eval, policy, value):
+        """After the network ran on the rows of ``select_cached``: row m of (net_logits, net_value) goes to row eval_rows[m]
+        of (policy, value) and into the cache, for m < n_eval."""
+        assert net_logits.dtype == torch.float32 and net_logits.is_contiguous() and net_value.dtype == torch.float32
+        assert policy.dtype == torch.float32 and policy.is_contiguous() and value.dtype == torch.float32
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.hz_evalcache_fill(self.handle, _ptr(net_logits), _ptr(net_value), _ptr(eval_rows), _ptr(n_eval),
+                                                  _ptr(policy), _ptr(value), self._stream()), "hz_evalcache_fill")
 
 
 def search_keys_tensor(keys, device="cuda"):

@@ -398,6 +398,60 @@ int hz_tree_stats(hz_tree *t, int32_t *n_nodes, int32_t *n_edges, uint8_t *statu
 int hz_tree_root_edges(hz_tree *t, int32_t *N, double *W, float *P, int32_t *child,
                        void *stream);
 
+/* ---- leaf evaluation cache -----------------------------------------------------------------
+ * An opt-in memo of the evaluator's rows, so that a step sends only the leaves that need the network through it.  The
+ * reference builds a new tree for every move and so does this library, but three of the four actions of a turn (the pile
+ * choice and the first two placements) draw nothing: the positions under the played child are then exactly positions
+ * that the previous search of the game evaluated.  A hit returns the bits the evaluator would return, so every search is
+ * bit-identical with the cache on or off (given the precondition below).
+ *  key:       (canon_hash(leaf, HZ_KEY_EXACT), frame): words 0..22 with meta & 0x0F, every bit the encoders read, in
+ *             both tree key modes (HZ_KEY_REFERENCE node keys alias positions whose encodings differ, so they are not
+ *             used); frame = g_r of hz_tree_set_symmetry (0 with the mode off).  g_r depends on the search key, so
+ *             under HZ_SYM_BOARD about a quarter of the hits survive and under HZ_SYM_FULL about none.
+ *  value:     the evaluator's raw row as hz_tree_expand_backup reads it: 143 fp32 (logits with is_logits) + the fp32
+ *             value.  Identity = key equality, as in the tree; with -DHZ_TREE_FULL_COMPARE=1 an entry also keeps its
+ *             23 key words and a hit compares them.
+ *  capacity:  `entries` (a positive multiple of 8, <= 2^31) in buckets of 8 ways; an insert evicts the way whose last
+ *             insert or hit is oldest (by a step stamp).  Eviction costs hits, never correctness.  About 600 bytes per
+ *             entry: one search of n trees needs about n * sims * leaves entries.
+ *  rows:      hz_tree_select_cached sorts the leaf rows r = t*K + j of the active trees:
+ *             - a terminal leaf gets no network row (hz_tree_expand_backup uses its outcome);
+ *             - a hit writes its stored row into policy[r], value[r];
+ *             - a miss gets network row m from a dense prefix, eval_rows[m] = r, and the leaf is encoded into row m of
+ *               (board, glob) in the layout of the call (as hz_tree_select would encode row r).  The order of the
+ *               misses is set by atomics.
+ *             *n_eval (a DEVICE int32, zeroed by the call) = the number of misses: pass it as n_active to
+ *             hz_tower_forward_heads and hz_net_heads_fc_active, so one captured CUDA graph serves every step.  Then
+ *             hz_evalcache_fill copies row m of the network's compact output to policy[eval_rows[m]],
+ *             value[eval_rows[m]] and inserts it; hz_tree_expand_backup follows unchanged.
+ *  precondition: the evaluator is row-invariant: a board's output bits do not depend on its row, its neighbours in the
+ *             batch or the active count.  Otherwise a hit need not equal a fresh evaluation.
+ *  counters:  int64 [6] since the last hz_evalcache_clear: rows looked up, hits, terminal rows, misses, inserts,
+ *             evictions of live entries.  (looked up = hits + terminal + misses.)
+ * The workspace must be zeroed (or cleared with hz_evalcache_clear) before the first select.  Clear after a weight
+ * reload: entries of other weights would be stale.  One cache serves one stream at a time. */
+typedef struct hz_evalcache hz_evalcache;
+
+/* Bytes of device workspace (0 for bad sizes).  max_rows: leaf rows per step of the trees it serves (n_trees * leaves). */
+size_t hz_evalcache_bytes(int64_t entries, int max_rows);
+/* Over caller-owned, 256-byte-aligned workspace (HZ_ERR_WORKSPACE if short or misaligned). */
+int hz_evalcache_create(hz_evalcache **out, void *workspace, size_t bytes, int64_t entries, int max_rows);
+int hz_evalcache_destroy(hz_evalcache *c);
+/* Drops every entry and zeroes the counters. */
+int hz_evalcache_clear(hz_evalcache *c, void *stream);
+/* counters: DEVICE int64 [6] (see above). */
+int hz_evalcache_stats(hz_evalcache *c, int64_t *counters, void *stream);
+/* hz_tree_select with the cache (rows above).  board and glob are required; policy [n_trees*leaves,143] and value
+ * [n_trees*leaves] receive the hits; eval_rows [n_trees*leaves] int32; n_eval: DEVICE int32.  HZ_ERR_ARG when
+ * n_trees * leaves > max_rows of the cache. */
+int hz_tree_select_cached(hz_tree *t, hz_evalcache *c, float cpuct, void *leaf_states, void *board, void *glob,
+                          int dtype, int layout, float *policy, float *value, int32_t *eval_rows, int32_t *n_eval,
+                          void *stream);
+/* After the network: net_logits [>= *n_eval, 143] and net_value [>= *n_eval] are its compact output (rows m of the
+ * select's encoding).  Scatters them to policy/value at eval_rows[m] and inserts them. */
+int hz_evalcache_fill(hz_evalcache *c, const float *net_logits, const float *net_value, const int32_t *eval_rows,
+                      const int32_t *n_eval, float *policy, float *value, void *stream);
+
 /* ---- network tail (model.py) ----------------------------------------------------------- */
 
 /* Fused policy/value heads of AlphaZeroModel.forward (model.py:340-355) on the residual
