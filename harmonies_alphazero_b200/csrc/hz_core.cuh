@@ -852,8 +852,14 @@ __device__ __forceinline__ bool playout_round(State& s, RandTab rtab) {
 // Plays s with hz_playout's semantics until the game is over, no move is legal, or max_steps actions were applied, and
 // returns the number of actions applied.  The final scoring is deferred: a game that ended here is left at phase game_over
 // with winner None, and the caller scores it with the lanes of the block converged (partial_scores + resolve_water).
-// lut and rtab: the block's shared neighbour LUT and rand table.
-__device__ __forceinline__ uint32_t play_random(State& s, int max_steps, const NbrLut* lut, RandTab rtab) {
+// lut and rtab: the block's shared neighbour LUT and rand table.  mark(i) runs at the end of loop iteration i (a whole
+// round on the round path, one action otherwise); only k_playout's -DHZ_PLAYOUT_TIMELINE build passes one that does
+// anything.
+struct NoMark {
+    __device__ __forceinline__ void operator()(int) const {}
+};
+template <typename Mark = NoMark>
+__device__ __forceinline__ uint32_t play_random(State& s, int max_steps, const NbrLut* lut, RandTab rtab, Mark mark = Mark()) {
     uint32_t k = 0;
 #ifdef HZ_PLAYOUT_CHECKED   // A/B: the three general calls on a mover-relative state (validation + board copy in apply_move)
     if (player_of(s)) swap_boards(s);
@@ -869,16 +875,19 @@ __device__ __forceinline__ uint32_t play_random(State& s, int max_steps, const N
     // in max_steps, single steps elsewhere: mid-turn starts, the tail of a max_steps slice and irregular rounds.
     // HZ_PLAYOUT_STEPWISE: steps only (A/B).  A step branches on the player once: fresh games move in lockstep (same
     // player, same phase in every lane until games end), and inside a branch the mover's planes are fixed registers.
+    int it = 0;
     while ((int)k < max_steps && phase_of(s) != HZ_PHASE_OVER) {
 #ifndef HZ_PLAYOUT_STEPWISE
         if ((int)k <= max_steps - 8 && round_ready(s) && playout_round(s, rtab)) {
             k += 8;
+            mark(it++);
             continue;
         }
 #endif
         const bool ok = player_of(s) ? playout_step<1, true>(s, lut, rtab) : playout_step<0, true>(s, lut, rtab);
         if (!ok) break;  // stuck position (no legal move, not over): harmonies_engine.py:205-208
         k++;
+        mark(it++);
     }
 #endif
     return k;

@@ -259,6 +259,58 @@ constexpr int PTPB = 64;   // 65,536 games -> 1024 blocks: 6.9 per SM, <2 % tail
 // (meta word, score word, actions played) leave the chip: 8 B in, 12 B out per game.
 // 7 blocks per SM hold a 65,536-game wave: the register cap of 7 x 64 threads (<= 144 per thread) leaves the round path
 // room without spills, where the compiler's own choice for __launch_bounds__(PTPB) alone was 80 registers and a spill.
+#ifdef HZ_PLAYOUT_TIMELINE
+// Device-side phase timeline of k_playout, profiling builds only (profiles/playout_timeline.py).  Per warp TL_WORDS
+// uint64: [0] %smid, then per event e the pair [1 + 2e] %globaltimer (ns), [2 + 2e] clock64 (SM cycles), written by the
+// warp's lowest active lane.  Events: kernel entry, tables ready (after the block barrier), records in registers, end of
+// play_random, after partial_scores, after resolve_water, after the store, and TL_ROUND + i at the end of play_random's
+// loop iteration i (a whole round on the round path; iterations >= TL_ROUNDS - 1 share the last slot).
+enum { TL_ENTRY, TL_TABLES, TL_RECORDS, TL_PLAYED, TL_PARTIAL, TL_RESOLVED, TL_STORED, TL_ROUND };
+constexpr int TL_ROUNDS = 24, TL_WORDS = 64, TL_SINK = 63;
+static_assert(1 + 2 * (TL_ROUND + TL_ROUNDS) <= TL_SINK, "timeline slots overlap the sink word");
+__device__ unsigned long long* g_tl = nullptr;
+__device__ long long g_tl_warps = 0;
+// dep: a value the stamp must wait for (the volatile store to the sink word orders the clock reads after its arrival)
+__device__ __forceinline__ void tl_mark(unsigned long long* w, int e, uint32_t dep = 0) {
+    if (w && (int)(threadIdx.x & 31) == __ffs(__activemask()) - 1) {
+        *reinterpret_cast<volatile unsigned long long*>(w + TL_SINK) = dep;
+        unsigned long long t;
+        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t) :: "memory");
+        w[1 + 2 * e] = t;
+        w[2 + 2 * e] = clock64();
+    }
+}
+struct TlRoundMark {
+    unsigned long long* w;
+    __device__ __forceinline__ void operator()(int i) const { tl_mark(w, TL_ROUND + min(i, TL_ROUNDS - 1)); }
+};
+#define HZ_TL(e, ...) tl_mark(tl, e, ##__VA_ARGS__)
+#else
+#define HZ_TL(e, ...) do { } while (0)
+#endif
+
+// The block's two tables (3 KB neighbour LUT, 4 KB rand table) in one round trip: each thread issues all of its 16 loads
+// before its first shared-memory store.  build_nbr_lut / build_rand_table loop over blockDim.x and wait for one batch of
+// loads per iteration: four round trips in a row, 2.3-2.4 us of a 65,536-game wave on a B200 at 1,000 W (playout_timeline.py)
+// during which no warp of the SM has anything else to do.  -DHZ_PLAYOUT_LOOPED_TABLES keeps the looped copy (A/B).
+struct PlayoutTables {
+    uint32_t lut[768 / PTPB];
+    uint4 rt[RTAB_N / 2 / PTPB];
+};
+static_assert(768 % PTPB == 0 && (RTAB_N / 2) % PTPB == 0, "k_playout's table copy: whole rows per thread");
+__device__ __forceinline__ void fetch_tables(PlayoutTables& t) {
+#pragma unroll
+    for (int i = 0; i < 768 / PTPB; i++) t.lut[i] = __ldg(NBR_LUT_G + threadIdx.x + i * PTPB);
+#pragma unroll
+    for (int i = 0; i < RTAB_N / 2 / PTPB; i++) t.rt[i] = __ldg(reinterpret_cast<const uint4*>(RAND_TAB_G) + threadIdx.x + i * PTPB);
+}
+__device__ __forceinline__ void store_tables(const PlayoutTables& t, NbrLut* lut, uint64_t* rtab) {
+#pragma unroll
+    for (int i = 0; i < 768 / PTPB; i++) (&lut->t[0][0])[threadIdx.x + i * PTPB] = t.lut[i];
+#pragma unroll
+    for (int i = 0; i < RTAB_N / 2 / PTPB; i++) reinterpret_cast<uint4*>(rtab)[threadIdx.x + i * PTPB] = t.rt[i];
+}
+
 template <bool FROM_KEYS>
 __global__ void __launch_bounds__(PTPB, 7) k_playout(void* states, int64_t n, int max_steps, uint32_t* steps,
                                                   unsigned long long* total_steps, const uint64_t* keys,
@@ -266,11 +318,31 @@ __global__ void __launch_bounds__(PTPB, 7) k_playout(void* states, int64_t n, in
     __shared__ NbrLut lut;
     __shared__ __align__(16) uint64_t rtab_s[RTAB_N];
     __shared__ WaterQueue<2 * PTPB, 2 * PTPB> wq;
+#ifdef HZ_PLAYOUT_TIMELINE
+    unsigned long long* tl = nullptr;
+    {
+        const long long warp = ((long long)blockIdx.x * PTPB + threadIdx.x) >> 5;
+        if (g_tl && warp < g_tl_warps) tl = g_tl + warp * TL_WORDS;
+        uint32_t smid;
+        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+        if (tl && (threadIdx.x & 31) == 0) tl[0] = smid;
+        HZ_TL(TL_ENTRY);
+    }
+#endif
+#ifdef HZ_PLAYOUT_LOOPED_TABLES
     build_nbr_lut(&lut);
     build_rand_table(rtab_s);
+#else
+    {
+        PlayoutTables tabs;
+        fetch_tables(tabs);
+        store_tables(tabs, &lut, rtab_s);
+    }
+#endif
     const RandTab rtab = rand_table_handle(rtab_s);
     water_queue_init(&wq);
     __syncthreads();
+    HZ_TL(TL_TABLES);
     int64_t g = (int64_t)blockIdx.x * PTPB + threadIdx.x;
     uint32_t k = 0;
     State s;
@@ -279,15 +351,26 @@ __global__ void __launch_bounds__(PTPB, 7) k_playout(void* states, int64_t n, in
     if (g < n) {
         if (FROM_KEYS) init_state(s, keys ? keys[g] : rand64(seed, first_id + (uint64_t)g), rtab);
         else load_state(s, states, g);
+#ifdef HZ_PLAYOUT_TIMELINE
+        uint32_t dep = 0;
+#pragma unroll
+        for (int i = 0; i < SW; i++) dep ^= s.w[i];
+        HZ_TL(TL_RECORDS, dep);
+        k = play_random(s, max_steps, &lut, rtab, TlRoundMark{tl});
+        HZ_TL(TL_PLAYED);
+#else
         k = play_random(s, max_steps, &lut, rtab);
+#endif
         // final scoring deferred to here: the lanes of the warp are converged again; rivers of >= 5
         // hexes go to the block's queue and get a whole warp each (resolve_water)
         fin = phase_of(s) == HZ_PHASE_OVER && winner_code(s) == 0;
         if (fin) partial_scores(s, &lut, &wq, s0, s1);
+        HZ_TL(TL_PARTIAL);
     }
     __syncthreads();
     resolve_water(&lut, &wq);
     __syncthreads();
+    HZ_TL(TL_RESOLVED);
     if (g < n) {
         if (fin) store_final_scores(s, s0 + wq.extra[threadIdx.x * 2], s1 + wq.extra[threadIdx.x * 2 + 1]);
         if (FROM_KEYS) {
@@ -299,6 +382,7 @@ __global__ void __launch_bounds__(PTPB, 7) k_playout(void* states, int64_t n, in
             if (steps) steps[g] = k;
         }
     }
+    HZ_TL(TL_STORED);
     if (total_steps) {
         uint32_t sum = k;
 #pragma unroll
@@ -555,5 +639,15 @@ int hz_playout_keys(const uint64_t* keys, int64_t n, uint64_t seed, uint64_t fir
                                                                             keys, seed, first_id, results);
     return hz_launched(1);
 }
+
+#ifdef HZ_PLAYOUT_TIMELINE
+// Profiling builds only, not part of the ABI: the following k_playout launches write their phase timeline to buf
+// (TL_WORDS uint64 per warp, in warp order; warps past n_warps record nothing).  buf = NULL turns it off.
+int hz_playout_set_timeline(unsigned long long* buf, long long n_warps) {
+    cudaError_t e = cudaMemcpyToSymbol(g_tl, &buf, sizeof buf);
+    if (e == cudaSuccess) e = cudaMemcpyToSymbol(g_tl_warps, &n_warps, sizeof n_warps);
+    return hz_record_launch(0, e);
+}
+#endif
 
 }  // extern "C"

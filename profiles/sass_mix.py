@@ -5,8 +5,8 @@ k_playout<false> and k_playout<true> and splits each into basic blocks.  The rou
 round is one straight line of several hundred instructions; the next largest block is a quarter of it or less), the
 prologue is everything ahead of the first BAR.SYNC (the block's tables are ready there).  Opcodes on the integer ALU pipe
 (LOP3, SEL, SHF, ISETP, IADD3, LEA, PRMT, ...) are summed apart from IMAD, which issues to the FMA pipe.  Local-memory
-accesses (STL, LDL: register spills) are counted in the round body, the prologue and the rest of the kernel.  No GPU
-needed.
+accesses (STL, LDL: register spills) are counted in the round body, the prologue and the rest of the kernel, and each
+instantiation's registers, stack, shared and local memory are printed from `cuobjdump -res-usage`.  No GPU needed.
 
     python profiles/sass_mix.py [--src DIR]     # DIR: another checkout's harmonies_alphazero_b200/csrc (A/B)
 """
@@ -40,7 +40,15 @@ def cubin_sass(csrc):
         cubin = os.path.join(tmp, "hz_engine.cubin")
         subprocess.run([nvcc] + build.NVCC_FLAGS + ["-cubin", "-o", cubin, os.path.join(csrc, "hz_engine.cu")], check=True)
         text = subprocess.run([os.path.join(cuda_bin, "nvdisasm"), cubin], check=True, capture_output=True, text=True).stdout
-    return text
+        res = subprocess.run([os.path.join(cuda_bin, "cuobjdump"), "-res-usage", cubin], check=True, capture_output=True,
+                             text=True).stdout
+    return text, res
+
+
+def resources(res, mangled):
+    """'REG:104 STACK:0 SHARED:8452 LOCAL:0' of one kernel"""
+    line = res.split("Function " + mangled + ":")[1].strip().splitlines()[0]
+    return " ".join(f for f in line.split() if f.split(":")[0] in ("REG", "STACK", "SHARED", "LOCAL"))
 
 
 def kernel_sass(text, mangled):
@@ -82,11 +90,11 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--src", default=build.CSRC, help="csrc directory to compile (default: this tree's)")
     a = ap.parse_args()
-    text = cubin_sass(a.src)
+    text, res = cubin_sass(a.src)
     for name, mangled in KERNELS.items():
         ins, blocks = blocks_of(kernel_sass(text, mangled))
         sizes = sorted((len(b) for b in blocks), reverse=True)
-        print(f"{a.src}: {name} {len(ins)} instructions, largest basic blocks {sizes[:4]}")
+        print(f"{a.src}: {name} {len(ins)} instructions, largest basic blocks {sizes[:4]}, {resources(res, mangled)}")
         body = max(blocks, key=len)
         report("round body (largest basic block)", body)
         report("prologue (ahead of the first BAR.SYNC)", ins[:ins.index("BAR")])
