@@ -42,6 +42,9 @@ SIGNATURES = {
     "hz_tree_leaf_frames": (_i, [_vp, _vp, _vp]),
     "hz_tree_select": (_i, [_vp, _f, _vp, _vp, _vp, _i, _i, _vp]),
     "hz_tree_expand_backup": (_i, [_vp, _vp, _vp, _i, _vp, _d, _vp]),
+    "hz_tree_gumbel_bytes": (C.c_size_t, [_vp, _i, _i]),
+    "hz_tree_set_gumbel": (_i, [_vp, _vp, C.c_size_t, _i, _i, _f, _f, _f, _vp]),
+    "hz_tree_gumbel_root": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "hz_tree_fake_eval": (_i, [_vp, _vp, _vp, _vp]),
     "hz_tree_rollout_eval": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "hz_tree_root_policy": (_i, [_vp, _vp, _vp, _vp]),

@@ -51,7 +51,7 @@ GREEDY = "greedy"   # pass as either side to play the 1-ply greedy agent of eval
 
 
 def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cuda", seed=0, key_mode=hb.KEY_REFERENCE, leaves=1,
-               symmetry=None, eval_cache=0):
+               symmetry=None, eval_cache=0, search="puct"):
     """Returns dict(candidate_wins, best_wins, draws, win_rate, games).  Each side is an
     InferenceNet on ``device``, ``arena.GREEDY`` (run_tournament of evaluation.py:7-65:
     AlphaZero vs the greedy agent, sides alternating by game index) or a
@@ -62,8 +62,18 @@ def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cud
     (BatchedMCTS.set_symmetry).
     eval_cache: entries of a leaf evaluation cache per side (tree.EvalCache), 0 = off.  One player makes all four actions
     of a turn, so a side's searches reuse its own earlier evaluations; the results are unchanged.  Network sides must be
-    row-invariant; a rollout side raises ValueError."""
+    row-invariant; a rollout side raises ValueError.
+    search: "puct" (the reference's), "gumbel" (BatchedMCTS.set_gumbel without noise: the move of the greedy Gumbel
+    search; m, c_visit, c_scale from mcts_config_eval's gumbel_m / gumbel_c_visit / gumbel_c_scale, default 16 / 50 / 0.1)
+    or a pair (candidate's, best's).  Gumbel needs leaves = 1."""
     dev = torch.device(device)
+    modes = (search, search) if isinstance(search, str) else tuple(search)
+    if len(modes) != 2 or any(x not in ("puct", "gumbel") for x in modes):
+        raise ValueError("search must be 'puct', 'gumbel' or a (candidate, best) pair of them")
+    if "gumbel" in modes and leaves != 1:
+        raise ValueError("Gumbel search runs one simulation in flight per tree: leaves must be 1")
+    gumbel_kw = dict(m=int(mcts_config_eval.get("gumbel_m", 16)), c_visit=float(mcts_config_eval.get("gumbel_c_visit", 50.0)),
+                     c_scale=float(mcts_config_eval.get("gumbel_c_scale", 0.1)), scale=0.0)
     if eval_cache:
         for side in (candidate_net, best_net):
             if side is not GREEDY:
@@ -121,8 +131,15 @@ def play_match(candidate_net, best_net, num_games, mcts_config_eval, device="cud
             if net is GREEDY:                                        # evaluation.py:137-196, one kernel
                 actions = hb.greedy_actions(states)
             else:
+                if modes[side] == "gumbel":
+                    tree.set_gumbel(num_sims=sims, **gumbel_kw)
+                else:
+                    tree.set_gumbel(None)
                 _search(tree, net, states, sims, cpuct, bufs, None if caches is None else caches[side], cbufs)
-                actions = tree.choose()                              # first max N: testing=True
+                if modes[side] == "gumbel":
+                    actions = tree.gumbel_root()[1]                  # gumbel_scale = 0: the greedy Gumbel move
+                else:
+                    actions = tree.choose()                          # first max N: testing=True
             actions = torch.where(live, actions, torch.full_like(actions, -1))
             hb.apply(states, actions)
         if tree is not None:

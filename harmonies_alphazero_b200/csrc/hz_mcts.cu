@@ -13,13 +13,26 @@
 //           (MCTS.py:184-186; -DHZ_TREE_FULL_COMPARE=1 adds a 23-word compare on hits)
 // Parity mode is one in-flight simulation per tree (the reference is strictly sequential,
 // MCTS.py:291-352); parallelism comes from thousands of concurrent trees.
+#include <float.h>
 #include <math.h>
 #include <stdlib.h>
+
+#include <algorithm>
+#include <cmath>
+#include <vector>
 
 #include "hz_common.cuh"
 #include "hz_core.cuh"
 #include "hz_evalcache.cuh"
 #include "hz_sym.cuh"
+
+// Gumbel mode (hz_tree_set_gumbel), passed to the kernels that use it as a parameter of their own; node_value == NULL: off
+struct hz_gumbel_args {
+    float* node_value;        // [n_trees * max_nodes] the evaluator's value of every node, stored when the node is expanded
+    const int32_t* table;     // [(m + 1) * n_sims] considered-visit table: table[k * n_sims + i]
+    int m, n_sims;
+    float c_visit, c_scale, scale;
+};
 
 struct hz_tree {
     int n_trees, max_sims, max_nodes, max_edges, table_size, key_mode;
@@ -50,6 +63,13 @@ struct hz_tree {
     int sym_mode;           // HZ_SYM_* of the launches that follow (hz_tree_set_symmetry)
     int frames_on;          // host side: the last hz_tree_select ran with a mode on
 };
+
+// What hz_tree_create allocates: the handle the kernels take by value, and host-only state that stays out of their
+// parameters (so the kernels of the modes that do not use it keep their parameter layout).
+struct hz_tree_host : hz_tree {
+    hz_gumbel_args gumbel;  // hz_tree_set_gumbel
+};
+static inline hz_gumbel_args& gumbel_of(hz_tree* t) { return static_cast<hz_tree_host*>(t)->gumbel; }
 
 namespace hz {
 
@@ -190,13 +210,106 @@ __device__ __forceinline__ bool cache_row(const EvalCacheArgs& EC, const uint32_
     return true;
 }
 
+// ---- Gumbel search (hz_tree_set_gumbel; semantics in include/harmonies_b200.h) ----------------------------------------
+// Completed-Q transform of one node whose edges k = lane + 32 r (k < ne) are in registers, ns = sum N (already reduced),
+// vhat = the node's raw value.  Out: lg[r] = logit, sg[r] = sigma of edge k (0 past ne), mxn = max N.
+__device__ __forceinline__ void gumbel_sigma(const hz_gumbel_args& GB, int ne, int lane, int ns, const int (&N)[3],
+                                             const double (&W)[3], const float (&P)[3], float vhat, double (&lg)[3],
+                                             double (&sg)[3], int& mxn) {
+    double sp = 0.0;
+    int mx = 0;
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+        if (lane + 32 * r < ne) { sp += (double)P[r]; mx = max(mx, N[r]); }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        sp += __shfl_xor_sync(FULL, sp, o);
+        mx = max(mx, __shfl_xor_sync(FULL, mx, o));
+    }
+    double spi = 0.0, spq = 0.0;                                        // sums over the visited edges of clamped pi, pi * q
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+        if (lane + 32 * r < ne && N[r] > 0) {
+            const double pi = fmax((double)P[r] / sp, (double)FLT_MIN);
+            spi += pi;
+            spq += pi * (W[r] / (double)N[r]);
+        }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        spi += __shfl_xor_sync(FULL, spi, o);
+        spq += __shfl_xor_sync(FULL, spq, o);
+    }
+    const double vmix = ((double)vhat + (double)ns * (spi > 0.0 ? spq / spi : 0.0)) / (1.0 + (double)ns);
+    double qt[3], qmin = INFINITY, qmax = -INFINITY;
+#pragma unroll
+    for (int r = 0; r < 3; r++) {
+        qt[r] = N[r] > 0 ? W[r] / (double)N[r] : vmix;
+        if (lane + 32 * r < ne) { qmin = fmin(qmin, qt[r]); qmax = fmax(qmax, qt[r]); }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        qmin = fmin(qmin, __shfl_xor_sync(FULL, qmin, o));
+        qmax = fmax(qmax, __shfl_xor_sync(FULL, qmax, o));
+    }
+    const double span = fmax(qmax - qmin, 1e-8), vs = ((double)GB.c_visit + (double)mx) * (double)GB.c_scale;
+#pragma unroll
+    for (int r = 0; r < 3; r++) {
+        const bool on = lane + 32 * r < ne;
+        lg[r] = on ? log((double)fmaxf(P[r], FLT_MIN)) : 0.0;
+        sg[r] = on ? vs * ((qt[r] - qmin) / span) : 0.0;
+    }
+    mxn = mx;
+}
+
+// g(a) = scale * -log(-log(u)), u = ((rand64(sk ^ HZ_GUMBEL_SALT, a) >> 11) + 0.5) * 2^-53
+__device__ __forceinline__ double gumbel_noise(uint64_t skey, int action, float scale) {
+    const uint64_t z = rand64(skey ^ HZ_GUMBEL_SALT, (uint64_t)action);
+    return (double)scale * -log(-log(((double)(z >> 11) + 0.5) * 0x1p-53));
+}
+
+// root score of the edges with N == cv (sequential halving; -INFINITY elsewhere): max(-1e9, g + (logit - max logit) + sigma)
+__device__ __forceinline__ void gumbel_root_scores(const hz_gumbel_args& GB, uint64_t skey, int ne, int lane, int cv,
+                                                   const int (&N)[3], const int (&A)[3], const double (&lg)[3],
+                                                   const double (&sg)[3], double (&sc)[3]) {
+    double mlg = -INFINITY;
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+        if (lane + 32 * r < ne) mlg = fmax(mlg, lg[r]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mlg = fmax(mlg, __shfl_xor_sync(FULL, mlg, o));
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+        sc[r] = lane + 32 * r < ne && N[r] == cv ? fmax(-1e9, gumbel_noise(skey, A[r], GB.scale) + (lg[r] - mlg) + sg[r]) : -INFINITY;
+}
+
+// e[r] = exp(z[r] - max z) over the node's edges (0 past ne), returns their sum: softmax(z) = e / sum
+__device__ __forceinline__ double softmax_terms(int ne, int lane, const double (&z)[3], double (&e)[3]) {
+    double zm = -INFINITY;
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+        if (lane + 32 * r < ne) zm = fmax(zm, z[r]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) zm = fmax(zm, __shfl_xor_sync(FULL, zm, o));
+    double s = 0.0;
+#pragma unroll
+    for (int r = 0; r < 3; r++) {
+        e[r] = lane + 32 * r < ne ? exp(z[r] - zm) : 0.0;
+        s += e[r];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(FULL, s, o);
+    return s;
+}
+
 // ---- select: move_to_leaf (MCTS.py:63-149) + create_state_tensors(leaf) (MCTS.py:299) ---------
 // G = order of the symmetry group of the leaf frames (0: off, the reference's select)
 // CACHE: look every leaf up in the evaluation cache EC (hz_tree_select_cached); only misses are encoded, into the dense
 // network rows handed out by EC.n_eval.  EC is the last parameter, so the cache-off kernels' parameters keep their offsets.
-template <typename OT, int LAYOUT, int G, bool CACHE>
+// GUMBEL: the descent of hz_tree_set_gumbel (root: sequential halving, deeper: completed-Q selection) instead of PUCT;
+// K == 1.  GB follows EC for the same reason.
+template <typename OT, int LAYOUT, int G, bool CACHE, bool GUMBEL>
 __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, uint4* leaf_states, OT* board, OT* glob,
-                                                      EvalCacheArgs EC) {
+                                                      EvalCacheArgs EC, hz_gumbel_args GB) {
     __shared__ uint32_t sm_words[WPB][32];
     __shared__ uint32_t sm_mask[WPB][40];
     constexpr bool FAST40 = (LAYOUT == HZ_LAYOUT_NHWC40 || LAYOUT == HZ_LAYOUT_T16K) && sizeof(OT) == 2;
@@ -215,6 +328,8 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
     TreeView v = view_of(T, t);
     const int K = T.leaves;
     [[maybe_unused]] unsigned long long n_hit = 0, n_terminal = 0;
+    [[maybe_unused]] uint64_t gkey = 0;
+    if constexpr (GUMBEL) gkey = T.search_key[t];
     // K descents per tree and step.  K == 1 is the reference's move_to_leaf.  For K > 1 every
     // edge of an already chosen path carries an in-flight visit V: N' = N + V, W' = W - V
     // (a provisional loss for the mover), so the later descents of the step spread out.
@@ -228,6 +343,9 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
         while (ne != 0) {                                                // is_leaf, MCTS.py:18-20,76
             int N[3]; double W[3]; float P[3]; uint32_t C[3], CI[3];
             int ns = 0;
+            [[maybe_unused]] int A[3] = {0, 0, 0};
+            [[maybe_unused]] float vhat = 0.0f;
+            if constexpr (GUMBEL) vhat = GB.node_value[(size_t)t * T.max_nodes + node];   // with the edges: one round trip
 #pragma unroll
             for (int r = 0; r < 3; r++) {
                 int k = lane + 32 * r;
@@ -239,6 +357,7 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
                 P[r] = on ? v.edge_P[e0 + k] : 0.0f;
                 C[r] = on ? v.edge_child[e0 + k] : 0u;
                 CI[r] = on ? v.edge_cinfo[e0 + k] : 0u;
+                if (GUMBEL && depth == 0) A[r] = on ? v.edge_am[e0 + k] & 0xFF : 0;
                 if (K > 1 && on) {
                     int vl = v.edge_V[e0 + k];
                     N[r] += vl;
@@ -248,9 +367,29 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
             }
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) ns += __shfl_xor_sync(FULL, ns, o);               // :95-97
-            double sqrt_ns = sqrt(ns > 1 ? (double)ns : 1.0);                                  // :99
             double best = -INFINITY;
             int best_k = -1;
+            if constexpr (GUMBEL) {
+                double lg[3], sg[3], sc[3];
+                int mxn;
+                gumbel_sigma(GB, ne, lane, ns, N, W, P, vhat, lg, sg, mxn);
+                if (depth == 0) {                                        // root: the considered set of sequential halving
+                    const int kc = min(GB.m, ne), i = min(ns, GB.n_sims - 1);
+                    HZ_BOUND(kc * GB.n_sims + i, (GB.m + 1) * GB.n_sims, 105);
+                    gumbel_root_scores(GB, gkey, ne, lane, GB.table[kc * GB.n_sims + i], N, A, lg, sg, sc);
+                } else {                                                 // interior: softmax(logit + sigma) - N / (1 + sum N)
+                    double z[3], ez[3];
+#pragma unroll
+                    for (int r = 0; r < 3; r++) z[r] = lg[r] + sg[r];
+                    const double s = softmax_terms(ne, lane, z, ez);
+#pragma unroll
+                    for (int r = 0; r < 3; r++) sc[r] = ez[r] / s - (double)N[r] / (1.0 + (double)ns);
+                }
+#pragma unroll
+                for (int r = 0; r < 3; r++)
+                    if (lane + 32 * r < ne && sc[r] > best) { best = sc[r]; best_k = lane + 32 * r; }
+            } else {
+            double sqrt_ns = sqrt(ns > 1 ? (double)ns : 1.0);                                  // :99
 #pragma unroll
             for (int r = 0; r < 3; r++) {
                 int k = lane + 32 * r;
@@ -263,6 +402,7 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
                     if (sc > best) { best = sc; best_k = k; }            // strict >, ascending k: :118
                 }
             }
+            }
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) {
                 double ob = __shfl_xor_sync(FULL, best, o);
@@ -270,6 +410,7 @@ __global__ void __launch_bounds__(TTPB) k_tree_select(hz_tree T, float cpuct, ui
                 bool take = ok >= 0 && (best_k < 0 || ob > best || (ob == best && ok < best_k));
                 if (take) { best = ob; best_k = ok; }
             }
+            if (GUMBEL && best_k < 0 && depth == 0) best_k = 0;         // no edge has the considered count: argmax of -inf
             if (best_k < 0) break;                                       // :125-133
             uint32_t e = e0 + (uint32_t)best_k;
             if (depth > T.max_sims) { if (lane == 0) T.status[t] |= 4; break; }
@@ -392,9 +533,10 @@ __device__ __forceinline__ int frame_action(int a, uint32_t fr) {
 }
 
 // SYM: the leaf rows are in the frames of k_tree_select (hz_tree_set_symmetry); false = the reference's expansion
-template <bool SYM>
+// GUMBEL: an expansion also keeps the evaluator's value of the leaf in node_value (hz_tree_set_gumbel)
+template <bool SYM, bool GUMBEL>
 __global__ void __launch_bounds__(TTPB, HZ_EXPAND_MIN_BLOCKS) k_tree_expand_backup(hz_tree T, const float* policy, const float* value,
-                                                             int is_logits, const float* noise, double eps) {
+                                                             int is_logits, const float* noise, double eps, float* node_value) {
     __shared__ uint32_t sm_words[WPB][32];
     // scoring happens only for children that end the game: read the neighbour LUT in place
     // (global memory, L1-cached) instead of staging 3 KB per block
@@ -552,6 +694,7 @@ __global__ void __launch_bounds__(TTPB, HZ_EXPAND_MIN_BLOCKS) k_tree_expand_back
             v.node_info[leaf] = (uint32_t)n_new_edges | ((uint32_t)leaf_player << 8) | (SYM ? (leaf_info & 0xFFFF0000u) : 0u);
             T.n_nodes[t] = n_nodes;
             T.n_edges[t] = e0 + n_new_edges;
+            if (GUMBEL) node_value[(size_t)t * T.max_nodes + leaf] = val_f;
         }
     } else {                                                         // terminal leaf, :333-341
         int oc = outcome_of(ls);
@@ -773,6 +916,85 @@ __global__ void __launch_bounds__(TTPB) k_tree_root_edges(hz_tree T, int32_t* N,
     }
 }
 
+// ---- Gumbel root: played action, policy target and raw value (hz_tree_gumbel_root) ------------------------------------
+__global__ void __launch_bounds__(TTPB) k_tree_gumbel_root(hz_tree T, hz_gumbel_args GB, float* policy, int16_t* actions,
+                                                           float* root_value) {
+    int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    int t = blockIdx.x * WPB + warp;
+    if (t >= T.n_trees) return;
+    float* prow = policy + (size_t)t * HZ_ACTION_SIZE;
+    if (t >= active_trees(T)) {                                          // beyond the active prefix: no search, no move
+        for (int a = lane; a < HZ_ACTION_SIZE; a += 32) prow[a] = 0.0f;
+        if (lane == 0) {
+            actions[t] = -1;
+            if (root_value) root_value[t] = 0.0f;
+        }
+        return;
+    }
+    TreeView v = view_of(T, t);
+    const int ne = (int)(v.node_info[0] & 0xFFu);
+    const uint32_t e0 = v.node_edge0[0];
+    const float vhat = GB.node_value[(size_t)t * T.max_nodes];
+    const uint64_t skey = T.search_key[t];
+    int N[3], A[3], ns = 0;
+    double W[3];
+    float P[3];
+#pragma unroll
+    for (int r = 0; r < 3; r++) {
+        const int k = lane + 32 * r;
+        const bool on = k < ne;
+        if (on) HZ_BOUND(e0 + k, T.max_edges, 106);
+        N[r] = on ? v.edge_N[e0 + k] : 0;
+        W[r] = on ? v.edge_W[e0 + k] : 0.0;
+        P[r] = on ? v.edge_P[e0 + k] : 0.0f;
+        A[r] = on ? v.edge_am[e0 + k] & 0xFF : 0;
+        ns += N[r];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) ns += __shfl_xor_sync(FULL, ns, o);
+    for (int a = lane; a < HZ_ACTION_SIZE; a += 32) prow[a] = 0.0f;
+    __syncwarp();
+    if (ne == 0) {                                                       // terminal or unexpanded root
+        if (lane == 0) {
+            actions[t] = -1;
+            if (root_value) root_value[t] = 0.0f;
+        }
+        return;
+    }
+    double lg[3], sg[3], sc[3], z[3], ez[3];
+    int mxn;
+    gumbel_sigma(GB, ne, lane, ns, N, W, P, vhat, lg, sg, mxn);
+    gumbel_root_scores(GB, skey, ne, lane, mxn, N, A, lg, sg, sc);       // considered visit = max N
+    double best = -INFINITY;
+    int best_k = -1;
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+        if (lane + 32 * r < ne && sc[r] > best) { best = sc[r]; best_k = lane + 32 * r; }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        double ob = __shfl_xor_sync(FULL, best, o);
+        int ok = __shfl_xor_sync(FULL, best_k, o);
+        bool take = ok >= 0 && (best_k < 0 || ob > best || (ob == best && ok < best_k));
+        if (take) { best = ob; best_k = ok; }
+    }
+    if (best_k < 0) best_k = 0;
+    const int br = best_k >> 5;                                          // warp-uniform
+    const int act = __shfl_sync(FULL, br == 0 ? A[0] : br == 1 ? A[1] : A[2], best_k & 31);
+#pragma unroll
+    for (int r = 0; r < 3; r++) z[r] = lg[r] + sg[r];
+    const double s = softmax_terms(ne, lane, z, ez);
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+        if (lane + 32 * r < ne) {
+            HZ_BOUND(A[r], HZ_ACTION_SIZE, 107);
+            prow[A[r]] = (float)(ez[r] / s);
+        }
+    if (lane == 0) {
+        actions[t] = (int16_t)act;
+        if (root_value) root_value[t] = vhat;
+    }
+}
+
 }  // namespace hz
 
 using namespace hz;
@@ -818,7 +1040,7 @@ int hz_tree_create(hz_tree** out, void* workspace, size_t workspace_bytes, int n
     Layout L = layout_for(n_trees, max_sims, max_nodes, leaves);
     if (L.max_edges >= (1 << 24)) return HZ_ERR_ARG;     // edge_cinfo packs the first-edge index into 24 bits
     if (workspace_bytes < L.total || ((uintptr_t)workspace & 255)) return HZ_ERR_WORKSPACE;
-    hz_tree* t = new hz_tree;
+    hz_tree_host* t = new hz_tree_host;
     char* b = (char*)workspace;
     t->n_trees = n_trees; t->max_sims = max_sims; t->max_nodes = L.max_nodes; t->max_edges = L.max_edges;
     t->table_size = L.table_size; t->key_mode = key_mode; t->leaves = leaves;
@@ -836,12 +1058,13 @@ int hz_tree_create(hz_tree** out, void* workspace, size_t workspace_bytes, int n
     t->n_active = nullptr;
     t->sym_mode = HZ_SYM_OFF;
     t->frames_on = 0;
+    t->gumbel = hz_gumbel_args{};
     *out = t;
     return HZ_OK;
 }
 
 int hz_tree_destroy(hz_tree* t) {
-    delete t;
+    delete static_cast<hz_tree_host*>(t);
     return HZ_OK;
 }
 
@@ -874,17 +1097,18 @@ int hz_tree_reset(hz_tree* t, const void* root_states, const uint64_t* search_ke
 
 }  // extern "C"
 
-template <bool CACHE>
+template <bool CACHE, bool GUMBEL>
 static int launch_select(hz_tree* t, float cpuct, void* leaf_states, void* board, void* glob, int dtype, int layout,
                          const EvalCacheArgs& ec, cudaStream_t st) {
+    const hz_gumbel_args gb = GUMBEL ? gumbel_of(t) : hz_gumbel_args{};
     int grid = tree_blocks(t->n_trees, WPB);
     uint4* ls = (uint4*)leaf_states;
     if (layout != HZ_LAYOUT_NCHW && layout != HZ_LAYOUT_NHWC && layout != HZ_LAYOUT_NHWC40 && layout != HZ_LAYOUT_T16K) return HZ_ERR_ARG;
     if (layout == HZ_LAYOUT_T16K && dtype != HZ_DTYPE_BF16) return HZ_ERR_ARG;
 #define HZ_SELECT(T, L)                                                                                                         \
-    (t->sym_mode == HZ_SYM_FULL    ? k_tree_select<T, L, 480, CACHE><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec) \
-     : t->sym_mode == HZ_SYM_BOARD ? k_tree_select<T, L, 4, CACHE><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec)   \
-                                   : k_tree_select<T, L, 0, CACHE><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec))
+    (t->sym_mode == HZ_SYM_FULL    ? k_tree_select<T, L, 480, CACHE, GUMBEL><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec, gb) \
+     : t->sym_mode == HZ_SYM_BOARD ? k_tree_select<T, L, 4, CACHE, GUMBEL><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec, gb)   \
+                                   : k_tree_select<T, L, 0, CACHE, GUMBEL><<<grid, TTPB, 0, st>>>(*t, cpuct, ls, (T*)board, (T*)glob, ec, gb))
     if (dtype == HZ_DTYPE_F32) {
         if (layout == HZ_LAYOUT_NHWC40) HZ_SELECT(float, HZ_LAYOUT_NHWC40);
         else if (layout == HZ_LAYOUT_NHWC) HZ_SELECT(float, HZ_LAYOUT_NHWC);
@@ -906,7 +1130,9 @@ extern "C" {
 
 int hz_tree_select(hz_tree* t, float cpuct, void* leaf_states, void* board, void* glob, int dtype, int layout, void* stream) {
     if (!t || (board && !glob)) return HZ_ERR_ARG;
-    return launch_select<false>(t, cpuct, leaf_states, board, glob, dtype, layout, EvalCacheArgs{}, (cudaStream_t)stream);
+    if (gumbel_of(t).node_value)
+        return launch_select<false, true>(t, cpuct, leaf_states, board, glob, dtype, layout, EvalCacheArgs{}, (cudaStream_t)stream);
+    return launch_select<false, false>(t, cpuct, leaf_states, board, glob, dtype, layout, EvalCacheArgs{}, (cudaStream_t)stream);
 }
 
 int hz_tree_select_cached(hz_tree* t, hz_evalcache* c, float cpuct, void* leaf_states, void* board, void* glob, int dtype,
@@ -916,16 +1142,25 @@ int hz_tree_select_cached(hz_tree* t, hz_evalcache* c, float cpuct, void* leaf_s
     cudaStream_t st = (cudaStream_t)stream;
     cudaError_t e = cudaMemsetAsync(n_eval, 0, sizeof(int32_t), st);     // misses of this step count from 0
     if (e != cudaSuccess) return hz_record_launch(0, e);
-    return launch_select<true>(t, cpuct, leaf_states, board, glob, dtype, layout, EvalCacheArgs{*c, policy, value, eval_rows, n_eval}, st);
+    const EvalCacheArgs ec{*c, policy, value, eval_rows, n_eval};
+    if (gumbel_of(t).node_value) return launch_select<true, true>(t, cpuct, leaf_states, board, glob, dtype, layout, ec, st);
+    return launch_select<true, false>(t, cpuct, leaf_states, board, glob, dtype, layout, ec, st);
 }
 
 int hz_tree_expand_backup(hz_tree* t, const float* policy, const float* value, int is_logits, const float* noise,
                           double eps, void* stream) {
     if (!t || !policy || !value) return HZ_ERR_ARG;
-    if (t->sym_mode != HZ_SYM_OFF)
-        k_tree_expand_backup<true><<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value, is_logits, noise, eps);
-    else
-        k_tree_expand_backup<false><<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, policy, value, is_logits, noise, eps);
+    float* nv = gumbel_of(t).node_value;
+    if (nv && noise) return HZ_ERR_ARG;                                  // Gumbel noise replaces the Dirichlet noise
+    const int grid = tree_blocks(t->n_trees, WPB);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (t->sym_mode != HZ_SYM_OFF) {
+        if (nv) k_tree_expand_backup<true, true><<<grid, TTPB, 0, st>>>(*t, policy, value, is_logits, noise, eps, nv);
+        else k_tree_expand_backup<true, false><<<grid, TTPB, 0, st>>>(*t, policy, value, is_logits, noise, eps, nullptr);
+    } else {
+        if (nv) k_tree_expand_backup<false, true><<<grid, TTPB, 0, st>>>(*t, policy, value, is_logits, noise, eps, nv);
+        else k_tree_expand_backup<false, false><<<grid, TTPB, 0, st>>>(*t, policy, value, is_logits, noise, eps, nullptr);
+    }
     return hz_launched(1);
 }
 
@@ -972,6 +1207,57 @@ int hz_tree_stats(hz_tree* t, int32_t* n_nodes, int32_t* n_edges, uint8_t* statu
     if (e == cudaSuccess && n_edges) e = cudaMemcpyAsync(n_edges, t->n_edges, (size_t)t->n_trees * 4, cudaMemcpyDeviceToDevice, st);
     if (e == cudaSuccess && status) e = cudaMemcpyAsync(status, t->status, (size_t)t->n_trees, cudaMemcpyDeviceToDevice, st);
     return hz_record_launch(0, e);
+}
+
+// get_sequence_of_considered_visits(m, n) of mctx (seq_halving.py): the root visit count that simulation i considers
+static void considered_visits(int m, int n, int32_t* seq) {
+    if (m <= 1) {
+        for (int i = 0; i < n; i++) seq[i] = i;
+        return;
+    }
+    int log2max = 0;
+    while ((1 << log2max) < m) log2max++;                                // ceil(log2(m))
+    int visits[64] = {0}, len = 0, nc = m;
+    while (len < n) {
+        const int extra = std::max(1, (int)((double)n / (double)(log2max * nc)));
+        for (int x = 0; x < extra; x++) {
+            for (int i = 0; i < nc && len < n; i++) seq[len++] = visits[i];
+            for (int i = 0; i < nc; i++) visits[i]++;
+        }
+        nc = std::max(2, nc / 2);
+    }
+}
+
+size_t hz_tree_gumbel_bytes(const hz_tree* t, int max_considered, int num_sims) {
+    if (!t || max_considered < 1 || max_considered > 64 || num_sims < 1 || num_sims > t->max_sims) return 0;
+    return align256((size_t)t->n_trees * t->max_nodes * 4) + align256((size_t)(max_considered + 1) * num_sims * 4);
+}
+
+int hz_tree_set_gumbel(hz_tree* t, void* buffer, size_t bytes, int max_considered, int num_sims, float c_visit, float c_scale,
+                       float gumbel_scale, void* stream) {
+    if (!t) return HZ_ERR_ARG;
+    if (!buffer) {
+        gumbel_of(t) = hz_gumbel_args{};
+        return HZ_OK;
+    }
+    if (t->leaves != 1 || max_considered < 1 || max_considered > 64 || num_sims < 1 || num_sims > t->max_sims) return HZ_ERR_ARG;
+    if (!std::isfinite(c_visit) || !std::isfinite(c_scale) || !std::isfinite(gumbel_scale)) return HZ_ERR_ARG;
+    if (bytes < hz_tree_gumbel_bytes(t, max_considered, num_sims) || ((uintptr_t)buffer & 255)) return HZ_ERR_WORKSPACE;
+    const size_t nv_bytes = align256((size_t)t->n_trees * t->max_nodes * 4);
+    std::vector<int32_t> table((size_t)(max_considered + 1) * num_sims);
+    for (int k = 0; k <= max_considered; k++) considered_visits(k, num_sims, table.data() + (size_t)k * num_sims);
+    int32_t* dtable = (int32_t*)((char*)buffer + nv_bytes);
+    cudaError_t e = cudaMemcpyAsync(dtable, table.data(), table.size() * 4, cudaMemcpyHostToDevice, (cudaStream_t)stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize((cudaStream_t)stream);   // the table is a host temporary
+    if (e != cudaSuccess) return hz_record_launch(0, e);
+    gumbel_of(t) = hz_gumbel_args{(float*)buffer, dtable, max_considered, num_sims, c_visit, c_scale, gumbel_scale};
+    return HZ_OK;
+}
+
+int hz_tree_gumbel_root(hz_tree* t, float* policy, int16_t* actions, float* root_value, void* stream) {
+    if (!t || !policy || !actions || !gumbel_of(t).node_value) return HZ_ERR_ARG;
+    k_tree_gumbel_root<<<tree_blocks(t->n_trees, WPB), TTPB, 0, (cudaStream_t)stream>>>(*t, gumbel_of(t), policy, actions, root_value);
+    return hz_launched(1);
 }
 
 int hz_tree_root_edges(hz_tree* t, int32_t* N, double* W, float* P, int32_t* child, void* stream) {

@@ -5,7 +5,8 @@ pickled whole every iteration (buffer.py:7-67, trainer.py:127,146-153,250-254). 
 examples stay packed on the device — 128 B state + 143 x int16 visit counts + z = 418 B — and
 a training batch is produced on the fly by hz_encode: no H2D copy and no DataLoader on the
 training path.  ``to_reference_buffer`` exports the reference's exact structure so that
-``buffer.save_buffer`` / ``ReplayBufferDataset`` keep working.
+``buffer.save_buffer`` / ``ReplayBufferDataset`` keep working.  A ring of Gumbel-search examples
+(Trajectories.policy) also stores their fp32 policy targets (+572 B per example) and trains on them.
 """
 
 from collections import deque
@@ -21,6 +22,7 @@ class ReplayRing:
         self.states = torch.zeros((self.capacity, 32), dtype=torch.int32, device=self.device)
         self.visits = torch.zeros((self.capacity, 143), dtype=torch.int16, device=self.device)
         self.z = torch.zeros(self.capacity, dtype=torch.float32, device=self.device)
+        self.policy = None  # float32 [capacity, 143], allocated by the first extend with Gumbel policy targets
         self.size = 0      # valid examples
         self.head = 0      # next write position (oldest example once full) — deque(maxlen) semantics
 
@@ -33,11 +35,22 @@ class ReplayRing:
         n = len(traj)
         if n == 0:
             return
+        has_policy = getattr(traj, "policy", None) is not None
+        if self.size and has_policy != (self.policy is not None):
+            raise ValueError("a replay ring holds either Gumbel policy targets or visit counts, not both")
+        if has_policy and self.policy is None:
+            self.policy = torch.zeros((self.capacity, 143), dtype=torch.float32, device=self.device)
+        if not has_policy:
+            self.policy = None
         S, V, Z = traj.states.to(self.device), traj.visits.to(self.device), traj.z.to(self.device)
+        P = traj.policy.to(self.device) if has_policy else None
         if n >= self.capacity:                      # only the newest `capacity` examples survive
             S, V, Z, n = S[-self.capacity:], V[-self.capacity:], Z[-self.capacity:], self.capacity
+            P = None if P is None else P[-self.capacity:]
         idx = (self.head + torch.arange(n, device=self.device)) % self.capacity
         self.states[idx], self.visits[idx], self.z[idx] = S, V, Z
+        if P is not None:
+            self.policy[idx] = P
         self.head = (self.head + n) % self.capacity
         self.size = min(self.capacity, self.size + n)
 
@@ -67,15 +80,19 @@ class ReplayRing:
         return random_elements(n, augment, device=self.device, generator=generator)
 
     def _batch(self, idx, dtype=torch.float32, sym=None):
-        states, visits = self.states[idx].contiguous(), self.visits[idx]
+        states = self.states[idx].contiguous()
+        target = self.visits[idx] if self.policy is None else self.policy[idx]
         if sym is not None:
             from .symmetry import transform_actions, transform_states
 
-            visits = transform_actions(visits.contiguous(), sym, states)
+            target = transform_actions(target.contiguous(), sym, states)
             transform_states(states, sym, out=states)
         board, glob = hb.encode(states, dtype=dtype)
-        v = visits.to(torch.float64)
-        pi = (v / v.sum(dim=1, keepdim=True).clamp_min(1)).to(torch.float32)      # trainer.py:535
+        if self.policy is not None:
+            pi = target
+        else:
+            v = target.to(torch.float64)
+            pi = (v / v.sum(dim=1, keepdim=True).clamp_min(1)).to(torch.float32)      # trainer.py:535
         return board, glob, pi, self.z[idx].view(-1, 1)
 
     def epoch(self, batch_size, shuffle=True, generator=None, augment=None):
@@ -101,12 +118,19 @@ class ReplayRing:
 
     def state_dict(self):
         order = self._ordered_index()
-        return {"states": self.states[order].cpu(), "visits": self.visits[order].cpu(), "z": self.z[order].cpu(),
-                "capacity": self.capacity}
+        sd = {"states": self.states[order].cpu(), "visits": self.visits[order].cpu(), "z": self.z[order].cpu(),
+              "capacity": self.capacity}
+        if self.policy is not None:
+            sd["policy"] = self.policy[order].cpu()
+        return sd
 
     def load_state_dict(self, sd):
         n = min(self.capacity, sd["states"].shape[0])
         self.states[:n] = sd["states"][-n:].to(self.device)
         self.visits[:n] = sd["visits"][-n:].to(self.device)
         self.z[:n] = sd["z"][-n:].to(self.device)
+        self.policy = None
+        if sd.get("policy") is not None:
+            self.policy = torch.zeros((self.capacity, 143), dtype=torch.float32, device=self.device)
+            self.policy[:n] = sd["policy"][-n:].to(self.device)
         self.size, self.head = n, n % self.capacity

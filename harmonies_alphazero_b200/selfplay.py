@@ -12,7 +12,8 @@ Output contract = the reference worker's (trainer.py:531-538): one example per a
 every completed game: (board f32[38,5,7], global f32[42], pi f32[143], z f32[1]) with the
 state encoded BEFORE the search of that move, pi = root visit distribution, z = final
 outcome from the mover's perspective (0 on a draw).  Examples are kept packed on the device
-(128 B state + int16 visit counts) and expanded on demand.
+(128 B state + int16 visit counts) and expanded on demand.  With SelfPlayConfig.search = "gumbel" pi is the Gumbel
+search's improved policy (Trajectories.policy, fp32) instead.
 """
 
 import time
@@ -49,11 +50,20 @@ class SelfPlayConfig:
     # needs about n_slots * num_simulations entries (leaves_per_step rows per simulation step) at about 600 B each; fewer
     # entries evict and cost hits, never correctness.  Needs a row-invariant network (InferenceNet on the tile path).
     eval_cache: int = 0
+    # Root search: "puct" (the reference's) or "gumbel" (BatchedMCTS.set_gumbel: sequential halving over the top gumbel_m
+    # root actions, completed-Q targets; DESIGN.md §13).  Gumbel play takes its moves and its policy targets from the
+    # search (Trajectories.policy) and ignores turns_until_tau0 and the Dirichlet settings; testing sets the noise to 0.
+    search: str = "puct"
+    gumbel_m: int = 16
+    gumbel_c_visit: float = 50.0
+    gumbel_c_scale: float = 0.1
+    gumbel_scale: float = 1.0
 
     @classmethod
     def from_mcts_config(cls, mcts_config, **kw):
         """Reads the keys MCTS.py reads (SURVEY.md §5): num_simulations, cpuct,
-        dirichlet_alpha, dirichlet_epsilon, turns_until_tau0, testing."""
+        dirichlet_alpha, dirichlet_epsilon, turns_until_tau0, testing; and search, gumbel_m, gumbel_c_visit,
+        gumbel_c_scale where present."""
         m = dict(
             num_simulations=int(mcts_config["num_simulations"]),
             cpuct=float(mcts_config["cpuct"]),
@@ -62,6 +72,9 @@ class SelfPlayConfig:
             turns_until_tau0=int(mcts_config.get("turns_until_tau0", 15)),
             testing=bool(mcts_config.get("testing", False)),
         )
+        for key, conv in (("search", str), ("gumbel_m", int), ("gumbel_c_visit", float), ("gumbel_c_scale", float)):
+            if key in mcts_config:
+                m[key] = conv(mcts_config[key])
         m.update(kw)
         return cls(**m)
 
@@ -75,11 +88,15 @@ class Trajectories:
     game_id: torch.Tensor   # int64 [M]
     move_no: torch.Tensor   # int32 [M]
     stats: dict = field(default_factory=dict)
+    policy: torch.Tensor = None   # float32 [M, 143] the Gumbel search's improved policy (search="gumbel"), else None
 
     def __len__(self):
         return int(self.states.shape[0])
 
     def pi(self):
+        """The training target: the Gumbel policy when present, else visits / sum (trainer.py:535)."""
+        if self.policy is not None:
+            return self.policy.clone()
         v = self.visits.to(torch.float64)
         return (v / v.sum(dim=1, keepdim=True).clamp_min(1)).to(torch.float32)   # trainer.py:535
 
@@ -97,27 +114,32 @@ class Trajectories:
         if n == 0:
             return []
         lo = 0 if last is None else max(0, n - int(last))
-        sub = self if lo == 0 else Trajectories(self.states[lo:], self.visits[lo:], self.z[lo:], self.game_id[lo:], self.move_no[lo:])
+        sub = self if lo == 0 else Trajectories(self.states[lo:], self.visits[lo:], self.z[lo:], self.game_id[lo:], self.move_no[lo:],
+                                                policy=None if self.policy is None else self.policy[lo:])
         board, glob = sub.encode()
         fields = [t.cpu().numpy() for t in (board, glob, sub.pi(), sub.z.view(-1, 1))]
         fn = torch.from_numpy
         return [tuple(fn(f[i].copy()) for f in fields) for i in range(n - lo)]
 
     def transform(self, sym):
-        """A copy with every example mapped by a group element (symmetry.py): states T_g(state), visits
+        """A copy with every example mapped by a group element (symmetry.py): states T_g(state), visits and policy
         x'[sigma_g(a)] = x[a], z and the ids unchanged.  sym: int or int[M] (0..479)."""
         from .symmetry import transform_actions, transform_states
 
+        pol = None if self.policy is None else self.policy.clone()
         if len(self) == 0:
             return Trajectories(self.states.clone(), self.visits.clone(), self.z.clone(), self.game_id.clone(),
-                                self.move_no.clone(), dict(self.stats))
+                                self.move_no.clone(), dict(self.stats), pol)
         states = self.states.contiguous()
+        if pol is not None:
+            pol = transform_actions(self.policy.contiguous(), sym, states)
         return Trajectories(transform_states(states, sym), transform_actions(self.visits.contiguous(), sym, states),
-                            self.z.clone(), self.game_id.clone(), self.move_no.clone(), dict(self.stats))
+                            self.z.clone(), self.game_id.clone(), self.move_no.clone(), dict(self.stats), pol)
 
     def to(self, device):
         return Trajectories(self.states.to(device), self.visits.to(device), self.z.to(device),
-                            self.game_id.to(device), self.move_no.to(device), dict(self.stats))
+                            self.game_id.to(device), self.move_no.to(device), dict(self.stats),
+                            None if self.policy is None else self.policy.to(device))
 
 
 class SyntheticEvaluator:
@@ -178,6 +200,14 @@ class _Group:
             raise ValueError("num_simulations must be a multiple of leaves_per_step")
         self.tree = BatchedMCTS(n, cfg.num_simulations, device=dev, key_mode=cfg.key_mode, max_nodes=cfg.max_nodes, leaves=K)
         self.tree.set_symmetry(cfg.eval_symmetry)     # before any capture: a graph keeps the mode it was captured with
+        if cfg.search not in ("puct", "gumbel"):
+            raise ValueError(f"search must be 'puct' or 'gumbel', not {cfg.search!r}")
+        self.gumbel = cfg.search == "gumbel"
+        if self.gumbel:
+            if K != 1:
+                raise ValueError("Gumbel search runs one simulation in flight per tree: leaves_per_step must be 1")
+            self.tree.set_gumbel(m=cfg.gumbel_m, num_sims=cfg.num_simulations, c_visit=cfg.gumbel_c_visit,
+                                 c_scale=cfg.gumbel_c_scale, scale=0.0 if cfg.testing else cfg.gumbel_scale)
         rows = n * K                  # the network sees K leaves per tree and step
         dt, cl = net.dtype, owner.channels_last
         self.tiles = bool(getattr(net, "wants_tiles", False))   # leaves go straight into the hand-written tower's input image
@@ -203,8 +233,9 @@ class _Group:
             self.net_value = torch.zeros(rows, dtype=torch.float32, device=dev)
             self.eval_rows = torch.zeros(rows, dtype=torch.int32, device=dev)
             self.n_eval = torch.zeros(1, dtype=torch.int32, device=dev)
-        self.noise = None if cfg.testing else torch.ones((n, 143), dtype=torch.float32, device=dev)
-        self.alpha = None if cfg.testing else torch.full((n, 143), cfg.dirichlet_alpha, dtype=torch.float32, device=dev)
+        no_noise = cfg.testing or self.gumbel        # the Gumbel noise replaces the root's Dirichlet noise
+        self.noise = None if no_noise else torch.ones((n, 143), dtype=torch.float32, device=dev)
+        self.alpha = None if no_noise else torch.full((n, 143), cfg.dirichlet_alpha, dtype=torch.float32, device=dev)
         self.graph = None
         self.graph_version = 0
         self.stream = torch.cuda.Stream(device=dev) if owner.n_groups > 1 else None
@@ -346,6 +377,11 @@ class BatchedSelfPlay:
         parts = [g.tree.root_policy() for g in self.groups]
         return torch.cat([p[0] for p in parts]), torch.cat([p[1] for p in parts])
 
+    def gumbel_root(self):
+        """(policy [B,143], actions [B], root_value [B]) of the Gumbel searches (BatchedMCTS.gumbel_root)"""
+        parts = [g.tree.gumbel_root() for g in self.groups]
+        return tuple(torch.cat([p[i] for p in parts]) for i in range(3))
+
     def choose(self, u01=None, exploratory=None):
         return torch.cat([
             g.tree.choose(None if u01 is None else u01[g.lo:g.hi].contiguous(),
@@ -370,6 +406,7 @@ class BatchedSelfPlay:
         chunks, bad_status = [], torch.zeros((), dtype=torch.uint8, device=dev)
         live_sims = 0
         compact = cfg.compact_live and self.n_groups == 1
+        gumbel = cfg.search == "gumbel"
         for g in self.groups:
             g.set_active(g.hi - g.lo)             # (a previous call that raised may have left a smaller active prefix)
             if g.cache is not None:
@@ -411,12 +448,15 @@ class BatchedSelfPlay:
             snap = states.clone()
             self.search(states)
             visits, _ = self.root_policy()
-            expl = None
-            u01 = None
-            if not cfg.testing and cfg.turns_until_tau0 > 0:
-                expl = (move_no < cfg.turns_until_tau0).to(torch.uint8)   # MCTS.py:399-402
-                u01 = torch.rand(B, device=dev, dtype=torch.float32)
-            actions = self.choose(u01, expl)
+            if gumbel:                                           # the move and the target come from the search
+                policy, actions, _ = self.gumbel_root()
+            else:
+                expl = None
+                u01 = None
+                if not cfg.testing and cfg.turns_until_tau0 > 0:
+                    expl = (move_no < cfg.turns_until_tau0).to(torch.uint8)   # MCTS.py:399-402
+                    u01 = torch.rand(B, device=dev, dtype=torch.float32)
+                actions = self.choose(u01, expl)
             # a root without visits (num_simulations <= leaves_per_step, or a search that only ever
             # reached the unexpanded root) has no move to offer: the reference then plays a random
             # legal move and records the all-zero visit vector (MCTS.py:382-392,425-433 — its uniform
@@ -425,7 +465,7 @@ class BatchedSelfPlay:
             actions = torch.where(live, actions, torch.full_like(actions, -1))
             status = hb.apply(states, actions)                   # the real move re-draws independently (trainer.py:502)
             bad_status = torch.maximum(bad_status, torch.where(live, status, torch.zeros_like(status)).max())
-            chunks.append((snap, visits.to(torch.int16), game_id.clone(), move_no, live.clone()))
+            chunks.append((snap, visits.to(torch.int16), game_id.clone(), move_no, live.clone()) + ((policy,) if gumbel else ()))
             live_sims += n_live * cfg.num_simulations
             step += 1
             if step % 8 == 0:
@@ -444,12 +484,14 @@ class BatchedSelfPlay:
             G = torch.cat([c[2] for c in chunks]); M = torch.cat([c[3] for c in chunks]); L = torch.cat([c[4] for c in chunks])
             keep = L & finished[G.clamp_max(num_games - 1)]
             S, V, G, M = S[keep], V[keep], G[keep], M[keep]
+            Pol = torch.cat([c[5] for c in chunks])[keep] if gumbel else None
             mover = ((S[:, 22] >> 24) & 1).to(torch.float32)
             z = outcome[G].to(torch.float32) * (1.0 - 2.0 * mover)   # trainer.py:523-528
         else:
             S = torch.empty((0, 32), dtype=torch.int32, device=dev); V = torch.empty((0, 143), dtype=torch.int16, device=dev)
             G = torch.empty(0, dtype=torch.int64, device=dev); M = torch.empty(0, dtype=torch.int32, device=dev)
             z = torch.empty(0, dtype=torch.float32, device=dev)
+            Pol = torch.empty((0, 143), dtype=torch.float32, device=dev) if gumbel else None
         stats = {"sims": live_sims, "seconds": secs, "sims_per_s": live_sims / secs if secs > 0 else 0.0,
                  "games": int(finished.sum().item()), "examples": int(S.shape[0]), "move_steps": step,
                  "searched_slots": searched_slots}
@@ -459,4 +501,4 @@ class BatchedSelfPlay:
             c.update(hit_rate=c["hits"] / max(1, c["looked_up"]), terminal_fraction=c["terminal"] / max(1, c["looked_up"]),
                      net_rows_per_step=c["misses"] / max(1, steps), bytes=sum(g.cache.bytes for g in self.groups))
             stats["eval_cache"] = c
-        return Trajectories(S, V, z, G + cfg.first_game_id, M, stats)
+        return Trajectories(S, V, z, G + cfg.first_game_id, M, stats, Pol)

@@ -61,6 +61,39 @@ class BatchedMCTS:
 
         _lib.check(self.lib.hz_tree_set_symmetry(self.handle, mode_code(mode)), "hz_tree_set_symmetry")
 
+    def set_gumbel(self, m=16, num_sims=None, c_visit=50.0, c_scale=0.1, scale=1.0):
+        """Gumbel search (hz_tree_set_gumbel; include/harmonies_b200.h states the rules): sequential halving over the top m
+        root actions by Gumbel noise + logit, completed-Q selection below the root, for searches of num_sims simulations
+        (default max_sims).  scale = 0 removes the noise (evaluation play).  m=None switches the mode off.  Acts on the
+        calls that follow (set it before ``reset``); this object owns the mode's buffer and reuses it when the mode is set
+        again."""
+        if m is None:
+            _lib.check(self.lib.hz_tree_set_gumbel(self.handle, None, 0, 0, 0, 0.0, 0.0, 0.0, None), "hz_tree_set_gumbel")
+            return
+        n = int(num_sims or self.max_sims)
+        nbytes = self.lib.hz_tree_gumbel_bytes(self.handle, int(m), n)
+        if nbytes == 0 or self.leaves != 1:
+            raise ValueError("Gumbel search needs leaves == 1, 1 <= m <= 64 and 1 <= num_sims <= max_sims")
+        buf = getattr(self, "_gumbel", None)
+        if buf is None or buf.numel() < nbytes:
+            buf = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.hz_tree_set_gumbel(self.handle, buf.data_ptr(), buf.numel(), int(m), n, float(c_visit), float(c_scale),
+                                                   float(scale), self._stream()), "hz_tree_set_gumbel")
+        self._gumbel = buf
+
+    def gumbel_root(self):
+        """(policy fp32 [n,143], actions int16 [n], root_value fp32 [n]) of the Gumbel search: the improved policy target
+        softmax(logit + sigma) over the root's edges, the played action (-1 for a root without edges) and the root's raw
+        value."""
+        policy = torch.empty((self.n, 143), dtype=torch.float32, device=self.device)
+        actions = torch.empty(self.n, dtype=torch.int16, device=self.device)
+        value = torch.empty(self.n, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.hz_tree_gumbel_root(self.handle, _ptr(policy), _ptr(actions), _ptr(value), self._stream()),
+                       "hz_tree_gumbel_root")
+        return policy, actions, value
+
     def leaf_frames(self):
         """int64[rows]: the frame g of every leaf row of the last ``select`` (0 when it ran with the mode off)."""
         out = torch.empty(self.rows, dtype=torch.int16, device=self.device)

@@ -398,6 +398,45 @@ int hz_tree_stats(hz_tree *t, int32_t *n_nodes, int32_t *n_edges, uint8_t *statu
 int hz_tree_root_edges(hz_tree *t, int32_t *N, double *W, float *P, int32_t *child,
                        void *stream);
 
+/* ---- Gumbel search (Danihelka et al., ICLR 2022; mctx's gumbel_muzero_policy with qtransform_completed_by_mix_value) ----
+ * An opt-in replacement of the PUCT descent for searches of a few simulations.  Off by default; with it off every search
+ * is the reference's PUCT search bit for bit.  One simulation in flight per tree (leaves == 1).  All arithmetic is fp64.
+ * For a node with edges b (legal moves, ascending action) and their N, W, P:
+ *  pi(b)     = P(b) / sum_b P(b)   (P is a softmax over all 143 logits, so the legal edges need not sum to 1);
+ *  logit(b)  = log(max(P(b), FLT_MIN));   q(b) = W(b) / N(b) for N(b) > 0 (the node's player-to-move view);
+ *  vhat      = the evaluator's value of the node, kept when it was expanded (hz_tree_set_gumbel's node_value);
+ *  v_mix     = (vhat + sum N * S_q / S_pi) / (1 + sum N),  S_pi = sum_{N>0} max(pi, FLT_MIN),
+ *              S_q = sum_{N>0} max(pi, FLT_MIN) * q  (S_q / S_pi := 0 when no edge is visited);
+ *  Qc(b)     = q(b) if N(b) > 0 else v_mix, rescaled by the node's min and max: (Qc - min) / max(max - min, 1e-8);
+ *  sigma(b)  = ((c_visit + max_b N(b)) * c_scale) * Qc(b);
+ *  interior  = argmax_b  softmax(logit + sigma)(b) - N(b) / (1 + sum N);  ties: lowest edge index (PUCT's first maximum);
+ *  root      = with k = min(m, root edges), i = min(sum_root N, n - 1), cv = table[k][i] (mctx's
+ *              get_table_of_considered_visits(m, n)): argmax over the edges with N(b) == cv of
+ *              max(-1e9, g(b) + (logit(b) - max logit) + sigma(b)); lowest index on ties, edge 0 if no edge has N == cv;
+ *  g(a)      = gumbel_scale * -log(-log(u)),  u = ((rand64(search_key ^ HZ_GUMBEL_SALT, a) >> 11) + 0.5) * 2^-53 (a = action):
+ *              the search key only, so a captured graph needs no host state;
+ *  played    = the root rule with cv = max_b N(b) (zero root visits: a Gumbel-top-1 sample of the prior);
+ *  target    = softmax(logit + sigma) over the root edges, fp32 [143] by action, 0 off the legal set.
+ * A root with one edge plays it with a one-hot target; a terminal or unexpanded root gives action -1 and a zero row.
+ * mctx's defaults: m = 16, c_visit = 50, c_scale = 0.1, gumbel_scale = 1 (0 for evaluation play). */
+#define HZ_GUMBEL_SALT 0x47554D42454C5F31ull
+
+/* Bytes of the caller-owned Gumbel buffer (0 for bad arguments): node_value (fp32 per node slot of every tree) and the
+ * considered-visit table for k = 0..max_considered.  max_considered in 1..64, num_sims in 1..max_sims. */
+size_t hz_tree_gumbel_bytes(const hz_tree *t, int max_considered, int num_sims);
+/* Switches Gumbel mode on for the launches that follow (buffer == NULL: off).  The buffer (256-byte aligned, >=
+ * hz_tree_gumbel_bytes, else HZ_ERR_WORKSPACE) belongs to the caller and must outlive the mode; the call writes the table
+ * into it.  HZ_ERR_ARG for leaves != 1, max_considered outside 1..64, num_sims outside 1..max_sims, or a non-finite
+ * constant.  In Gumbel mode hz_tree_expand_backup refuses Dirichlet noise (HZ_ERR_ARG) and stores node_value at every
+ * expansion; hz_tree_select and hz_tree_select_cached descend by the rules above (composes with the cache and the
+ * symmetry frames).  Set it before hz_tree_reset; a captured CUDA graph keeps the mode of its capture. */
+int hz_tree_set_gumbel(hz_tree *t, void *buffer, size_t bytes, int max_considered, int num_sims, float c_visit,
+                       float c_scale, float gumbel_scale, void *stream);
+/* One warp per tree: policy [n_trees,143] fp32 = the target, actions [n_trees] int16 = the played action, root_value
+ * [n_trees] fp32 (nullable) = vhat(root) (0 for a root without edges).  Trees beyond the active prefix
+ * (hz_tree_set_active) get action -1, a zero row and value 0.  HZ_ERR_ARG when the mode is off. */
+int hz_tree_gumbel_root(hz_tree *t, float *policy, int16_t *actions, float *root_value, void *stream);
+
 /* ---- leaf evaluation cache -----------------------------------------------------------------
  * An opt-in memo of the evaluator's rows, so that a step sends only the leaves that need the network through it.  The
  * reference builds a new tree for every move and so does this library, but three of the four actions of a turn (the pile
